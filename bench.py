@@ -2,12 +2,23 @@
 """Benchmark of the hot path: ContactNets loss + backward, cube, fp64 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--dtype f64|f32] [--impl reference]
+                    [--dump-outputs DIR]
 
 One step = one pass of ``system.contactnets_loss(x, u, x_plus).mean().backward()`` over one
 synthetic batch (SURVEY.md section 8(d)) of B state pairs per GPU.  Prints ONE JSON line (rank 0).
+The headline figure is the mean over exactly K timed steps after W (at least 3) untimed ones; the default K = 3000
+makes that window about 1 s at the default batch (0.35 ms per step on a B200 at its 1,000 W power limit), long enough
+for the clock sampler (nvidia-smi every 100 ms) to sample inside it.  The eager, kernel-only and end-to-end timings take
+their step counts from K as well.
 For N > 1 launch with ``python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N``:
 one process per GPU, the batch sharded by sample (each rank its own B samples: weak scaling),
 NCCL all-reduce of the 15-double gradient/loss buffer inside every step.
+
+``--dump-outputs DIR`` writes what the last timed step computed: ``loss.npy`` (the per-sample losses in
+generator order; a fixed, seeded sample of 4,194,304 of them when the batch is larger), ``loss_mean.npy`` and
+``grad.<parameter name>.npy``.  The inputs depend only on the arguments, so two builds run with the same
+arguments can be compared output for output: the per-sample losses repeat bit for bit, the gradients only to
+rounding (they are sums in the order the dynamic schedule hands out the work).
 
 ``--impl reference`` times the reference's CPU path instead: the oracle port
 (oracle/contactnets_oracle.py: the reference's algorithm restated in batched fp64 PyTorch +
@@ -37,7 +48,7 @@ METRIC = 'ContactNets loss+backward samples/s, cube'
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=3000, help='timed steps of the headline measurement')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--batch', type=int, default=1 << 20, help='samples per step: global (strong scaling) or per GPU (weak)')
     ap.add_argument('--dtype', choices=['f64', 'f32'], default='f64')
@@ -54,7 +65,14 @@ def parse_args():
                     help='gradient exchange: in-kernel peer-memory all-reduce (default) or NCCL after the step')
     ap.add_argument('--order', choices=['cost', 'natural'], default='cost',
                     help='batch order: by decreasing Newton count of the previous pass (default) or generator order')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the loss and the gradients of the last timed step as DIR/<name>.npy (one process only)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs is not None and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA path: not with --impl reference')
+    return args
 
 
 class ClockSampler:
@@ -420,6 +438,22 @@ def secondary_configs(device, peak_flops):
     return out
 
 
+DUMP_MAX_ROWS = 1 << 22      # per-sample losses written by --dump-outputs: 32 MB in float64, the dump stays under 64 MB
+
+
+def dump_outputs(out_dir, loss, mean, grads, names):
+    """Writes out_dir/<name>.npy: the per-sample losses (a fixed, seeded sample of DUMP_MAX_ROWS of them when there
+    are more), the mean loss and the gradient of every parameter."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    if loss.shape[0] > DUMP_MAX_ROWS:
+        pick = torch.randperm(loss.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ROWS].sort().values
+        loss = loss.index_select(0, pick.to(loss.device))
+    arrays = {'loss': loss, 'loss_mean': mean, **{f'grad.{n}': g for n, g in zip(names, grads)}}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().cpu().numpy())
+
+
 def cpu_reference_step(batch, threads):
     """Builds the oracle-port step (loss + backward) on the host; returns a callable."""
     from dair_pll_b200 import synthetic
@@ -504,6 +538,8 @@ def main():
     if world != args.gpus:
         if world == 1 and args.gpus > 1:
             raise SystemExit('launch N>1 with torch.distributed.run --nproc-per-node N')
+    if args.dump_outputs is not None and world > 1:
+        raise SystemExit('--dump-outputs needs a single process (--gpus 1)')
     # N < visible GPUs: spread the ranks over the box (rank r -> GPU r * stride).  On the HGX boards of this pool four GPUs
     # share one PCIe root (measured: ~105 GB/s of pinned host->device copies per group of four, 51 GB/s per GPU), so four
     # ranks on GPUs 0-3 get half the end-to-end copy bandwidth of four ranks on GPUs 0, 2, 4, 6; NVLink is all-to-all.
@@ -540,6 +576,7 @@ def main():
     system.record_newton_iters = False
 
     def shard(order):
+        """This rank's (x, x_plus) in the given order and their rows of the generated batch (None: all, in order)."""
         if scaling == 'strong':
             if order == 'cost':      # dealt round-robin from the cost-ordered global batch: equally expensive shards
                 idx = torch.argsort(hint, descending=True, stable=True)[rank::world]
@@ -549,8 +586,8 @@ def main():
         else:
             idx = torch.argsort(hint, descending=True, stable=True) if order == 'cost' else None
         if idx is None:
-            return xg, xpg
-        return xg.index_select(0, idx).contiguous(), xpg.index_select(0, idx).contiguous()
+            return xg, xpg, None
+        return xg.index_select(0, idx).contiguous(), xpg.index_select(0, idx).contiguous(), idx
 
     comm = None
     if world > 1 and args.allreduce == 'peer':
@@ -563,29 +600,22 @@ def main():
             dist.barrier()
         torch.cuda.synchronize(device)
 
-    def timed(fn, steps, warmup, min_ms=0.0):
-        """Mean ms per call of fn over repetitions of `steps` calls lasting at least min_ms in total (device
-        time, CUDA events, max over ranks).  Returns (ms per step, number of timed steps)."""
+    def timed(fn, steps, warmup):
+        """Mean ms per call of fn over `steps` calls after `warmup` untimed ones (device time, CUDA events, max
+        over ranks)."""
         for _ in range(warmup):
             fn()
         barrier()
-        reps, total_ms, total_steps = 1, 0.0, 0
-        while True:
-            start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            start.record()
-            for _ in range(reps * steps):
-                fn()
-            stop.record()
-            barrier()
-            ms = torch.tensor([start.elapsed_time(stop)], device=device, dtype=torch.float64)
-            if world > 1:
-                dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-            total_ms += ms.item()
-            total_steps += reps * steps
-            if total_ms >= min_ms:
-                return total_ms / total_steps, total_steps
-            # the same repetition count on every rank: derived from the all-reduced time
-            reps = max(1, min(100000, int((min_ms - total_ms) / max(ms.item() / (reps * steps), 1e-3) / steps) + 1))
+        start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        start.record()
+        for _ in range(steps):
+            fn()
+        stop.record()
+        barrier()
+        ms = torch.tensor([start.elapsed_time(stop)], device=device, dtype=torch.float64)
+        if world > 1:
+            dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+        return ms.item() / steps
 
     L2_BYTES = 126e6
 
@@ -593,7 +623,7 @@ def main():
         """The public-API step on this rank's shard: loss.mean().backward() -> (global) mean loss + param.grad.
         A shard that would fit the L2 (strong scaling, N > 1) is replicated into enough distinct buffers that consecutive
         steps never read rows still resident from the previous ones: the steps cycle through > 2 L2 sizes of inputs."""
-        x, xp = shard(order)
+        x, xp, rows = shard(order)
         step_bytes = 2 * x.shape[0] * 13 * x.element_size()
         copies = 1 if step_bytes > L2_BYTES else int(2.5 * L2_BYTES / step_bytes) + 1
         bufs = [(x, xp)] + [(x.clone(), xp.clone()) for _ in range(copies - 1)]
@@ -609,41 +639,54 @@ def main():
                 else:
                     for p in params:
                         p.grad = None
-                mean = system.contactnets_loss(xx, u, xxp).mean()
+                loss = system.contactnets_loss(xx, u, xxp)
+                mean = loss.mean()
                 mean.backward()
+                # once captured, these are the graph's own output buffers: every replay rewrites them
+                step_local.outputs = (loss.detach(), mean.detach(), [p.grad for p in params])
                 return reducer.stage(mean) if reducer is not None else mean
             return step_local
         locals_ = [make_local(xx, xxp) for xx, xxp in bufs]
+
+        def in_generator_order(outputs):
+            loss, mean, grads = outputs
+            if rows is not None:
+                loss = torch.empty_like(loss).index_copy_(0, rows, loss)
+            return loss, mean, grads
 
         def step_eager():
             turn['eager'] = (turn['eager'] + 1) % copies
             out = locals_[turn['eager']]()
             return reducer.reduce() if reducer is not None else out
         if args.no_graph:
-            return step_eager, step_eager, x, xp, copies
+            return step_eager, step_eager, x, xp, copies, lambda: in_generator_order(locals_[turn['eager']].outputs)
         # with the in-kernel exchange the WHOLE step is one CUDA graph; with NCCL the all-reduce follows the replay
         graphs = [parallel.GraphedStep(fn, device) for fn in locals_]
+        # a capture's outputs are its graph's own buffers, rewritten by every replay (eager steps rebind fn.outputs)
+        captured = [fn.outputs for fn in locals_]
 
         def step_graphed():
             turn['graph'] = (turn['graph'] + 1) % copies
             out = graphs[turn['graph']]()
             return reducer.reduce() if reducer is not None else out
-        return step_graphed, step_eager, x, xp, copies
+        return step_graphed, step_eager, x, xp, copies, lambda: in_generator_order(captured[turn['graph']])
 
     # ---- device-resident throughput (value): both batch orders, the configured one is the headline ----------
     orders = {}
     sampler = ClockSampler(dev_index)
     for order in (['natural', 'cost'] if args.order == 'cost' else ['cost', 'natural']):   # headline order last
-        step, step_eager, x, xp, input_copies = make_step(order)
-        ms_eager, _ = timed(step_eager, args.steps, max(args.warmup, 3))
+        step, step_eager, x, xp, input_copies, last_outputs = make_step(order)
+        ms_eager = timed(step_eager, args.steps, max(args.warmup, 3))
         headline = order == args.order
         if headline and rank == 0:
             sampler.start()
-        ms_step, n_timed = timed(step, args.steps, max(args.warmup, 3), min_ms=1000.0 if headline else 200.0)
+        ms_step = timed(step, args.steps, max(args.warmup, 3))
         if headline:
             clocks = sampler.stop() if rank == 0 else None
+            if args.dump_outputs is not None:
+                dump_outputs(args.dump_outputs, *last_outputs(), [n for n, _ in system.named_parameters()])
         orders[order] = {'ms_per_step': ms_step, 'value': Bg / (ms_step * 1e-3), 'eager_ms_per_step': ms_eager,
-                         'timed_steps': n_timed}
+                         'timed_steps': args.steps}
     if comm is not None:
         comm.check()
     ms_step, value = orders[args.order]['ms_per_step'], orders[args.order]['value']
@@ -676,7 +719,8 @@ def main():
             dist.all_reduce(flat)
             out_host.copy_(flat, non_blocking=True)
             torch.cuda.current_stream().synchronize()      # the user reads the loss / gradients on the host
-    ms_e2e, _ = timed(step_e2e, max(3, args.steps // 2), 3, min_ms=300.0)
+    # an end-to-end step lasts ~12 device-resident steps (the PCIe copy of the batch): a tenth of the steps keeps the window
+    ms_e2e = timed(step_e2e, max(3, args.steps // 10), 3)
     e2e_value = Bg / (ms_e2e * 1e-3)
     h2d = 2 * B * 13 * x.element_size()
     d2h = out_host.numel() * 8
@@ -692,7 +736,7 @@ def main():
             for p in params:
                 p.grad = None
             system.contactnets_loss(xv, None, xpv).mean().backward()
-        ms_views, _ = timed(step_views, args.steps, 3)
+        ms_views = timed(step_views, args.steps, 3)
         strided = {'ms_per_step_eager': ms_views, 'contiguous_eager_ms_per_step': orders[args.order]['eager_ms_per_step'],
                    'note': 'row strides go through the ABI (dpll_cube_loss_leaf_dp_*): no .contiguous() copy'}
 
@@ -705,7 +749,7 @@ def main():
 
     def kernel_only():
         ops.cube_loss_leaf_dp_raw(x, xp, *leaves, DT, 1e-3, flags=flags)
-    ms_kernel, _ = timed(kernel_only, args.steps, 3, min_ms=200.0)
+    ms_kernel = timed(kernel_only, args.steps, 3)
     flops_per_sample = F0_CUBE + FIT_CUBE * mean_iters
     achieved_tflops = B * flops_per_sample / (ms_kernel * 1e-3) / 1e12
     sms = torch.cuda.get_device_properties(device).multi_processor_count

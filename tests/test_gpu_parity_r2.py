@@ -55,6 +55,31 @@ def test_bench_batch_subset_matches_oracle():
     assert max_rel_to_scale(gl, P.length_params[0].grad.numpy()) < 1e-9
 
 
+@pytest.mark.parametrize('mode', [['--order', 'cost'], ['--order', 'natural', '--no-graph']])
+def test_bench_dump_outputs_are_the_last_timed_step(mode, tmp_path):
+    """bench.py --dump-outputs writes the per-sample losses (in generator order), the mean loss and the gradients of a
+    timed step (every step computes the same values, so which one is not checked): the same as the public API's on the
+    same seeded batch.  20,000 pairs fit the L2, so the graphed run cycles through many captured copies of the batch."""
+    import json
+    import subprocess
+    sys.path.insert(0, ROOT)
+    import bench
+    run = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '3', '--warmup', '1', '--batch', '20000',
+                          '--no-secondary', '--no-cpu-baseline', '--dump-outputs', str(tmp_path)] + mode,
+                         check=True, stdout=subprocess.PIPE, text=True)
+    assert json.loads(run.stdout)['config']['timed_steps'] == 3
+    system = bench.make_system(torch.device(DEV), torch.float64)
+    x, xp = bench.make_batch(system, 20000, seed=0, device=torch.device(DEV), dtype=torch.float64)
+    loss = system.contactnets_loss(x, None, xp)
+    mean = loss.mean()
+    mean.backward()
+    assert rel_err(np.load(tmp_path / 'loss.npy'), loss.detach().cpu().numpy(), 1e-9).max() < 1e-12
+    assert rel_err(np.load(tmp_path / 'loss_mean.npy'), mean.item()) < 1e-12
+    for name, p in system.named_parameters():
+        got = np.load(tmp_path / f'grad.{name}.npy')
+        assert got.dtype == np.float64 and max_rel_to_scale(got, p.grad.cpu().numpy()) < 1e-12, name
+
+
 def _elbow_random(n, assets_dir, seed):
     from dair_pll_b200.inertia import InertialParameterConverter as IPC
     pi, fr, half = synthetic.elbow_learnables_perturbed(seed)

@@ -428,3 +428,30 @@ def test_mixed_box_and_mesh_elbow_parses(assets_dir):
     names = [k for k, _ in s.named_parameters()]
     assert 'multibody_terms.contact_terms.geometries.0.length_params' in names
     assert 'multibody_terms.contact_terms.geometries.1.network.output_weight' in names
+
+
+def test_bench_dump_outputs_files_and_row_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float .npy per output; above DUMP_MAX_ROWS per-sample losses the same seeded,
+    ordered subset of rows is written on every run."""
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_MAX_ROWS', 5)
+    loss = torch.arange(12, dtype=torch.float64)
+    grads = [torch.ones(1, 10, dtype=torch.float64), torch.zeros(2, dtype=torch.float64)]
+    for out in (tmp_path / 'a', tmp_path / 'b'):
+        bench.dump_outputs(str(out), loss, loss.mean(), grads, ['p.first', 'p.second'])
+    assert sorted(os.listdir(tmp_path / 'a')) == ['grad.p.first.npy', 'grad.p.second.npy', 'loss.npy', 'loss_mean.npy']
+    rows = np.load(tmp_path / 'a' / 'loss.npy')
+    assert rows.dtype == np.float64 and rows.shape == (5,) and np.all(np.diff(rows) > 0) and set(rows) <= set(range(12))
+    assert np.array_equal(rows, np.load(tmp_path / 'b' / 'loss.npy'))
+    assert np.load(tmp_path / 'a' / 'loss_mean.npy') == 5.5
+    assert np.array_equal(np.load(tmp_path / 'a' / 'grad.p.first.npy'), np.ones((1, 10)))
+
+
+@pytest.mark.parametrize('argv', [['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'out']])
+def test_bench_refuses_arguments_it_cannot_honour(argv, monkeypatch):
+    """No timed step to report, or a dump the CPU reference path would not write: refused before any work."""
+    import bench
+    monkeypatch.setattr('sys.argv', ['bench.py'] + argv)
+    with pytest.raises(SystemExit) as e:
+        bench.parse_args()
+    assert e.value.code == 2
