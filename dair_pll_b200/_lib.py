@@ -9,7 +9,7 @@ import os
 from dair_pll_b200 import build as _build
 
 _LIB = None
-ABI_VERSION = 212        # DPLL_VERSION of include/dair_pll_b200.h this binding was written against
+ABI_VERSION = 213        # DPLL_VERSION of include/dair_pll_b200.h this binding was written against
 
 _c_void_p = ctypes.c_void_p
 _i64, _i32, _f64, _f32, _sz = ctypes.c_int64, ctypes.c_int32, ctypes.c_double, ctypes.c_float, ctypes.c_size_t
@@ -42,11 +42,8 @@ EXPORTS = {
     'dpll_cube_rollout_grad_f64': ([_c_void_p] * 4 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
     'dpll_cube_rollout_saved_f64': ([_c_void_p] * 4 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 3, ctypes.c_int),
     'dpll_cube_rollout_backward_f64': ([_c_void_p] * 5 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_elbow_rollout_grad_f64': ([_c_void_p] * 5 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_elbow_loss_f64': ([_c_void_p] * 8 + [_f64, _f64, _i64] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_elbow_loss_f32': ([_c_void_p] * 8 + [_f32, _f32, _i64] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_elbow_loss_ex_f64': ([_c_void_p] * 8 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_elbow_loss_ex_f32': ([_c_void_p] * 8 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
+    'dpll_elbow_loss_f64': ([_c_void_p] * 8 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
+    'dpll_elbow_loss_f32': ([_c_void_p] * 8 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
     'dpll_elbow_rollout_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
     'dpll_elbow_rollout_f32': ([_c_void_p] * 6 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
     'dpll_icnn_input_f64': ([_c_void_p, _c_void_p, _i64, _i32, _f64, _c_void_p, _c_void_p], ctypes.c_int),

@@ -81,17 +81,6 @@ template <typename T> struct CubeProb {
   CN_HD T& rho(int k) const { return p[(9 + k) * s]; }   // world lever arms, 3 per contact
   CN_HD T& q(int k) const { return p[(21 + k) * s]; }    // QP linear term, sappy order [tx,ty,n] per contact
 };
-// Read-only view of a record held in another precision (U), converted to T on every read: the single-precision Newton
-// visits of the mixed-precision solver read the double-precision slot through it.  The solver functions below take the
-// view type as a deduced template parameter PV.
-template <typename T, typename U> struct CubeProbCvt {
-  const U* p;
-  int s;
-  CN_HD T IW(int i) const { return T(p[i * s]); }
-  CN_HD T mcW(int i) const { return T(p[(6 + i) * s]); }
-  CN_HD T rho(int k) const { return T(p[(9 + k) * s]); }
-  CN_HD T q(int k) const { return T(p[(21 + k) * s]); }
-};
 
 // [aw; av] = M^-1 [tau; frc]  (tau, aw body frame; frc, av world frame); Schur complement = I_sym.
 template <typename T>
@@ -107,8 +96,8 @@ CN_HD void cube_minv(const CubeParams<T>& P, const T* R, const T* tau, const T* 
 }
 
 // u^ -> M^ u^ in world-twist coordinates
-template <typename T, typename PV>
-CN_HD void cube_mass_mul(const CubeParams<T>& P, const PV& S, const T* u, T* o) {
+template <typename T>
+CN_HD void cube_mass_mul(const CubeParams<T>& P, const CubeProb<T>& S, const T* u, T* o) {
   const T I0 = S.IW(0), I1 = S.IW(1), I2 = S.IW(2), I3 = S.IW(3), I4 = S.IW(4), I5 = S.IW(5);
   const T mc[3] = {S.mcW(0), S.mcW(1), S.mcW(2)};
   T b[3], c[3];
@@ -217,8 +206,8 @@ CN_HD void cube_free_accel(const CubeParams<T>& P, const T* R, const T* wB, T* a
 }
 
 // residual of contact c at twist u:  r = D_mu (u_w x rho_c + u_v) + q_c
-template <typename T, typename PV>
-CN_HD void cube_contact_residual(const CubeParams<T>& P, const PV& S, int c, const T* u, T* rho, T* r) {
+template <typename T>
+CN_HD void cube_contact_residual(const CubeParams<T>& P, const CubeProb<T>& S, int c, const T* u, T* rho, T* r) {
   rho[0] = S.rho(3 * c); rho[1] = S.rho(3 * c + 1); rho[2] = S.rho(3 * c + 2);
   T e[3];
   cross3(u, rho, e);
@@ -230,8 +219,8 @@ CN_HD void cube_contact_residual(const CubeParams<T>& P, const PV& S, int c, con
 // Gradient (and optionally Hessian) of the primal objective at u (world twist).
 //   g = M u - sum_c J_c^T f~_c ;  H = M + sum_c J_c^T K_c J_c   (H: full 6x6 row-major, lower part)
 // Also returns the scaled norms used by the stopping test.
-template <typename T, bool WANT_H, int UNR, typename PV>
-CN_HD void cube_eval(const CubeParams<T>& P, const PV& S, const T* u, T* g, T* H, T& res2, T& scale2) {
+template <typename T, bool WANT_H, int UNR>
+CN_HD void cube_eval(const CubeParams<T>& P, const CubeProb<T>& S, const T* u, T* g, T* H, T& res2, T& scale2) {
   T Mu[6];
   cube_mass_mul(P, S, u, Mu);
   T z[6] = {T(0), T(0), T(0), T(0), T(0), T(0)};
@@ -321,8 +310,8 @@ template <typename T> struct CubeTrial {
 // finishes without the confirming evaluation.
 //   it: bits 0-7 Newton directions taken, 8-15 trials on the pending direction (0xff = forced
 //   accept), 16+ rounding-floor counter.  Returns NEWTON_DONE or NEWTON_CONTINUE.
-template <typename T, int UNR, typename PV>
-CN_HD int cube_newton_visit(const CubeParams<T>& P, const PV& S, const SolverCfg<T>& cfg, T* u, T* d,
+template <typename T, int UNR>
+CN_HD int cube_newton_visit(const CubeParams<T>& P, const CubeProb<T>& S, const SolverCfg<T>& cfg, T* u, T* d,
                             T& d0, T& best_res2, CubeTrial<T>& tr, int& it) {
   T g[6], H[36], res2, scale2;
   CN_STAT_UNIT();
@@ -401,55 +390,6 @@ CN_HD int cube_solve(const CubeParams<T>& P, const CubeProb<T>& S, const SolverC
     while (cube_newton_visit<T, UNR>(P, S, cfg, u, d, d0, best, tr, it) != NEWTON_DONE) {}
   }
   return it & 0xff;
-}
-
-// ---------------------------------------------------------------------------
-// Mixed-precision solve (EXPERIMENT, measured and not shipped in the kernels -- DESIGN.md section 9,
-// profiles/r2_exp_mixed_precision.txt).  The optimum is unique and the Newton iteration is self-correcting, so the visits that
-// only have to FIND the cone case of every contact and get within ~1e-4 of the optimum can run in single precision; the
-// double-precision iteration started from that point then needs two visits (one step and the final step) in 89% of the
-// solves of the bench batch and three in 11% -- measured on the CPU with this very code (tools/exp_mixed.cpp): 7.41 double
-// visits per solve become 6.25 single + 2.11 double, the optima differ by < 1e-11 relative.  Stage 1 stops on its own
-// (looser) tolerances, or after CN_MIXED_VISIT_CAP visits when single-precision rounding keeps it from settling (0.07% of
-// the solves).  On the B200 a single-precision visit turned out to cost what a double-precision one does (both are bound by
-// dependent-issue latency at two warps per sub-partition, not by the FP64 pipe), so the wavefront kernel stays all-double.
-// ---------------------------------------------------------------------------
-#ifndef CN_MIXED_VISIT_CAP
-#define CN_MIXED_VISIT_CAP 40
-#endif
-CN_HD SolverCfg<float> mixed_stage_cfg() { return {1e-4f, 1e-2f, 0.9f, 25, 1e-3f, false}; }
-
-// the fields the Newton visit reads (mu, inv_eps, m, dscale), and the rest for completeness
-template <typename T> CN_HD void cube_params_to_float(const CubeParams<T>& P, CubeParams<float>& F) {
-  F.m = float(P.m); F.mu = float(P.mu); F.dt = float(P.dt); F.eps = float(P.eps); F.inv_eps = float(P.inv_eps);
-  F.grav = float(P.grav); F.inv_m = float(P.inv_m);
-  for (int i = 0; i < 3; ++i) { F.c[i] = float(P.c[i]); F.h[i] = float(P.h[i]); }
-  for (int i = 0; i < 6; ++i) {
-    F.Isym[i] = float(P.Isym[i]); F.Io[i] = float(P.Io[i]); F.Isym_inv[i] = float(P.Isym_inv[i]);
-    F.dscale[i] = float(P.dscale[i]);
-  }
-}
-
-// Stage 1 + stage 2 for one sample.  u: in start point, out optimum.  Returns single + double directions taken;
-// visits[0], visits[1] (nullable): evaluations spent in each stage.
-template <typename T, int UNR>
-CN_HD int cube_solve_mixed(const CubeParams<T>& P, const CubeProb<T>& S, const SolverCfg<T>& cfg, T* u, int* visits = nullptr) {
-  CubeParams<float> Pf;
-  cube_params_to_float(P, Pf);
-  const SolverCfg<float> cfgf = mixed_stage_cfg();
-  const CubeProbCvt<float, T> Sf{S.p, S.s};
-  float uf[6], df[6], d0f = 0.f, bestf = -1.f;
-  CubeTrial<float> trf{1.f, 0.f, 1.f};
-  int itf = 0, nv = 0;
-  for (int i = 0; i < 6; ++i) uf[i] = float(u[i]);
-  while (cube_newton_visit<float, UNR>(Pf, Sf, cfgf, uf, df, d0f, bestf, trf, itf) != NEWTON_DONE && ++nv < CN_MIXED_VISIT_CAP) {}
-  for (int i = 0; i < 6; ++i) u[i] = T(uf[i]);
-  T d[6], d0 = T(0), best = T(-1);
-  CubeTrial<T> tr{T(1), T(0), T(1)};
-  int it = 0, nv2 = 1;
-  while (cube_newton_visit<T, UNR>(P, S, cfg, u, d, d0, best, tr, it) != NEWTON_DONE) ++nv2;
-  if (visits) { visits[0] = nv + 1; visits[1] = nv2; }
-  return (itf & 0xff) + (it & 0xff);
 }
 
 // ---------------------------------------------------------------------------

@@ -76,9 +76,7 @@ template <typename T> struct ElbowKin {
 };
 
 // View of the per-sample quantities that stay fixed during the Newton solve: element k of the 121-field record
-// at p[k * s].  s = 1 over a local array; s = block size over a thread-interleaved shared-memory array (the
-// two-phase loss kernel: the record is read on every Newton visit, and as a per-thread local array it
-// overflows L1 -- ncu: 41% of the stall samples on local loads).
+// at p[k * s].  Every user holds the record in a per-thread local array (s = 1).
 constexpr int ELBOW_PROB_FIELDS = 121;
 template <typename T> struct ElbowProb {
   T* p;
@@ -579,33 +577,13 @@ CN_HD T elbow_loss_sample(const ElbowParams<T>& P, const SolverCfg<T>& cfg, cons
   return elbow_loss_epilogue(P, S, A, u, grad, force_out, grad ? grad_pts : (T*)nullptr);
 }
 
-// The same loss path for the two-phase kernel: `solve` = false is the triage pass -- a sample that needs the solver
-// is left untouched (returns false); `solve` = true runs the full path.  One code instance serves both passes.
-template <typename T>
-CN_HD bool elbow_loss_sample_phase(const ElbowParams<T>& P, const SolverCfg<T>& cfg, bool solve, const ElbowProb<T>& S,
-                                   const T* x, const T* xp, const T* pts, T* grad, T* force_out, T* grad_pts,
-                                   int* iters_out, T* loss_out) {
-  ElbowLossAux<T> A;
-  elbow_loss_prologue(P, x, xp, pts, S, A);
-  if (!solve && !elbow_trivially_solved(S)) return false;
-  T u[7] = {T(0), T(0), T(0), T(0), T(0), T(0), T(0)};
-  const int it = elbow_solve(P, S, cfg, u);            // returns at once for a trivially solved sample
-  if (iters_out) *iters_out = it;
-  if (!grad && grad_pts) for (int i = 0; i < 24; ++i) grad_pts[i] = T(0);
-  *loss_out = elbow_loss_epilogue(P, S, A, u, grad, force_out, grad ? grad_pts : (T*)nullptr);
-  return true;
-}
-
 // ---------------------------------------------------------------------------
 // learnable time step
 // ---------------------------------------------------------------------------
 template <typename T>
 CN_HD int elbow_step_sample(const ElbowParams<T>& P, const SolverCfg<T>& cfg, const T* x, const T* pts, T* xn,
-                            T* force_out, T* u_out = nullptr, const T* u_fixed = nullptr) {
-  // u_out: receives the QP optimum u* (world twist + hinge rate; v+ = v- + u*).  u_fixed: the optimum is KNOWN (kept by the
-  // forward rollout): instead of solving, take ONE Newton step at it.  In plain arithmetic that changes nothing; in
-  // dual-number arithmetic with u_fixed entered as a constant the step's tangent is -H(u*)^-1 dg/d(direction) -- the
-  // implicit-function derivative of the solve -- at the cost of one evaluation instead of a whole dual-number solve.
+                            T* force_out, T* u_out = nullptr) {
+  // u_out: receives the QP optimum u* (world twist + hinge rate; v+ = v- + u*).
   T store[ELBOW_PROB_FIELDS];
   const ElbowProb<T> S{store, 1};
   ElbowKin<T> K;
@@ -628,20 +606,7 @@ CN_HD int elbow_step_sample(const ElbowParams<T>& P, const SolverCfg<T>& cfg, co
     S.q(3 * c + 2) = e[2] + (S.rho(3 * c + 2) + x[6]) * inv_dt;
   }
   T u[7] = {T(0), T(0), T(0), T(0), T(0), T(0), T(0)};
-  int it = 0;
-  if (u_fixed) {
-    for (int i = 0; i < 7; ++i) u[i] = u_fixed[i];
-    if (!elbow_trivially_solved(S)) {
-      T g[7], H[49], res2, scale2, inv_diag[7], ng[7], d[7];
-      elbow_eval<T, true>(P, S, u, g, H, res2, scale2);
-      chol_factor<T, 7>(H, inv_diag);
-      for (int i = 0; i < 7; ++i) ng[i] = -g[i];
-      chol_solve<T, 7>(H, inv_diag, ng, d);
-      for (int i = 0; i < 7; ++i) u[i] += d[i];
-    }
-  } else {
-    it = elbow_solve(P, S, cfg, u);
-  }
+  const int it = elbow_solve(P, S, cfg, u);
   if (u_out) for (int i = 0; i < 7; ++i) u_out[i] = u[i];
   if (force_out)
     for (int c = 0; c < EL_NC; ++c) {

@@ -785,7 +785,8 @@ template <typename T>
 CN_HD int elbow_step_sample_wf(const ElbowParams<T>& P, const SolverCfg<T>& cfg, const T* x, const T* pts, T* xn,
                                T* force_out, T* u_out, const T* u_fixed = nullptr) {
   // u_fixed: the optimum is known (kept by the forward rollout) and entered as a constant; ONE Newton step at it then
-  // carries, in dual-number arithmetic, the implicit-function derivative of the solve (see elbow_step_sample, cn_elbow.cuh)
+  // carries, in dual-number arithmetic, the implicit-function derivative of the solve, -H(u*)^-1 dg/d(direction), at the
+  // cost of one evaluation instead of a whole dual-number solve (in plain arithmetic the step changes nothing)
   T store[EW_REC];
   const ElbowRec<T> S{store, 1};
   ElbowSetup<T> E;

@@ -720,7 +720,8 @@ cube_terms_kernel(const IO* __restrict__ q, const IO* __restrict__ v, const IO* 
 }
 
 // ---------------------------------------------------------------------------
-// Elbow (floating base + hinge, 8 contacts): one sample per thread, problem in thread-local arrays.
+// Elbow (floating base + hinge, 8 contacts): the loss kernel is the wavefront kernel in cn_elbow_wf.cu; rollout
+// and terms run one sample per thread, problem in thread-local arrays.
 // ---------------------------------------------------------------------------
 constexpr int kNAccE = 32;   // 28 parameter gradients + loss sum + pad
 
@@ -733,138 +734,6 @@ __device__ __forceinline__ void load_elbow_params(cn::ElbowParams<T>& P, const I
   for (int i = 0; i < 6; ++i) h[i] = half ? T(half[i]) : T(0);
   for (int i = 0; i < cn::EL_NKIN; ++i) kn[i] = T(kin[i]);
   cn::elbow_params_init(P, in, m, h, kn, dt, eps);
-}
-
-template <typename T, typename IO>
-__global__ void __launch_bounds__(kLossThreads)
-elbow_loss_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const IO* __restrict__ weight,
-                  const IO* __restrict__ inertia, const IO* __restrict__ mu, const IO* __restrict__ half,
-                  const IO* __restrict__ kin, const IO* __restrict__ pts, T dt, T eps, int64_t B, IO* __restrict__ loss,
-                  IO* __restrict__ force, IO* __restrict__ grad_pts, int32_t* __restrict__ iters,
-                  T* __restrict__ partials, int want_grad, const int32_t* __restrict__ skip_flag) {
-  if (skip_flag && *skip_flag) return;
-  cn::ElbowParams<T> P;
-  load_elbow_params<T, IO>(P, inertia, mu, half, kin, dt, eps);
-  const cn::SolverCfg<T> cfg = cn::default_cfg<T>();
-  T acc[kNAccE];
-  for (int i = 0; i < kNAccE; ++i) acc[i] = T(0);
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += stride) {
-    T xs[15], xps[15], gs[DPLL_ELBOW_NPARAM], fo[24], pt[24], gp[24];
-    for (int i = 0; i < 15; ++i) { xs[i] = T(x[b * 15 + i]); xps[i] = T(xp[b * 15 + i]); }
-    if (pts) for (int i = 0; i < 24; ++i) pt[i] = T(pts[b * 24 + i]);
-    for (int i = 0; i < DPLL_ELBOW_NPARAM; ++i) gs[i] = T(0);
-    int it;
-    const T l = cn::elbow_loss_sample<T>(P, cfg, xs, xps, pts ? pt : (const T*)nullptr, want_grad ? gs : (T*)nullptr,
-                                         force ? fo : (T*)nullptr, grad_pts ? gp : (T*)nullptr, &it);
-    if (force) for (int i = 0; i < 24; ++i) force[b * 24 + i] = IO(fo[i]);
-    const T w = weight ? T(weight[b]) : T(1);
-    if (grad_pts) for (int i = 0; i < 24; ++i) grad_pts[b * 24 + i] = IO(w * gp[i]);
-    for (int i = 0; i < DPLL_ELBOW_NPARAM; ++i) acc[i] += w * gs[i];
-    if (loss) loss[b] = IO(l);
-    acc[DPLL_ELBOW_NPARAM] += l;
-    if (iters) iters[b] = it;
-  }
-  if (!partials) return;
-  __shared__ T red[kLossThreads / 32][kNAccE];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int i = 0; i < kNAccE; ++i) {
-    const T s = warp_sum(acc[i]);
-    if (lane == 0) red[warp][i] = s;
-  }
-  __syncthreads();
-  if (threadIdx.x < kNAccE) {
-    T s = T(0);
-    for (int w = 0; w < kLossThreads / 32; ++w) s += red[w][threadIdx.x];
-    partials[(int64_t)blockIdx.x * kNAccE + threadIdx.x] = s;
-  }
-}
-
-// Two-phase variant of the elbow loss kernel.  62% of a toss data set is free flight and the others need 4 .. 36
-// Newton visits, so with one sample per thread a warp waits for its slowest lane while two thirds of its lanes
-// have nothing to solve (sorting the batch by iteration count makes the simple kernel 2.1x faster,
-// tools/elbow_sort_exp.py).  Here each warp alternates two warp-uniform passes over its static sample range:
-//   triage  the next 32 samples: build the problem; free flight is finalised on the spot, the others only push
-//           their index into a per-warp list (shared memory);
-//   solve   32 listed samples, one per lane: the full path (problem, Newton solve, loss + backward).
-// Every lane of a solve pass has work, and the per-sample code is the one instance of elbow_loss_sample_phase.
-constexpr int kElbowList = 64;
-template <typename T, typename IO>
-__global__ void __launch_bounds__(kLossThreads)
-elbow_loss_2p_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const IO* __restrict__ weight,
-                     const IO* __restrict__ inertia, const IO* __restrict__ mu, const IO* __restrict__ half,
-                     const IO* __restrict__ kin, const IO* __restrict__ pts, T dt, T eps, int64_t B, IO* __restrict__ loss,
-                     IO* __restrict__ force, IO* __restrict__ grad_pts, int32_t* __restrict__ iters,
-                     T* __restrict__ partials, int want_grad, const int32_t* __restrict__ skip_flag) {
-  if (skip_flag && *skip_flag) return;
-  __shared__ int32_t list[kLossThreads / 32][kElbowList];
-  cn::ElbowParams<T> P;
-  load_elbow_params<T, IO>(P, inertia, mu, half, kin, dt, eps);
-  const cn::SolverCfg<T> cfg = cn::default_cfg<T>();
-  T acc[kNAccE];
-  for (int i = 0; i < kNAccE; ++i) acc[i] = T(0);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const unsigned lt_mask = (1u << lane) - 1u;
-  const int64_t gw = (int64_t)blockIdx.x * (kLossThreads / 32) + warp, W = (int64_t)gridDim.x * (kLossThreads / 32);
-  const int64_t base = B / W, rem = B % W;
-  const int64_t lo = gw * base + (gw < rem ? gw : rem);
-  const int64_t hi = lo + base + (gw < rem ? 1 : 0);
-  int64_t next = lo;
-  int n_list = 0, h_list = 0;
-  while (next < hi || n_list > 0) {
-    const bool solve = n_list >= 32 || next >= hi;       // warp-uniform
-    int64_t b = -1;
-    if (solve) {
-      const int k = n_list < 32 ? n_list : 32;
-      if (lane < k) b = lo + list[warp][(h_list + lane) % kElbowList];
-      h_list = (h_list + k) % kElbowList; n_list -= k;
-    } else {
-      if (next + lane < hi) b = next + lane;
-      next += (hi - next < 32 ? hi - next : 32);
-    }
-    bool push = false;
-    if (b >= 0) {
-      T xs[15], xps[15], gs[DPLL_ELBOW_NPARAM], fo[24], pt[24], gp[24];
-      for (int i = 0; i < 15; ++i) { xs[i] = T(x[b * 15 + i]); xps[i] = T(xp[b * 15 + i]); }
-      if (pts) for (int i = 0; i < 24; ++i) pt[i] = T(pts[b * 24 + i]);
-      for (int i = 0; i < DPLL_ELBOW_NPARAM; ++i) gs[i] = T(0);
-      int it = 0;
-      T l = T(0);
-      T store[cn::ELBOW_PROB_FIELDS];        // problem record (measured: thread-interleaved shared memory at 6 warps
-      const cn::ElbowProb<T> S{store, 1};     // per SM is 1.6x slower than this local array at 8 warps per SM)
-      const bool done = cn::elbow_loss_sample_phase<T>(P, cfg, solve, S, xs, xps, pts ? pt : (const T*)nullptr,
-                                                       want_grad ? gs : (T*)nullptr, force ? fo : (T*)nullptr,
-                                                       grad_pts ? gp : (T*)nullptr, &it, &l);
-      if (done) {
-        if (force) for (int i = 0; i < 24; ++i) force[b * 24 + i] = IO(fo[i]);
-        const T w = weight ? T(weight[b]) : T(1);
-        if (grad_pts) for (int i = 0; i < 24; ++i) grad_pts[b * 24 + i] = IO(w * gp[i]);
-        for (int i = 0; i < DPLL_ELBOW_NPARAM; ++i) acc[i] += w * gs[i];
-        if (loss) loss[b] = IO(l);
-        acc[DPLL_ELBOW_NPARAM] += l;
-        if (iters) iters[b] = it;
-      } else {
-        push = true;
-      }
-    }
-    __syncwarp();
-    const unsigned m_push = __ballot_sync(0xffffffffu, push);
-    if (push) list[warp][(h_list + n_list + __popc(m_push & lt_mask)) % kElbowList] = (int32_t)(b - lo);
-    n_list += __popc(m_push);
-    __syncwarp();
-  }
-  if (!partials) return;
-  __shared__ T red[kLossThreads / 32][kNAccE];
-  for (int i = 0; i < kNAccE; ++i) {
-    const T s = warp_sum(acc[i]);
-    if (lane == 0) red[warp][i] = s;
-  }
-  __syncthreads();
-  if (threadIdx.x < kNAccE) {
-    T s = T(0);
-    for (int w = 0; w < kLossThreads / 32; ++w) s += red[w][threadIdx.x];
-    partials[(int64_t)blockIdx.x * kNAccE + threadIdx.x] = s;
-  }
 }
 
 template <typename T, typename IO>
@@ -922,10 +791,10 @@ elbow_terms_kernel(const IO* __restrict__ q, const IO* __restrict__ v, const IO*
 }
 
 template <typename T, typename IO>
-int launch_elbow_loss(int variant, const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
+int launch_elbow_loss(const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
                       const IO* kin, const IO* pts, T dt, T eps, int64_t B, IO* loss, IO* force, IO* grad_pts,
                       int32_t* iters, IO* grad, IO* loss_sum,
-                      const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream, int flags = 0) {
+                      const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream, int flags) {
   if (B < 0 || !inertia || !mu || (!half && !pts) || !kin || (grad_pts && (!pts || !grad))) return DPLL_EINVAL;
   if (B > 0 && (!x || !xp)) return DPLL_EINVAL;
   const bool want_red = grad || loss_sum;
@@ -933,42 +802,19 @@ int launch_elbow_loss(int variant, const IO* x, const IO* xp, const IO* weight, 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const DeviceInfo di = device_info();
   T* partials = want_red ? static_cast<T*>(workspace) : nullptr;
-  int blocks;
-  if (variant == 0) {
-    // wavefront kernel (default): per-visit scheduling over shared-memory records
-    int err = DPLL_OK;
-    unsigned long long* dyn = nullptr;
-    if (flags & DPLL_LOSS_DYNAMIC) {
-      if (!workspace || workspace_bytes < dpll_workspace_bytes()) return DPLL_EWORKSPACE;
-      dyn = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + kWsQueueOffset);
-      cudaError_t em = cudaMemsetAsync(dyn, 0, kWsQueueBytes, st);
-      if (em != cudaSuccess) return (int)em;
-    }
-    blocks = ::launch_elbow_loss_wf<T, IO>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B, loss, force, grad_pts,
-                                         iters, partials, grad ? 1 : 0, skip_flag, di.sms, st, &err, dyn);
-    if (err != DPLL_OK) return err;
-  } else {
-    const bool two_phase = variant != 1;          // 1 = one sample per thread, 2 = triage / solve passes (A/B measurements)
-    int per_sm = 0;
-    if (two_phase) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, elbow_loss_2p_kernel<T, IO>, kLossThreads, 0);
-    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, elbow_loss_kernel<T, IO>, kLossThreads, 0);
-    if (per_sm < 1) per_sm = 1;
-    // two-phase: a warp wants a few solve passes' worth of samples (>= 128) to fill its lanes
-    const int64_t per_block = two_phase ? (int64_t)(kLossThreads / 32) * 128 : kLossThreads;
-    int64_t need = (B + per_block - 1) / per_block;
-    int64_t cap = (int64_t)di.sms * per_sm;
-    if (cap > kMaxBlocks) cap = kMaxBlocks;
-    blocks = (int)(need < cap ? need : cap);
-    if (blocks < 1) blocks = 1;
-    if (two_phase)
-      elbow_loss_2p_kernel<T, IO><<<blocks, kLossThreads, 0, st>>>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B,
-                                                                  loss, force, grad_pts, iters, partials, grad ? 1 : 0,
-                                                                  skip_flag);
-    else
-      elbow_loss_kernel<T, IO><<<blocks, kLossThreads, 0, st>>>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B,
-                                                               loss, force, grad_pts, iters, partials, grad ? 1 : 0,
-                                                               skip_flag);
+  // wavefront kernel: per-visit scheduling over shared-memory records
+  int err = DPLL_OK;
+  unsigned long long* dyn = nullptr;
+  if (flags & DPLL_LOSS_DYNAMIC) {
+    if (!workspace || workspace_bytes < dpll_workspace_bytes()) return DPLL_EWORKSPACE;
+    dyn = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + kWsQueueOffset);
+    cudaError_t em = cudaMemsetAsync(dyn, 0, kWsQueueBytes, st);
+    if (em != cudaSuccess) return (int)em;
   }
+  const int blocks = ::launch_elbow_loss_wf<T, IO>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B, loss, force,
+                                                   grad_pts, iters, partials, grad ? 1 : 0, skip_flag, di.sms, st, &err,
+                                                   dyn);
+  if (err != DPLL_OK) return err;
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;
   if (want_red) {
@@ -1158,8 +1004,9 @@ int launch_cube_rollout(const IO* x0, const IO* inertia, const IO* mu, const IO*
 
 extern "C" {
 
-// Kernel variant selector for A/B measurements (0 = wavefront, static ranges [default, deterministic];
+// Cube loss kernel selector for A/B measurements (0 = wavefront, static ranges [default, deterministic];
 // 1 = one sample per thread; 2 = wavefront with dynamic sample distribution [not bitwise reproducible]).
+// The elbow loss always runs its wavefront kernel.
 static int g_loss_variant = 0;
 int dpll_set_loss_variant(int variant) {
   if (variant < 0 || variant > 2) return DPLL_EINVAL;
@@ -1328,39 +1175,23 @@ int dpll_elbow_terms_f64(const double* q, const double* v, const double* inertia
 }
 
 int dpll_elbow_loss_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
-                        const double* mu_pair, const double* half, const double* kin, const double* pts, double dt, double eps,
-                        int64_t B, double* loss, double* force, double* grad_pts, int32_t* iters, double* grad, double* loss_sum,
-                        const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream) {
-  return launch_elbow_loss<double, double>(g_loss_variant, x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, loss, force,
-                                           grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream);
-}
-
-int dpll_elbow_loss_ex_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
-                           const double* mu_pair, const double* half, const double* kin, const double* pts, double dt,
-                           double eps, int64_t B, int32_t flags, double* loss, double* force, double* grad_pts,
-                           int32_t* iters, double* grad, double* loss_sum, const int32_t* skip_flag, void* workspace,
-                           size_t workspace_bytes, void* stream) {
-  return launch_elbow_loss<double, double>(g_loss_variant == 2 ? 2 : (g_loss_variant == 1 ? 1 : 0), x, x_plus, weight, inertia,
-                                           mu_pair, half, kin, pts, dt, eps, B, loss, force, grad_pts, iters, grad, loss_sum,
-                                           skip_flag, workspace, workspace_bytes, stream, flags);
-}
-
-int dpll_elbow_loss_ex_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
-                           const float* mu_pair, const float* half, const float* kin, const float* pts, float dt, float eps,
-                           int64_t B, int32_t flags, float* loss, float* force, float* grad_pts, int32_t* iters, float* grad,
-                           float* loss_sum, const int32_t* skip_flag, void* workspace, size_t workspace_bytes,
-                           void* stream) {
-  return launch_elbow_loss<double, float>(g_loss_variant == 2 ? 2 : (g_loss_variant == 1 ? 1 : 0), x, x_plus, weight, inertia,
-                                          mu_pair, half, kin, pts, (double)dt, (double)eps, B, loss, force, grad_pts, iters,
-                                          grad, loss_sum, skip_flag, workspace, workspace_bytes, stream, flags);
+                        const double* mu_pair, const double* half, const double* kin, const double* pts, double dt,
+                        double eps, int64_t B, int32_t flags, double* loss, double* force, double* grad_pts,
+                        int32_t* iters, double* grad, double* loss_sum, const int32_t* skip_flag, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  return launch_elbow_loss<double, double>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, loss, force,
+                                           grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream,
+                                           flags);
 }
 
 int dpll_elbow_loss_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
                         const float* mu_pair, const float* half, const float* kin, const float* pts, float dt, float eps,
-                        int64_t B, float* loss, float* force, float* grad_pts, int32_t* iters, float* grad, float* loss_sum,
-                        const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream) {
-  return launch_elbow_loss<double, float>(g_loss_variant, x, x_plus, weight, inertia, mu_pair, half, kin, pts, (double)dt, (double)eps, B,
-                                          loss, force, grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream);
+                        int64_t B, int32_t flags, float* loss, float* force, float* grad_pts, int32_t* iters, float* grad,
+                        float* loss_sum, const int32_t* skip_flag, void* workspace, size_t workspace_bytes,
+                        void* stream) {
+  return launch_elbow_loss<double, float>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, (double)dt, (double)eps, B,
+                                          loss, force, grad_pts, iters, grad, loss_sum, skip_flag, workspace,
+                                          workspace_bytes, stream, flags);
 }
 
 int dpll_elbow_rollout_f64(const double* x0, const double* inertia, const double* mu_pair, const double* half,

@@ -84,11 +84,4 @@ int dpll_elbow_rollout_grad_saved_f64(const double* x0, const double* inertia, c
   return e == cudaSuccess ? DPLL_OK : (int)e;
 }
 
-int dpll_elbow_rollout_grad_f64(const double* x0, const double* inertia, const double* mu_pair, const double* half,
-                                const double* kin, double dt, double eps, int64_t B, int32_t steps, const double* xbar,
-                                double* gparams, double* gx0, void* stream) {
-  return dpll_elbow_rollout_grad_saved_f64(x0, inertia, mu_pair, half, kin, nullptr, dt, eps, B, steps, xbar, gparams, gx0,
-                                           stream);
-}
-
 }  // extern "C"

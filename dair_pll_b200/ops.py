@@ -34,9 +34,10 @@ def _workspace(device: torch.device) -> Tensor:
 
 
 def set_loss_variant(variant: int) -> None:
-    """0 = warp-level wavefront kernel, static sample ranges (default; bitwise reproducible), 1 = one sample per
-    thread (A/B measurements), 2 = wavefront kernel with dynamic sample distribution (faster by the load imbalance,
-    gradient sums reproducible only to rounding)."""
+    """Selects the cube loss kernel: 0 = warp-level wavefront kernel, static sample ranges (default; bitwise
+    reproducible), 1 = one sample per thread (A/B measurements), 2 = wavefront kernel with dynamic sample distribution
+    (faster by the load imbalance, gradient sums reproducible only to rounding).  The elbow loss always runs its
+    wavefront kernel."""
     _lib.check(_lib.load().dpll_set_loss_variant(variant), 'dpll_set_loss_variant')
 
 
@@ -352,7 +353,7 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
                    want_force: bool = False, want_iters: bool = False, want_loss: bool = True,
                    skip_flag: Optional[Tensor] = None, grad_out: Optional[Tensor] = None,
                    pts: Optional[Tensor] = None, want_grad_pts: bool = False, flags: int = 0):
-    """Direct call of ``dpll_elbow_loss_ex_*`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,15); inertia (20), mu_pair (2), half (6) or
+    """Direct call of ``dpll_elbow_loss_*`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,15); inertia (20), mu_pair (2), half (6) or
     witness points pts (B,8,3), kin (12).  Returns (loss (B,) | None, grad (28,) | None, loss_sum (1,),
     force (B,24) | None, iters (B,) | None[, grad_pts (B,8,3)])."""
     dtype = _check_inputs(x, x_plus, inertia, mu_pair, kin, *([half] if half is not None else []),
@@ -380,7 +381,7 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
         weight = weight.to(dtype).contiguous()
     ws = _workspace(dev)
     grad_pts = torch.zeros((B, 8, 3), dtype=dtype, device=dev) if (want_grad_pts and want_grad) else None
-    fn = getattr(_lib.load(), 'dpll_elbow_loss_ex_' + _SUFFIX[dtype])
+    fn = getattr(_lib.load(), 'dpll_elbow_loss_' + _SUFFIX[dtype])
     with torch.cuda.device(dev):
         rc = fn(_ptr(x), _ptr(x_plus), _ptr(weight), _ptr(inertia), _ptr(mu_pair), _ptr(half), _ptr(kin), _ptr(pts),
                 dt, eps, B, flags, _ptr(loss), _ptr(force), _ptr(grad_pts), _ptr(iters), _ptr(grad), _ptr(loss_sum),

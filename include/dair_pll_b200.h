@@ -13,8 +13,8 @@
  *    (`workspace`, at least dpll_workspace_bytes() bytes, 16-byte aligned).
  *  - `stream` is a cudaStream_t passed as void*; every call is asynchronous on it and
  *    performs no host synchronisation.  Compute calls are re-entrant.  Mutable library state: the
- *    A/B selector dpll_set_loss_variant (process-wide, measurement only) and the communicator
- *    objects of the data-parallel exchange (dpll_comm_*, one stream at a time each).
+ *    cube loss-kernel selector dpll_set_loss_variant (process-wide, measurement only) and the
+ *    communicator objects of the data-parallel exchange (dpll_comm_*, one stream at a time each).
  *  - Return value: 0 on success, a positive cudaError_t value if a launch failed, a
  *    negative DPLL_E* value for argument errors.  Numerical failure of a sample's QP
  *    is NOT an error: as in the reference (multibody_learnable_system.py:186-192) that
@@ -44,7 +44,7 @@ extern "C" {
 #define DPLL_EWORKSPACE (-2) /* workspace too small */
 #define DPLL_ECOMM (-3)      /* a peer did not arrive within the exchange's timeout */
 
-#define DPLL_VERSION 212     /* bumped with every change of a signature below; the binding checks it */
+#define DPLL_VERSION 213     /* bumped with every change of a signature below; the binding checks it */
 
 #define DPLL_CUBE_NX 13
 #define DPLL_CUBE_NC 4
@@ -57,12 +57,12 @@ extern "C" {
 /* Library/ABI version (major*100 + minor). */
 int dpll_version(void);
 
-/* Selects the loss-kernel implementation, for A/B measurement only: 0 = warp-level wavefront
+/* Selects the cube loss-kernel implementation, for A/B measurement only: 0 = warp-level wavefront
  * scheduler with static sample ranges (default; gradient sums bitwise reproducible), 1 = one sample
  * per thread, 2 = wavefront scheduler whose warps draw 32-sample chunks from a global counter (as
  * DPLL_LOSS_DYNAMIC below).  All three produce bitwise-identical PER-SAMPLE losses and forces; the
  * summed gradient of variant 2 depends on the chunk-to-warp assignment and is reproducible to
- * rounding only.  Process-wide setting. */
+ * rounding only.  Process-wide setting.  The elbow loss always runs its wavefront kernel. */
 int dpll_set_loss_variant(int variant);
 
 /* Bytes of device scratch any entry point below may need. */
@@ -359,14 +359,6 @@ int dpll_cube_rollout_backward_f64(const double* traj, const double* usol, const
                                    int32_t steps, const double* xbar, double* gparams, double* gx0, void* stream);
 
 /*
- * The same backward for the two-body (elbow) system with box geometries: gparams (B, 28) =
- * [d/d inertia (20) | d/d mu_pair (2) | d/d half (6)], gx0 (B, 15).  43 tangent directions per toss.
- */
-int dpll_elbow_rollout_grad_f64(const double* x0, const double* inertia, const double* mu_pair, const double* half,
-                                const double* kin, double dt, double eps, int64_t B, int32_t steps, const double* xbar,
-                                double* gparams, double* gx0, void* stream);
-
-/*
  * Backward of ONE learnable step of the two-body system with caller-supplied witness points pts (B, 8, 3) -- the learned
  * (support-function) geometry, whose points depend on the state through the caller's networks, so the time loop of that
  * rollout runs step by step (forward_dynamics multibody_learnable_system.py:199-304 with geometry.py:309-325): given
@@ -380,10 +372,11 @@ int dpll_elbow_step_pts_grad_f64(const double* x, const double* inertia, const d
 
 /*
  * The two-body rollout keeping every step's QP optimum, usol (B, steps, 7) (world twist of the first link + hinge rate;
- * v+ = v- + u*), and the forward-mode backward that uses it: with the optimum known, a dual-number step is ONE evaluation
- * and one 7x7 Cholesky solve at u* (whose tangent is the implicit-function derivative) instead of a whole dual-number
- * Newton solve.  usol nullable in the two *_grad entry points (then every step is solved again in dual arithmetic, as
- * dpll_elbow_rollout_grad_f64 does).  pts as in dpll_elbow_rollout_f64 (steps <= 1 when given).
+ * v+ = v- + u*), and the forward-mode backward that uses it, for box geometries: gparams (B, 28) = [d/d inertia (20) |
+ * d/d mu_pair (2) | d/d half (6)], gx0 (B, 15), 43 tangent directions per toss.  With the optimum known, a dual-number
+ * step is ONE evaluation and one 7x7 Cholesky solve at u* (whose tangent is the implicit-function derivative) instead of
+ * a whole dual-number Newton solve.  usol nullable in the two *_grad entry points (then every step is solved again in
+ * dual arithmetic).  pts as in dpll_elbow_rollout_f64 (steps <= 1 when given).
  */
 int dpll_elbow_rollout_saved_f64(const double* x0, const double* inertia, const double* mu_pair, const double* half,
                                  const double* kin, const double* pts, double dt, double eps, int64_t B, int32_t steps,
@@ -410,30 +403,20 @@ int dpll_elbow_rollout_grad_saved_f64(const double* x0, const double* inertia, c
  * evaluated by the caller) -- `half` may then be NULL, and `grad_pts` (B, 8, 3), nullable, receives
  * w_b * d loss_b / d pts[b] for the caller's network backward (grad[22..27] stay zero).  The rollout
  * accepts `pts` only for steps <= 1 (witness points depend on the state).
+ *
+ * `flags` of the loss: DPLL_LOSS_DYNAMIC hands 32-sample chunks to the warps in batch order, for cost-ordered
+ * batches (see dpll_cube_loss_leaf_dp_*); 0 keeps static sample ranges.
  */
-int dpll_elbow_loss_f64(const double* x, const double* x_plus, const double* weight,
-                        const double* inertia, const double* mu_pair, const double* half,
-                        const double* kin, const double* pts, double dt, double eps, int64_t B,
-                        double* loss, double* force, double* grad_pts, int32_t* iters, double* grad,
-                        double* loss_sum, const int32_t* skip_flag, void* workspace,
-                        size_t workspace_bytes, void* stream);
+int dpll_elbow_loss_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
+                        const double* mu_pair, const double* half, const double* kin, const double* pts,
+                        double dt, double eps, int64_t B, int32_t flags, double* loss, double* force,
+                        double* grad_pts, int32_t* iters, double* grad, double* loss_sum,
+                        const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream);
 int dpll_elbow_loss_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
-                        const float* mu_pair, const float* half, const float* kin, const float* pts,
-                        float dt, float eps, int64_t B, float* loss, float* force, float* grad_pts,
+                        const float* mu_pair, const float* half, const float* kin, const float* pts, float dt,
+                        float eps, int64_t B, int32_t flags, float* loss, float* force, float* grad_pts,
                         int32_t* iters, float* grad, float* loss_sum, const int32_t* skip_flag,
                         void* workspace, size_t workspace_bytes, void* stream);
-/* The same with `flags` (DPLL_LOSS_DYNAMIC: 32-sample chunks handed to the warps in batch order, for cost-ordered
- * batches -- see dpll_cube_loss_leaf_dp_*). */
-int dpll_elbow_loss_ex_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
-                           const double* mu_pair, const double* half, const double* kin, const double* pts,
-                           double dt, double eps, int64_t B, int32_t flags, double* loss, double* force,
-                           double* grad_pts, int32_t* iters, double* grad, double* loss_sum,
-                           const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream);
-int dpll_elbow_loss_ex_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
-                           const float* mu_pair, const float* half, const float* kin, const float* pts, float dt,
-                           float eps, int64_t B, int32_t flags, float* loss, float* force, float* grad_pts,
-                           int32_t* iters, float* grad, float* loss_sum, const int32_t* skip_flag,
-                           void* workspace, size_t workspace_bytes, void* stream);
 int dpll_elbow_rollout_f64(const double* x0, const double* inertia, const double* mu_pair,
                            const double* half, const double* kin, const double* pts, double dt,
                            double eps, int64_t B, int32_t steps, double* traj, double* force,
@@ -469,7 +452,7 @@ int dpll_chain_rollout_f64(int32_t n_links, const double* x0, const double* iner
                            double* traj, void* stream);
 /* Backward of the chain rollout (prediction loss): xbar (B, steps, n_x) w.r.t. traj[:, 1:] -> gparams (B, 14 n) =
  * [d/d inertia (10 n) | d/d mu_pair (n) | d/d half (3 n)] and gx0 (B, n_x), by forward-mode tangents through the step code
- * (14 n + n_x directions per toss), as dpll_elbow_rollout_grad_f64. */
+ * (14 n + n_x directions per toss), as dpll_elbow_rollout_grad_saved_f64 without usol. */
 int dpll_chain_rollout_grad_f64(int32_t n_links, const double* x0, const double* inertia, const double* mu_pair,
                                 const double* half, const double* kin, double dt, double eps, int64_t B, int32_t steps,
                                 const double* xbar, double* gparams, double* gx0, void* stream);
