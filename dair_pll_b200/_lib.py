@@ -9,7 +9,7 @@ import os
 from dair_pll_b200 import build as _build
 
 _LIB = None
-ABI_VERSION = 213        # DPLL_VERSION of include/dair_pll_b200.h this binding was written against
+ABI_VERSION = 214        # DPLL_VERSION of include/dair_pll_b200.h this binding was written against
 
 _c_void_p = ctypes.c_void_p
 _i64, _i32, _f64, _f32, _sz = ctypes.c_int64, ctypes.c_int32, ctypes.c_double, ctypes.c_float, ctypes.c_size_t
@@ -29,7 +29,7 @@ EXPORTS = {
     'dpll_cube_rollout_f64': ([_c_void_p] * 4 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
     'dpll_cube_rollout_f32': ([_c_void_p] * 4 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
     'dpll_cube_terms_f64': ([_c_void_p] * 5 + [_i64] + [_c_void_p] * 6, ctypes.c_int),
-    'dpll_body_loss_pts_f64': ([_c_void_p] * 6 + [_i32, _f64, _f64, _i64] + [_c_void_p] * 6 + [_c_void_p, _sz, _c_void_p],
+    'dpll_body_loss_pts_f64': ([_c_void_p] * 6 + [_i32, _f64, _f64, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p],
                                ctypes.c_int),
     'dpll_body_step_pts_f64': ([_c_void_p] * 4 + [_i32, _f64, _f64, _i64] + [_c_void_p] * 3, ctypes.c_int),
     'dpll_chain_loss_f64': ([_i32] + [_c_void_p] * 7 + [_f64, _f64, _i64] + [_c_void_p] * 5 + [_c_void_p, _sz, _c_void_p],
@@ -50,6 +50,7 @@ EXPORTS = {
     'dpll_icnn_mask_f64': ([_c_void_p, _i64, _f64, _c_void_p], ctypes.c_int),
     'dpll_icnn_output_f64': ([_c_void_p] * 5 + [_i64, _i32, _f64, _c_void_p, _c_void_p], ctypes.c_int),
     'dpll_elbow_support_directions_f64': ([_c_void_p, _i64] + [_c_void_p] * 3 + [_i32, _i64] + [_c_void_p] * 3, ctypes.c_int),
+    'dpll_body_support_directions_f64': ([_c_void_p, _i64, _c_void_p, _i32, _i64, _c_void_p, _c_void_p], ctypes.c_int),
     'dpll_icnn_tc_image_bytes': ([], ctypes.c_size_t),
     'dpll_icnn_tc_const_bytes': ([], ctypes.c_size_t),
     'dpll_icnn_tc_prepare_f64': ([_c_void_p] * 4 + [_i32, _f64, _c_void_p, _c_void_p, _c_void_p], ctypes.c_int),

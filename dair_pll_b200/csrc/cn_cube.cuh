@@ -1004,6 +1004,295 @@ CN_HD T body_loss_sample_pts(const CubeParams<T>& P, const SolverCfg<T>& cfg, co
   return loss;
 }
 
+// ---------------------------------------------------------------------------
+// Witness-point pieces of the wavefront loss kernel (cube_loss_wf_kernel, PTS instance): the same per-sample
+// composition as body_loss_sample_pts -- triage, prologue, feasible-segment start, Newton visits, epilogue -- cut where
+// the box pieces above are cut.  pts points at the sample's 12 body-frame point coordinates (read in place: the
+// per-contact loops may be rolled, and a rolled loop over a register array would go through local memory).  Contacts
+// c >= n_c are switched off as in body_loss_sample_pts: rho_c = 0, q_c = (0, 0, contact_off), zero force, no
+// penetration term.  grad_pts (12, nullable, written) receives wpts * d loss / d p_c (zero rows for c >= n_c).
+// ---------------------------------------------------------------------------
+
+// Free-flight fast path (the triage phase), as cube_loss_free_flight: true (loss, grad11 += d loss / d [inertia | mu],
+// grad_pts written) when every active contact's q lies in the polar cone; false, nothing written, otherwise.
+template <typename T>
+CN_HD bool body_loss_free_flight_pts(const CubeParams<T>& P, const T* x, const T* xp, const T* pts, int n_c, T wpts,
+                                     T* grad11, T* grad_pts, T* loss_out) {
+  T R[9], vp[6], acc[6], dv[6];
+  quat_to_rot(xp, R);
+#pragma unroll
+  for (int i = 0; i < 6; ++i) vp[i] = xp[7 + i];
+  cube_free_accel(P, R, vp, acc, acc + 3);
+#pragma unroll
+  for (int i = 0; i < 6; ++i) dv[i] = vp[i] - (x[7 + i] + P.dt * acc[i]);
+  T dvW[3], vW[3];
+  rot3(R, dv, dvW); rot3(R, vp, vW);
+  bool open = true;
+  T pen = T(0);
+#pragma unroll 1
+  for (int c = 0; c < n_c; ++c) {
+    T rho[3], ed[3], ev[3];
+    rot3(R, pts + 3 * c, rho);
+    cross3(dvW, rho, ed); cross3(vW, rho, ev);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) { ed[i] += dv[3 + i]; ev[i] += vp[3 + i]; }
+    const T tx = P.mu * ev[0], ty = P.mu * ev[1];
+    const T speed2 = tx * tx + ty * ty;
+    const T speed = speed2 * t_rsqrt(t_max(speed2, t_tiny<T>()));
+    const T phic = rho[2] + xp[6];
+    const T q0 = -P.mu * ed[0] + P.dt * tx, q1 = -P.mu * ed[1] + P.dt * ty;
+    const T qn = -ed[2] + t_abs(phic) + P.dt * speed;
+    open = open && (qn >= T(0)) && (q0 * q0 + q1 * q1 <= qn * qn);
+    const T pneg = t_max(-phic, T(0));
+    pen += pneg * pneg;
+  }
+  if (!open) return false;
+  // 1/2 dv^T M dv in state coordinates, as cube_loss_free_flight
+  T vB[3], Iw[3], cxv[3];
+  rot3t(R, dv + 3, vB);
+  sym3_mul(P.Io, dv, Iw);
+  cross3(P.c, vB, cxv);
+  const T e = dot3(dv, Iw) + T(2) * P.m * dot3(dv, cxv) + P.m * dot3(dv + 3, dv + 3);
+  *loss_out = T(0.5) * e + pen;
+#pragma unroll 1
+  for (int c = 0; c < CUBE_NC; ++c) {
+    // d loss / d p_c at f = 0: the penetration term only, -2 max(-phi_c, 0) R^T e_z
+    const T phic = c < n_c ? R[6] * pts[3 * c] + R[7] * pts[3 * c + 1] + R[8] * pts[3 * c + 2] + xp[6] : T(0);
+    const T phibar = T(-2) * t_max(-phic, T(0)) * wpts;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) if (grad_pts) grad_pts[3 * c + k] = (grad11 && c < n_c) ? phibar * R[6 + k] : T(0);
+  }
+  if (grad11) {
+    T lam[6], Kww[9], N[9], trvv = T(0);
+#pragma unroll
+    for (int i = 0; i < 6; ++i) lam[i] = -P.dt * dv[i];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+        Kww[3 * i + j] = T(0.5) * dv[i] * dv[j] - lam[i] * acc[j];
+        N[3 * i + j] = dv[i] * dv[3 + j] - lam[i] * acc[3 + j] - lam[3 + j] * acc[i];
+      }
+#pragma unroll
+    for (int i = 0; i < 3; ++i) trvv += T(0.5) * dv[3 + i] * dv[3 + i] - lam[3 + i] * acc[3 + i];
+    rigid_body_inertia_adjoint<T>(P.m, P.c, R, vp, P.grav, Kww, N, trvv, lam, grad11);
+  }
+  return true;
+}
+
+// Prologue: the loss QP at (q+, v+) in the slot S and the sample's auxiliaries A (A.sel unused), as cube_loss_prologue.
+// A switched-off contact stays inside the polar cone along the whole start segment, so it takes no part in a_min.
+template <typename T, int UNR>
+CN_HD void body_loss_prologue_pts(const CubeParams<T>& P, const T* x, const T* xp, const T* pts, int n_c,
+                                  const CubeProb<T>& S, CubeLossAux<T>& A) {
+  T* R = A.R;
+  quat_to_rot(xp, R);
+  T Am[9];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const T r0 = R[3 * i], r1 = R[3 * i + 1], r2 = R[3 * i + 2];
+    Am[3 * i + 0] = r0 * P.Io[0] + r1 * P.Io[3] + r2 * P.Io[4];
+    Am[3 * i + 1] = r0 * P.Io[3] + r1 * P.Io[1] + r2 * P.Io[5];
+    Am[3 * i + 2] = r0 * P.Io[4] + r1 * P.Io[5] + r2 * P.Io[2];
+  }
+  S.IW(0) = Am[0] * R[0] + Am[1] * R[1] + Am[2] * R[2];
+  S.IW(1) = Am[3] * R[3] + Am[4] * R[4] + Am[5] * R[5];
+  S.IW(2) = Am[6] * R[6] + Am[7] * R[7] + Am[8] * R[8];
+  S.IW(3) = Am[0] * R[3] + Am[1] * R[4] + Am[2] * R[5];
+  S.IW(4) = Am[0] * R[6] + Am[1] * R[7] + Am[2] * R[8];
+  S.IW(5) = Am[3] * R[6] + Am[4] * R[7] + Am[5] * R[8];
+  T cW[3];
+  rot3(R, P.c, cW);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) S.mcW(i) = P.m * cW[i];
+  A.sel = 0u;
+  A.pos_z = xp[6];
+#pragma unroll
+  for (int i = 0; i < 6; ++i) A.vp[i] = xp[7 + i];
+  cube_free_accel(P, R, A.vp, A.acc, A.acc + 3);
+#pragma unroll
+  for (int i = 0; i < 6; ++i) A.dv[i] = A.vp[i] - (x[7 + i] + P.dt * A.acc[i]);
+  T dvW[6], vW[6];
+  rot3(R, A.dv, dvW); rot3(R, A.vp, vW);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) { dvW[3 + i] = A.dv[3 + i]; vW[3 + i] = A.vp[3 + i]; }
+  T pen = T(0), a_min = T(2);
+#pragma unroll UNR
+  for (int c = 0; c < CUBE_NC; ++c) {
+    if (c < n_c) {
+      T rho[3];
+      rot3(R, pts + 3 * c, rho);
+#pragma unroll
+      for (int i = 0; i < 3; ++i) S.rho(3 * c + i) = rho[i];
+      T ed[3], ev[3];
+      cross3(dvW, rho, ed); cross3(vW, rho, ev);
+#pragma unroll
+      for (int i = 0; i < 3; ++i) { ed[i] += dvW[3 + i]; ev[i] += vW[3 + i]; }
+      const T sx = P.mu * ev[0], sy = P.mu * ev[1];
+      const T speed2 = sx * sx + sy * sy;
+      const T speed = speed2 * t_rsqrt(t_max(speed2, t_tiny<T>()));
+      const T phic = rho[2] + A.pos_z;
+      const T s0 = P.dt * sx, s1 = P.dt * sy, s2 = t_abs(phic) + P.dt * speed;
+      const T e0 = -P.mu * ed[0], e1 = -P.mu * ed[1], e2 = -ed[2];
+      S.q(3 * c) = e0 + s0;
+      S.q(3 * c + 1) = e1 + s1;
+      S.q(3 * c + 2) = e2 + s2;
+      const T pneg = t_max(-phic, T(0));
+      pen += pneg * pneg;
+      if (CN_LOSS_START_FACTOR > 0) {
+        const T Aq = e0 * e0 + e1 * e1 - e2 * e2, Bq = T(2) * (s0 * e0 + s1 * e1 - s2 * e2);
+        const T Cq = t_min(s0 * s0 + s1 * s1 - s2 * s2, T(0));
+        const T disc = Bq * Bq - T(4) * Aq * Cq;
+        const T dpos = t_max(disc, T(0));
+        const T den = Bq + dpos * t_rsqrt(t_max(dpos, t_tiny<T>()));
+        const T a_c = (disc >= T(0) && den > T(0)) ? T(-2) * Cq * t_rcp(den) : T(2);
+        a_min = t_min(a_min, a_c);
+      }
+    } else {
+#pragma unroll
+      for (int i = 0; i < 3; ++i) S.rho(3 * c + i) = T(0);
+      S.q(3 * c) = T(0); S.q(3 * c + 1) = T(0); S.q(3 * c + 2) = contact_off<T>();
+    }
+  }
+  A.a_min = a_min;
+#pragma unroll
+  for (int i = 0; i < 6; ++i) A.dvW[i] = dvW[i];
+  T Mdv[6];
+  cube_mass_mul(P, S, dvW, Mdv);
+  T e = T(0);
+#pragma unroll
+  for (int i = 0; i < 6; ++i) e += dvW[i] * Mdv[i];
+  A.konst = T(0.5) * e + pen;
+}
+
+// Epilogue: loss at the optimum u; with grad11, grad11 += d loss / d [inertia | mu] and grad_pts = wpts d loss / d p_c
+// (the formulas of body_loss_sample_pts); without, grad_pts is zero.  PARK as in cube_loss_epilogue.
+template <typename T, int UNR, bool PARK = false>
+CN_HD T body_loss_epilogue_pts(const CubeParams<T>& P, const CubeProb<T>& S, const CubeLossAux<T>& A, const T* u, int n_c,
+                               T wpts, T* grad11, T* grad_pts, T* force_out) {
+  const T* R = A.R;
+  T zW[6] = {T(0), T(0), T(0), T(0), T(0), T(0)};
+  T qf = T(0), ff = T(0), fmax = T(0);
+#pragma unroll UNR
+  for (int c = 0; c < CUBE_NC; ++c) {
+    T f[3] = {T(0), T(0), T(0)};
+    if (c < n_c) {
+      T rho[3], r[3];
+      cube_contact_residual(P, S, c, u, rho, r);
+      cone_eval<T, false>(r, P.inv_eps, P.mu, f, (T*)nullptr);
+      const T ft[3] = {P.mu * f[0], P.mu * f[1], f[2]};
+      T tq[3];
+      cross3(rho, ft, tq);
+#pragma unroll
+      for (int i = 0; i < 3; ++i) {
+        zW[i] += tq[i]; zW[3 + i] += ft[i];
+        qf += S.q(3 * c + i) * f[i]; ff += f[i] * f[i];
+        const T af = t_abs(f[i]);
+        fmax = (af > fmax || af != af) ? af : fmax;
+      }
+      if (PARK) {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) S.q(3 * c + i) = f[i];
+      }
+    }
+    if (force_out) { force_out[c] = f[2]; force_out[4 + 2 * c] = f[0]; force_out[4 + 2 * c + 1] = f[1]; }
+  }
+  if (grad_pts) {
+#pragma unroll 1
+    for (int i = 0; i < 12; ++i) grad_pts[i] = T(0);
+  }
+  if (!(fmax <= T(1e3))) {
+    if (force_out) for (int i = 0; i < 12; ++i) force_out[i] = T(0);
+    return T(0);
+  }
+  T z[6], y[6];
+  rot3t(R, zW, z);
+#pragma unroll
+  for (int i = 0; i < 3; ++i) z[3 + i] = zW[3 + i];
+  cube_minv(P, R, z, z + 3, y, y + 3);
+  T zy = T(0);
+#pragma unroll
+  for (int i = 0; i < 6; ++i) zy += z[i] * y[i];
+  const T loss = T(0.5) * zy + T(0.5) * P.eps * ff + qf + A.konst;
+  if (!grad11) return loss;
+  const T* dv = A.dv; const T* a = A.acc; const T* w = A.vp;
+  T lam[6], b[6];
+#pragma unroll
+  for (int i = 0; i < 6; ++i) { b[i] = y[i] - dv[i]; lam[i] = P.dt * b[i]; }
+  T Kww[9], N[9], trvv = T(0);
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+      Kww[3 * i + j] = T(0.5) * (dv[i] * dv[j] - y[i] * y[j]) - lam[i] * a[j];
+      N[3 * i + j] = (dv[i] * dv[3 + j] - y[i] * y[3 + j]) - lam[i] * a[3 + j] - lam[3 + j] * a[i];
+    }
+#pragma unroll
+  for (int i = 0; i < 3; ++i) trvv += T(0.5) * (dv[3 + i] * dv[3 + i] - y[3 + i] * y[3 + i]) - lam[3 + i] * a[3 + i];
+  rigid_body_inertia_adjoint<T>(P.m, P.c, R, w, P.grav, Kww, N, trvv, lam, grad11);
+  T bW[3], wW[3];
+  rot3(R, b, bW); rot3(R, w, wW);
+  T gmu = T(0);
+#pragma unroll UNR
+  for (int c = 0; c < CUBE_NC; ++c) {
+    if (c < n_c) {
+      T rho[3], r[3], f[3];
+      if (PARK) {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) { rho[i] = S.rho(3 * c + i); f[i] = S.q(3 * c + i); }
+      } else {
+        cube_contact_residual(P, S, c, u, rho, r);
+        cone_eval<T, false>(r, P.inv_eps, P.mu, f, (T*)nullptr);
+      }
+      const T ftx = f[0], fty = f[1], fn = f[2];
+      T eb[3], ev[3];
+      cross3(bW, rho, eb); cross3(wW, rho, ev);
+#pragma unroll
+      for (int i = 0; i < 3; ++i) { eb[i] += b[3 + i]; ev[i] += w[3 + i]; }
+      const T sx = P.mu * ev[0], sy = P.mu * ev[1];
+      const T sinv = t_rsqrt(t_max(sx * sx + sy * sy, t_tiny<T>()));
+      const T ux = sx * sinv, uy = sy * sinv;
+      const T gx = P.dt * (fn * ux + ftx), gy = P.dt * (fn * uy + fty);
+      gmu += ftx * eb[0] + fty * eb[1] + gx * ev[0] + gy * ev[1];
+      const T ft[3] = {P.mu * ftx, P.mu * fty, fn};
+      const T gt[3] = {P.mu * gx, P.mu * gy, T(0)};
+      T ftB[3], gtB[3], p1[3], p2[3];
+      rot3t(R, ft, ftB); rot3t(R, gt, gtB);
+      cross3(ftB, b, p1); cross3(gtB, w, p2);
+      const T phic = rho[2] + A.pos_z;
+      const T phibar = (phic > T(0) ? fn : (phic < T(0) ? -fn : T(0))) - T(2) * t_max(-phic, T(0));
+#pragma unroll
+      for (int k = 0; k < 3; ++k) if (grad_pts) grad_pts[3 * c + k] = wpts * (p1[k] + p2[k] + phibar * R[6 + k]);
+    }
+  }
+  grad11[10] += gmu;
+  return loss;
+}
+
+// The wavefront kernel's per-sample composition in one thread (host emulation of the PTS instance): triage, then
+// prologue, feasible-segment start, Newton visits and epilogue.  Returns the loss; iters_out: Newton directions.
+template <typename T>
+CN_HD T body_loss_sample_pts_wf(const CubeParams<T>& P, const SolverCfg<T>& cfg, const T* x, const T* xp, const T* pts,
+                                int n_c, T* grad11, T* grad_pts, int* iters_out) {
+  T l = T(0);
+  if (body_loss_free_flight_pts<T>(P, x, xp, pts, n_c, T(1), grad11, grad_pts, &l)) {
+    if (iters_out) *iters_out = 0;
+    return l;
+  }
+  T store[CUBE_PROB_FIELDS];
+  const CubeProb<T> S{store, 1};
+  CubeLossAux<T> A;
+  body_loss_prologue_pts<T, 1>(P, x, xp, pts, n_c, S, A);
+  T u[6];
+  cube_loss_start<T>(A, T(CN_LOSS_START_FACTOR), u);
+  T d[6], d0 = T(0), best = T(-1);
+  CubeTrial<T> tr{T(1), T(0), T(1)};
+  int it = 0;
+  while (cube_newton_visit<T, 1>(P, S, cfg, u, d, d0, best, tr, it) != NEWTON_DONE) {}
+  if (iters_out) *iters_out = it & 0xff;
+  return body_loss_epilogue_pts<T, 1, true>(P, S, A, u, n_c, T(1), grad11, grad_pts, (T*)nullptr);
+}
+
 // learnable time step with witness points (forward_dynamics :260-304 + the Lie-group update)
 template <typename T>
 CN_HD int body_step_sample_pts(const CubeParams<T>& P, const SolverCfg<T>& cfg, const T* x, const T* pts, int n_c,

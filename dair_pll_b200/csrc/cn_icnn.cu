@@ -136,6 +136,25 @@ __global__ void elbow_support_directions_kernel(const double* __restrict__ q, in
   }
 }
 
+// Support directions of a single floating body against the ground (minus the third row of its world rotation, s = 2 / |q|^2
+// for the unnormalised quaternion) and their n_query perturbed, normalised copies, as elbow_support_directions_kernel for
+// one link.  One thread per sample.
+__global__ void body_support_directions_kernel(const double* __restrict__ q, int64_t q_stride, const double* __restrict__ pert,
+                                               int nq, int64_t B, double* __restrict__ dirs) {
+  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const double* qb = q + b * q_stride;
+  const double w = qb[0], x = qb[1], y = qb[2], z = qb[3];
+  const double s = 2.0 / (w * w + x * x + y * y + z * z);
+  const double r[3] = {s * (x * z - w * y), s * (y * z + w * x), 1 - s * (x * x + y * y)};      // R[2, :]
+  double* out = dirs + b * nq * 3;
+  for (int k = 0; k < nq; ++k) {
+    const double vx = -r[0] + pert[3 * k], vy = -r[1] + pert[3 * k + 1], vz = -r[2] + pert[3 * k + 2];
+    const double n = sqrt(vx * vx + vy * vy + vz * vz);
+    out[3 * k] = vx / n; out[3 * k + 1] = vy / n; out[3 * k + 2] = vz / n;
+  }
+}
+
 int grid_for(int64_t work, int per_block) {
   int64_t b = (work + per_block - 1) / per_block;
   return (int)(b < 1 ? 1 : (b > 2147483647LL ? 2147483647LL : b));
@@ -163,6 +182,17 @@ int dpll_elbow_support_directions_f64(const double* q, int64_t q_stride, const d
   if (!q || !dirs0 || !dirs1) return DPLL_EINVAL;
   elbow_support_directions_kernel<<<grid_for(B, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       q, q_stride, axis, pert0, pert1, n_query, B, dirs0, dirs1);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? DPLL_OK : (int)e;
+}
+
+int dpll_body_support_directions_f64(const double* q, int64_t q_stride, const double* pert, int32_t n_query, int64_t B,
+                                     double* dirs, void* stream) {
+  if (B < 0 || n_query <= 0 || q_stride < 4 || !pert) return DPLL_EINVAL;
+  if (B == 0) return DPLL_OK;
+  if (!q || !dirs) return DPLL_EINVAL;
+  body_support_directions_kernel<<<grid_for(B, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(q, q_stride, pert, n_query,
+                                                                                                  B, dirs);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? DPLL_OK : (int)e;
 }

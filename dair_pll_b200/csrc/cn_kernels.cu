@@ -201,7 +201,7 @@ template <typename T> struct WfWarpPool {
   int32_t q_in[kWfQin];         // offsets of triaged samples that need the solver, waiting for a slot
 };
 
-template <typename T, typename IO, int UNR, bool RACE = false>
+template <typename T, typename IO, int UNR, bool RACE = false, bool PTS = false>
 __global__ void __launch_bounds__(kWfWarps * 32, CN_WF_MIN_BLOCKS)
 cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const IO* __restrict__ weight,
                     const IO* __restrict__ inertia, const IO* __restrict__ mu, const IO* __restrict__ half, T dt,
@@ -219,6 +219,14 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
   // the rounding of the gradient sums) then depends on timing.  (Measured and dropped: a two-ended queue in which
   // the second block of every SM consumes the batch from its cheap end, so that no two warps of long chains share
   // an SM sub-partition -- 0.427 vs 0.398 ms at 1,048,576 pairs, 0.143 vs 0.129 ms at 131,072.)
+  // PTS (the witness-point instance, T = IO): the lever arms come from per-sample body-frame points instead of selected box
+  // corners (body_*_pts in cn_cube.cuh).  It takes its extra arguments through parameters the box instances have and it
+  // does not use -- extra kernel parameters change ptxas's register allocation of the box instances -- so that their
+  // code stays as it is:  half = the points (B, 4, 3), of which the first n_c are used;  u_out = grad_pts (B, 4, 3),
+  // w_b d loss_b / d pts_b (nullable);  want_grad = bit 0 as for the box | n_c << 1.  u_init must be null and RACE false.
+  // Accumulators: [d/d inertia 10 | d/d mu | loss sum].  Its code sits in `if constexpr` branches in front of the box
+  // statements, which keep their text: even a dead statement's line information changes the box instances' allocation.
+  static_assert(!(PTS && RACE), "no racing warps for witness points");
   if (skip_flag && *skip_flag) return;
   // DPLL_LOSS_RACE (the RACE instantiation): the warps of blocks [0, race_blocks) are RACING warps for the first `head`
   // samples (the expensive head of a cost-ordered batch); the other blocks run the wavefront scheduler over the rest.  A
@@ -244,6 +252,13 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
   const unsigned lt_mask = (1u << lane) - 1u;
 
   cn::CubeParams<T> P;
+  if constexpr (PTS) {
+    T in[10], m[1], h[3] = {T(0), T(0), T(0)};
+#pragma unroll
+    for (int i = 0; i < 10; ++i) in[i] = T(inertia[i]);
+    m[0] = T(mu[0]);
+    cn::cube_params_init(P, in, m, h, dt, eps);
+  } else
   load_cube_params<T, IO>(P, inertia, mu, half, dt, eps);
   const cn::SolverCfg<T> cfg = cn::default_cfg<T>();
   T acc[kNAcc];
@@ -306,6 +321,23 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
 #pragma unroll
         for (int i = 0; i < DPLL_CUBE_NPARAM; ++i) gs[i] = T(0);
         T l = T(0);
+        if constexpr (PTS) {
+          const T w = weight ? T(weight[b]) : T(1);
+          if (cn::body_loss_free_flight_pts<T>(P, xs, xps, half + b * 12, want_grad >> 1, w, (want_grad & 1) ? gs : (T*)nullptr,
+                                               u_out ? u_out + b * 12 : (IO*)nullptr, &l)) {
+            if (force) {
+#pragma unroll
+              for (int i = 0; i < 12; ++i) force[b * 12 + i] = IO(0);
+            }
+#pragma unroll
+            for (int i = 0; i < 11; ++i) acc[i] += w * gs[i];
+            if (loss) loss[b] = IO(l);
+            acc[11] += l;
+            if (iters) iters[b] = 0;
+          } else {
+            queue = true;
+          }
+        } else
         if (cn::cube_loss_free_flight<T>(P, xs, xps, want_grad ? gs : (T*)nullptr, &l)) {
           if (force) {
 #pragma unroll
@@ -404,8 +436,31 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
           for (int i = 0; i < 13; ++i) { xs[i] = T(x[b * ldx + i]); xps[i] = T(xp[b * ldxp + i]); }
           const cn::CubeProb<T> S{&pool->field[0][slot], kWfSlots};
           cn::CubeLossAux<T> A;
+          if constexpr (PTS) cn::body_loss_prologue_pts<T, kWfUnrPE>(P, xs, xps, half + b * 12, want_grad >> 1, S, A);
+          else
           cn::cube_loss_prologue<T, kWfUnrPE>(P, xs, xps, S, A);      // (re)builds IW, mcW, rho, q in the slot
           if (pass == 0) {
+            if constexpr (PTS) {
+              T u[6], gs[11], fo[12];
+#pragma unroll
+              for (int i = 0; i < 6; ++i) u[i] = pool->field[33 + i][slot];
+#pragma unroll
+              for (int i = 0; i < 11; ++i) gs[i] = T(0);
+              const T w = weight ? T(weight[b]) : T(1);
+              const T l = cn::body_loss_epilogue_pts<T, kWfUnrPE, true>(P, S, A, u, want_grad >> 1, w,
+                                                                        (want_grad & 1) ? gs : (T*)nullptr,
+                                                                        u_out ? u_out + b * 12 : (IO*)nullptr,
+                                                                        force ? fo : (T*)nullptr);
+              if (force) {
+#pragma unroll
+                for (int i = 0; i < 12; ++i) force[b * 12 + i] = IO(fo[i]);
+              }
+#pragma unroll
+              for (int i = 0; i < 11; ++i) acc[i] += w * gs[i];
+              if (loss) loss[b] = IO(l);
+              acc[11] += l;
+              if (iters) iters[b] = pool->iters[slot] & 0xff;
+            } else {
             T u[6];
 #pragma unroll
             for (int i = 0; i < 6; ++i) u[i] = pool->field[33 + i][slot];
@@ -427,6 +482,7 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
             if (u_out) {
 #pragma unroll
               for (int i = 0; i < 6; ++i) u_out[b * 6 + i] = IO(u[i]);
+            }
             }
             pool->sample[slot] = -1;
           } else {
@@ -601,70 +657,6 @@ cube_rollout_kernel(const IO* __restrict__ x0, const IO* __restrict__ inertia, c
       for (int i = 0; i < 13; ++i) { xc[i] = xn[i]; out[(int64_t)(s + 1) * 13 + i] = IO(xn[i]); }
     }
     if (iters) iters[b] = total;
-  }
-}
-
-// Single floating body with caller-supplied witness points (Sphere / Polygon / any plane-convex pair,
-// cn_cube.cuh:body_loss_sample_pts): one sample per thread.  Accumulators: [0, 11) d/d [inertia | mu], 11 = loss sum.
-template <typename T, typename IO>
-__global__ void __launch_bounds__(kLossThreads)
-body_pts_loss_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const IO* __restrict__ weight,
-                     const IO* __restrict__ inertia, const IO* __restrict__ mu, const IO* __restrict__ pts, int n_c, T dt,
-                     T eps, int64_t B, IO* __restrict__ loss, IO* __restrict__ force, IO* __restrict__ grad_pts,
-                     int32_t* __restrict__ iters, T* __restrict__ partials, int want_grad) {
-  cn::CubeParams<T> P;
-  {
-    T in[10], m[1], h[3] = {T(0), T(0), T(0)};
-#pragma unroll
-    for (int i = 0; i < 10; ++i) in[i] = T(inertia[i]);
-    m[0] = T(mu[0]);
-    cn::cube_params_init(P, in, m, h, dt, eps);
-  }
-  const cn::SolverCfg<T> cfg = cn::default_cfg<T>();
-  T acc[kNAcc];
-#pragma unroll
-  for (int i = 0; i < kNAcc; ++i) acc[i] = T(0);
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += stride) {
-    T xs[13], xps[13], pt[12], gs[11], gp[12], fo[12];
-#pragma unroll
-    for (int i = 0; i < 13; ++i) { xs[i] = T(x[b * 13 + i]); xps[i] = T(xp[b * 13 + i]); }
-#pragma unroll
-    for (int i = 0; i < 12; ++i) pt[i] = T(pts[b * 12 + i]);
-#pragma unroll
-    for (int i = 0; i < 11; ++i) gs[i] = T(0);
-    int it;
-    const T l = cn::body_loss_sample_pts<T>(P, cfg, xs, xps, pt, n_c, want_grad ? gs : (T*)nullptr, gp,
-                                            force ? fo : (T*)nullptr, &it);
-    const T w = weight ? T(weight[b]) : T(1);
-    if (force) {
-#pragma unroll
-      for (int i = 0; i < 12; ++i) force[b * 12 + i] = IO(fo[i]);
-    }
-    if (grad_pts) {
-#pragma unroll
-      for (int i = 0; i < 12; ++i) grad_pts[b * 12 + i] = IO(w * gp[i]);
-    }
-#pragma unroll
-    for (int i = 0; i < 11; ++i) acc[i] += w * gs[i];
-    if (loss) loss[b] = IO(l);
-    acc[11] += l;
-    if (iters) iters[b] = it;
-  }
-  if (!partials) return;
-  __shared__ T red[kLossThreads / 32][kNAcc];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int i = 0; i < kNAcc; ++i) {
-    const T s = warp_sum(acc[i]);
-    if (lane == 0) red[warp][i] = s;
-  }
-  __syncthreads();
-  if (threadIdx.x < kNAcc) {
-    T s = T(0);
-#pragma unroll
-    for (int w = 0; w < kLossThreads / 32; ++w) s += red[w][threadIdx.x];
-    partials[(int64_t)blockIdx.x * kNAcc + threadIdx.x] = s;
   }
 }
 
@@ -866,6 +858,21 @@ __global__ void __launch_bounds__(256) fma_peak_kernel(T* out, int64_t iters) {
   out[(int64_t)blockIdx.x * blockDim.x + threadIdx.x] = s;
 }
 
+// Grid of a wavefront loss launch: at most one resident set of blocks (*cap), fewer for small batches -- a warp needs a
+// few hundred samples to keep its pool full; with fewer, every SM would run many mostly-empty warps at the issue rate of
+// full ones.
+template <typename K>
+int wf_blocks(int64_t B, K kernel, size_t smem, int sms, int64_t* cap) {
+  int per_sm = 0;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kWfWarps * 32, smem);
+  if (per_sm < 1) per_sm = 1;
+  const int64_t need = (B + kWfWarps * kWfMinPerWarp - 1) / (kWfWarps * kWfMinPerWarp);
+  *cap = (int64_t)sms * per_sm;
+  if (*cap > kMaxBlocks) *cap = kMaxBlocks;
+  const int blocks = (int)(need < *cap ? need : *cap);
+  return blocks < 1 ? 1 : blocks;
+}
+
 constexpr int64_t kRaceMaxBatch = 300000;     // larger launches are bound by throughput, not by their longest chain
 constexpr int64_t kRaceMaxHead = 2048;
 
@@ -904,16 +911,8 @@ int launch_cube_loss(int variant, const IO* x, const IO* xp, const IO* weight, c
     if (ea == cudaSuccess)
       ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (ea != cudaSuccess) return (int)ea;
-    int per_sm = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cube_loss_wf_kernel<T, IO, kWfUnr>, kWfWarps * 32, smem);
-    if (per_sm < 1) per_sm = 1;
-    // A warp needs a few hundred samples to keep its pool full; with fewer, every SM would run many
-    // mostly-empty warps at the issue rate of full ones.  Small batches therefore use fewer warps.
-    int64_t need = (B + kWfWarps * kWfMinPerWarp - 1) / (kWfWarps * kWfMinPerWarp);
-    int64_t cap = (int64_t)di.sms * per_sm;
-    if (cap > kMaxBlocks) cap = kMaxBlocks;
-    blocks = (int)(need < cap ? need : cap);
-    if (blocks < 1) blocks = 1;
+    int64_t cap;
+    blocks = wf_blocks(B, cube_loss_wf_kernel<T, IO, kWfUnr>, smem, di.sms, &cap);
     unsigned long long* dyn = nullptr;
     if (variant == 2) {
       if (!workspace || workspace_bytes < dpll_workspace_bytes()) return DPLL_EWORKSPACE;
@@ -1105,30 +1104,43 @@ int dpll_cube_rollout_f32(const float* x0, const float* inertia, const float* mu
 
 int dpll_body_loss_pts_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
                            const double* mu_pair, const double* pts, int32_t n_contacts, double dt, double eps, int64_t B,
-                           double* loss, double* force, double* grad_pts, int32_t* iters, double* grad, double* loss_sum,
-                           void* workspace, size_t workspace_bytes, void* stream) {
+                           int32_t flags, double* loss, double* force, double* grad_pts, int32_t* iters, double* grad,
+                           double* loss_sum, const int32_t* skip_flag, void* workspace, size_t workspace_bytes,
+                           void* stream) {
   if (B < 0 || !inertia || !mu_pair || n_contacts < 1 || n_contacts > DPLL_CUBE_NC) return DPLL_EINVAL;
   if (B > 0 && (!x || !x_plus || !pts)) return DPLL_EINVAL;
   const bool want_red = grad || loss_sum;
-  if (want_red && (!workspace || workspace_bytes < dpll_workspace_bytes())) return DPLL_EWORKSPACE;
+  const bool dynamic = (flags & DPLL_LOSS_DYNAMIC) != 0;
+  if ((want_red || dynamic) && (!workspace || workspace_bytes < dpll_workspace_bytes())) return DPLL_EWORKSPACE;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const DeviceInfo di = device_info();
-  int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, body_pts_loss_kernel<double, double>, kLossThreads, 0);
-  if (per_sm < 1) per_sm = 1;
-  int64_t need = (B + kLossThreads - 1) / kLossThreads;
-  int64_t cap = (int64_t)di.sms * per_sm;
-  if (cap > kMaxBlocks) cap = kMaxBlocks;
-  int blocks = (int)(need < cap ? need : cap);
-  if (blocks < 1) blocks = 1;
+  // the box's wavefront kernel, witness-point instance; the same grid and the same choice of instance by batch size
+  const size_t smem = sizeof(WfWarpPool<double>) * kWfWarps;
+  cudaError_t ea = cudaFuncSetAttribute(cube_loss_wf_kernel<double, double, kWfUnr, false, true>,
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (ea == cudaSuccess)
+    ea = cudaFuncSetAttribute(cube_loss_wf_kernel<double, double, 4, false, true>,
+                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (ea != cudaSuccess) return (int)ea;
+  int64_t cap;
+  const int blocks = wf_blocks(B, cube_loss_wf_kernel<double, double, kWfUnr, false, true>, smem, di.sms, &cap);
+  unsigned long long* dyn = nullptr;
+  if (dynamic) {
+    dyn = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + kWsQueueOffset);
+    cudaError_t em = cudaMemsetAsync(dyn, 0, kWsQueueBytes, st);
+    if (em != cudaSuccess) return (int)em;
+  }
   double* partials = want_red ? static_cast<double*>(workspace) : nullptr;
-  body_pts_loss_kernel<double, double><<<blocks, kLossThreads, 0, st>>>(x, x_plus, weight, inertia, mu_pair, pts, n_contacts,
-                                                                      dt, eps, B, loss, force, grad_pts, iters, partials,
-                                                                      grad ? 1 : 0);
+  auto kernel = B <= cap * kWfWarps * 320 ? cube_loss_wf_kernel<double, double, 4, false, true>
+                                          : cube_loss_wf_kernel<double, double, kWfUnr, false, true>;
+  // (the points travel in `half`, grad_pts in `u_out`, n_contacts in the upper bits of `want_grad`: see the kernel)
+  kernel<<<blocks, kWfWarps * 32, smem, st>>>(x, x_plus, weight, inertia, mu_pair, pts, dt, eps, B, loss, force, iters,
+                                              partials, (grad ? 1 : 0) | (n_contacts << 1), skip_flag, dyn, 13, 13, nullptr,
+                                              grad_pts, 0, 0);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;
   if (want_red) {
-    reduce_partials_kernel<double, double, kNAcc, 11><<<1, 32 * kNAcc, 0, st>>>(partials, blocks, grad, loss_sum, nullptr);
+    reduce_partials_kernel<double, double, kNAcc, 11><<<1, 32 * kNAcc, 0, st>>>(partials, blocks, grad, loss_sum, skip_flag);
     e = cudaGetLastError();
     if (e != cudaSuccess) return (int)e;
   }

@@ -157,5 +157,9 @@ class DeepSupportConvex(CollisionGeometry):
         perturbed = perturbed / perturbed.norm(dim=-1, keepdim=True)
         return self.network(perturbed)
 
+    def support_points(self, directions: Tensor) -> Tensor:
+        """The witness points for (*, 3) directions, as every shape answers them (``get_vertices``)."""
+        return self.get_vertices(directions)
+
     def scalars(self) -> Dict[str, float]:
         return {}

@@ -79,12 +79,22 @@ class MultibodyLearnableSystem(System):
 
     def _body_witness_points(self, quat: Tensor):
         """(B,4) orientations -> ((B,4,3) witness points of the body geometry against the ground, n_contacts): the
-        shape's support points in the direction -R^T e_z (geometry.py:560-567), rows beyond n_query zero."""
+        shape's support points in the direction -R^T e_z (geometry.py:560-567), rows beyond n_query zero.  A learned shape
+        (DeepSupportConvex) answers through its network at the detached orientation: its support points are piecewise
+        constant in the direction, so no gradient reaches the state through them (as the two-body system's)."""
+        from dair_pll_b200.geometry import DeepSupportConvex
         geom = self.multibody_terms.contact_terms.geometries[0]
-        w, x, y, z = quat.unbind(-1)
-        s = 2.0 / (w * w + x * x + y * y + z * z)
-        d = -torch.stack((s * (x * z - w * y), s * (y * z + w * x), 1 - s * (x * x + y * y)), -1)
-        p = place_in_link_frame(geom, d)
+        learned = isinstance(geom, DeepSupportConvex)
+        if learned:
+            quat = quat.detach()
+        if learned and geom.frame is None and quat.is_cuda and quat.dtype == torch.float64:
+            # one launch for the perturbed, normalised directions; the network then evaluates them row by row
+            p = geom.network(ops.body_support_directions(quat, geom.perturbations))
+        else:
+            w, x, y, z = quat.unbind(-1)
+            s = 2.0 / (w * w + x * x + y * y + z * z)
+            d = -torch.stack((s * (x * z - w * y), s * (y * z + w * x), 1 - s * (x * x + y * y)), -1)
+            p = place_in_link_frame(geom, d)
         n_c = p.shape[-2]
         if n_c < 4:
             p = torch.cat((p, p.new_zeros(p.shape[:-2] + (4 - n_c, 3))), -2)
@@ -159,12 +169,22 @@ class MultibodyLearnableSystem(System):
         assert x.shape[-1] == self.space.n_x and x_plus.shape == x.shape
         batch = x.shape[:-1]
         if self._kind() == 'cube' and self.multibody_terms.contact_terms.has_witness_point_geometry():
-            # Sphere / Polygon: support points evaluated here, contact set handed to the witness-point kernel
+            # Sphere / Polygon / learned geometry: support points evaluated here, contact set handed to the witness-point
+            # kernel, whose d loss / d points reaches the shape parameters (network weights) through autograd
+            if self.data_parallel is not None:
+                raise NotImplementedError('the in-kernel gradient exchange is provided for the box; use '
+                                          'parallel.GradientAllReduce (NCCL) for this geometry')
             inertia, mu, _ = self._cube_params(torch.float64)
             xf, xpf = self._flat(x).to(torch.float64), self._flat(x_plus).to(torch.float64)
             pts, n_c = self._body_witness_points(xpf[:, :4])
-            loss = ops.BodyWitnessPointLoss.apply(xf, xpf, inertia, mu, pts, n_c, float(self.dt), LOSS_EPS)
-            return loss.to(x.dtype).reshape(batch)
+            flags = ops.LOSS_DYNAMIC if self.dynamic_schedule else 0
+            loss, iters = ops.BodyWitnessPointLoss.apply(xf, xpf, inertia, mu, pts, n_c, float(self.dt), LOSS_EPS, flags,
+                                                         self.record_newton_iters)
+            out = loss.to(x.dtype).reshape(batch).as_subclass(ops.BatchLoss)
+            out._dpll_fused = None           # mean() / sum() are plain reductions: the points' gradient needs the graph
+            out.newton_iters = iters.reshape(batch) if self.record_newton_iters else None
+            out.qp_solution = None
+            return out
         if self._kind() == 'cube':
             lt, ct = self.multibody_terms.lagrangian_terms, self.multibody_terms.contact_terms
             # the learnable leaves go straight to the library (parameter preparation, multibody_terms.py:230-231,

@@ -93,9 +93,9 @@ class ContactTerms(Module):
         return any(isinstance(g, DeepSupportConvex) for g in self.geometries)
 
     def has_witness_point_geometry(self) -> bool:
-        """True if a body geometry is evaluated through its support points here (Sphere, Polygon, or any shape that sits
-        in a collision frame of its own)."""
-        return any(isinstance(g, (Sphere, Polygon)) or g.frame is not None for g in self.geometries)
+        """True if a body geometry is evaluated through its support points here (Sphere, Polygon, DeepSupportConvex, or
+        any shape that sits in a collision frame of its own)."""
+        return any(isinstance(g, (Sphere, Polygon, DeepSupportConvex)) or g.frame is not None for g in self.geometries)
 
 
 class MultibodyTerms(Module):

@@ -634,55 +634,77 @@ class ElbowStepPts(torch.autograd.Function):
                 g[20:22].reshape(mu_pair.shape).to(mu_pair.dtype), gpts.reshape(pts.shape).to(pts.dtype), None, None, None)
 
 
+def body_loss_pts_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_contacts: int, dt: float,
+                      eps: float, weight: Optional[Tensor] = None, want_grad: bool = True, want_loss: bool = True,
+                      want_grad_pts: bool = True, want_iters: bool = False, want_force: bool = False, flags: int = 0,
+                      skip_flag: Optional[Tensor] = None, grad_out: Optional[Tensor] = None):
+    """Direct call of ``dpll_body_loss_pts_f64`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,13), inertia
+    (10), mu_pair (1), witness points pts (B,4,3) of which the first ``n_contacts`` rows are used.  Returns (loss (B,) | None,
+    grad (11,) | None, loss_sum (1,), grad_pts (B,4,3) | None, iters (B,) | None, force (B,12) | None)."""
+    _check_inputs(x, x_plus, inertia, mu_pair, pts)
+    if x.dtype != torch.float64:
+        raise TypeError('the witness-point kernels are provided in float64')
+    x, x_plus, pts = x.contiguous(), x_plus.contiguous(), pts.contiguous()
+    B, dev = x.shape[0], x.device
+    if x.dim() != 2 or x.shape[1] != 13 or x_plus.shape != x.shape:
+        raise ValueError(f'expected (B,13) states, got {tuple(x.shape)} / {tuple(x_plus.shape)}')
+    if tuple(pts.shape) != (B, 4, 3):
+        raise ValueError(f'pts must be (B,4,3), got {tuple(pts.shape)}')
+    loss = torch.empty(B, dtype=x.dtype, device=dev) if want_loss else None
+    grad = (grad_out if grad_out is not None else torch.empty(11, dtype=x.dtype, device=dev)) if want_grad else None
+    loss_sum = torch.empty(1, dtype=x.dtype, device=dev)
+    gpts = torch.empty((B, 4, 3), dtype=x.dtype, device=dev) if want_grad_pts else None
+    iters = torch.empty(B, dtype=torch.int32, device=dev) if want_iters else None
+    force = torch.empty((B, 12), dtype=x.dtype, device=dev) if want_force else None
+    if weight is not None:
+        weight = weight.to(x.dtype).contiguous()
+    ws = _workspace(dev)
+    with torch.cuda.device(dev):
+        rc = _lib.load().dpll_body_loss_pts_f64(_ptr(x), _ptr(x_plus), _ptr(weight), _ptr(inertia.contiguous()),
+                                                _ptr(mu_pair.contiguous()), _ptr(pts), n_contacts, dt, eps, B, flags,
+                                                _ptr(loss), _ptr(force), _ptr(gpts), _ptr(iters), _ptr(grad), _ptr(loss_sum),
+                                                _ptr(skip_flag), _ptr(ws), ws.numel(), _stream())
+    _lib.check(rc, 'dpll_body_loss_pts')
+    return loss, grad, loss_sum, gpts, iters, force
+
+
 class BodyWitnessPointLoss(torch.autograd.Function):
     """ContactNets loss of a single floating body whose contact set is given by witness points ``pts`` (B,4,3)
-    (first ``n_contacts`` rows used) -- Sphere, Polygon, any plane-convex pair: ``dpll_body_loss_pts_f64``.
-    Differentiable w.r.t. inertia (10), mu_pair (1) and ``pts``; float64."""
+    (first ``n_contacts`` rows used) -- Sphere, Polygon, DeepSupportConvex, any plane-convex pair: ``dpll_body_loss_pts_f64``,
+    the wavefront kernel.  Differentiable w.r.t. inertia (10), mu_pair (1) and ``pts``; float64.  Returns (loss, iters):
+    ``iters`` (B,) int32 Newton directions per sample when ``want_iters``, else empty.  Backward: a uniform upstream
+    gradient scales the forward's own sums; other weights take one weighted pass, which the device skips
+    (``skip_flag``) when they are uniform after all -- no host read, so the step can be captured into a CUDA graph."""
 
     @staticmethod
-    def forward(ctx, x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps):
-        _check_inputs(x, x_plus, inertia, mu_pair, pts)
-        if x.dtype != torch.float64:
-            raise TypeError('the witness-point kernels are provided in float64')
-        x, x_plus, pts = x.contiguous(), x_plus.contiguous(), pts.contiguous()
-        B, dev = x.shape[0], x.device
-        if tuple(pts.shape) != (B, 4, 3):
-            raise ValueError(f'pts must be (B,4,3), got {tuple(pts.shape)}')
-        loss = torch.empty(B, dtype=x.dtype, device=dev)
-        grad = torch.empty(11, dtype=x.dtype, device=dev)
-        loss_sum = torch.empty(1, dtype=x.dtype, device=dev)
-        gpts = torch.empty((B, 4, 3), dtype=x.dtype, device=dev)
-        ws = _workspace(dev)
-        with torch.cuda.device(dev):
-            rc = _lib.load().dpll_body_loss_pts_f64(_ptr(x), _ptr(x_plus), None, _ptr(inertia.contiguous()),
-                                                    _ptr(mu_pair.contiguous()), _ptr(pts), n_contacts, dt, eps, B,
-                                                    _ptr(loss), None, _ptr(gpts), None, _ptr(grad), _ptr(loss_sum),
-                                                    _ptr(ws), ws.numel(), _stream())
-        _lib.check(rc, 'dpll_body_loss_pts')
-        ctx.args = (n_contacts, dt, eps)
+    def forward(ctx, x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, flags=0, want_iters=False):
+        loss, grad, _, gpts, iters, _ = body_loss_pts_raw(x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, flags=flags,
+                                                          want_iters=want_iters)
+        ctx.args = (n_contacts, dt, eps, flags)
         ctx.shapes = (inertia.shape, mu_pair.shape)
         ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts)
-        return loss
+        if iters is None:
+            iters = torch.empty(0, dtype=torch.int32, device=loss.device)
+        ctx.mark_non_differentiable(iters)
+        return loss, iters
 
     @staticmethod
-    def backward(ctx, grad_loss):
+    def backward(ctx, grad_loss, _g_iters):
         grad, gpts, x, x_plus, inertia, mu_pair, pts = ctx.saved_tensors
-        n_contacts, dt, eps = ctx.args
-        grad_loss = grad_loss.contiguous()
-        B, dev = x.shape[0], x.device
-        # general upstream weights: one weighted pass (these shapes are not on a benchmark configuration)
-        g = torch.zeros_like(grad)
-        if B > 0:
-            ws = _workspace(dev)
-            with torch.cuda.device(dev):
-                rc = _lib.load().dpll_body_loss_pts_f64(_ptr(x), _ptr(x_plus), _ptr(grad_loss), _ptr(inertia.contiguous()),
-                                                        _ptr(mu_pair.contiguous()), _ptr(pts), n_contacts, dt, eps, B,
-                                                        None, None, None, None, _ptr(g), None, _ptr(ws), ws.numel(),
-                                                        _stream())
-            _lib.check(rc, 'dpll_body_loss_pts')
+        n_contacts, dt, eps, flags = ctx.args
+        if grad_loss.dim() == 1 and grad_loss.numel() > 0 and grad_loss.stride(0) == 0:
+            g = grad * grad_loss[0]
+        else:
+            grad_loss = grad_loss.contiguous()
+            lo, hi = torch.aminmax(grad_loss) if grad_loss.numel() > 0 else (grad_loss.new_zeros(()), grad_loss.new_zeros(()))
+            uniform = lo == hi
+            gw = torch.zeros_like(grad)
+            body_loss_pts_raw(x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, weight=grad_loss, want_loss=False,
+                              want_grad_pts=False, flags=flags, skip_flag=uniform.to(torch.int32), grad_out=gw)
+            g = torch.where(uniform, grad * lo, gw)
         s_in, s_mu = ctx.shapes
         return (None, None, g[0:10].reshape(s_in), g[10:11].reshape(s_mu), gpts * grad_loss.reshape(-1, 1, 1), None, None,
-                None)
+                None, None, None)
 
 
 def body_step_pts(x: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_contacts: int, dt: float,
@@ -995,6 +1017,23 @@ def elbow_support_directions(q: Tensor, axis: Tensor, pert0: Tensor, pert1: Tens
                                                            _ptr(d0), _ptr(d1), _stream())
     _lib.check(rc, 'dpll_elbow_support_directions')
     return d0, d1
+
+
+def body_support_directions(q: Tensor, pert: Tensor) -> Tensor:
+    """``dpll_body_support_directions_f64``: q (B, >= 4) rows (any row stride, quaternion first) -> the body's perturbed,
+    normalised support directions (B, n_query, 3) against the ground.  float64, no autograd (directions are data)."""
+    _check_inputs(q, pert)
+    if q.dtype != torch.float64:
+        raise TypeError('the support-network kernels are provided in float64')
+    if q.dim() != 2 or q.shape[1] < 4 or q.stride(1) != 1:
+        raise ValueError(f'expected (B, >= 4) configuration rows with unit column stride, got {tuple(q.shape)}')
+    B, nq = q.shape[0], pert.shape[0]
+    d = torch.empty((B, nq, 3), dtype=q.dtype, device=q.device)
+    with torch.cuda.device(q.device):
+        rc = _lib.load().dpll_body_support_directions_f64(_ptr(q), q.stride(0) if B > 1 else q.shape[1],
+                                                          _ptr(pert.contiguous()), nq, B, _ptr(d), _stream())
+    _lib.check(rc, 'dpll_body_support_directions')
+    return d
 
 
 def icnn_support_points(d: Tensor, Wd0: Tensor, Wd1: Tensor, Wh: Tensor, wout: Tensor, slope: float) -> Tensor:

@@ -225,9 +225,9 @@ class SystemSpec:
         if kind == 'cube':
             if len(geometries) != 1:
                 raise NotImplementedError('the single-body kernels take exactly one collision geometry')
-            if geometries[0].kind not in ('box', 'sphere'):
-                raise NotImplementedError('the single-body kernels take a <box> or <sphere> collision geometry '
-                                          '(a Polygon is set through the module API)')
+            if geometries[0].kind not in ('box', 'sphere', 'mesh'):
+                raise NotImplementedError('the single-body kernels take a <box>, <sphere> or <mesh> (learned geometry) '
+                                          'collision geometry (a Polygon is set through the module API)')
             # a collision frame that differs from the link frame (offset and / or rotation) is handled through the
             # witness-point kernels: the contact points are support points of the shape, moved into the link frame
         elif kind == 'chain':

@@ -1,14 +1,18 @@
 """ContactNets parameter learning from simulated tosses -- the B200 counterpart of the reference's
 ``examples/contactnets_simple.py`` (BASELINE config 1), with the reference's settings (256 tosses of 80 / 120 steps
 sampled uniformly around CUBE_X_0 / ELBOW_X_0, dt = 0.0068, Adam, lr 1e-3, batch 256; contactnets_simple.py:52-86),
-for the cube and the two-body elbow (box geometries), with the ContactNets loss or the prediction loss.
+for the cube and the two-body elbow, with box geometries or learned (mesh, ``DeepSupportConvex``) ones, with the
+ContactNets loss or the prediction loss.
 
 The reference generates its ground truth with Drake; here the ground-truth tosses come from the learnable system
 itself at the URDF's parameters (the same Anitescu step, multibody_learnable_system.py:199-304), and the learned
 system starts from perturbed inertia / friction / geometry.  Everything after data generation stays on the GPU:
 trajectories -> ``DeviceTrajectorySliceDataset`` -> ``contactnets_loss(...).mean().backward()`` -> Adam.
 
-    python examples/contactnets_simple.py --epochs 200 [--system elbow] [--prediction --t-prediction 2]
+    python examples/contactnets_simple.py --epochs 200 [--system elbow] [--geometry mesh] [--prediction --t-prediction 2]
+
+With ``--geometry mesh`` the ground truth is still the box system; the learned system's geometry is a support-function
+network initialised from the box's mesh (cube_mesh.urdf / elbow_mesh.urdf), as in the reference's *_mesh experiments.
 """
 import argparse
 import math
@@ -37,6 +41,8 @@ SAMPLER_RANGES = {'cube': CUBE_SAMPLER_RANGE, 'elbow': ELBOW_SAMPLER_RANGE}
 TRAJECTORY_LENGTHS = {'cube': 80, 'elbow': 120}
 URDFS = {'cube': os.path.join(ROOT, 'dair_pll_b200', 'assets', 'cube.urdf'),
          'elbow': os.path.join(ROOT, 'dair_pll_b200', 'assets', 'elbow.urdf')}
+MESH_URDFS = {'cube': os.path.join(ROOT, 'dair_pll_b200', 'assets', 'cube_mesh.urdf'),
+              'elbow': os.path.join(ROOT, 'dair_pll_b200', 'assets', 'elbow_mesh.urdf')}
 
 
 def sample_initial_states(system, kind: str, n: int, seed: int, device) -> torch.Tensor:
@@ -61,7 +67,7 @@ def parameter_report(system) -> dict:
 
 def run(epochs: int = 100, n_pop: int = N_POP, batch_size: int = 256, lr: float = 1e-3, seed: int = 0,
         perturbation: float = 0.3, device: str = 'cuda:0', verbose: bool = True, contactnets: bool = True,
-        t_prediction: int = 1, system: str = 'cube') -> dict:
+        t_prediction: int = 1, system: str = 'cube', geometry: str = 'box') -> dict:
     """``contactnets=False`` trains on the prediction loss instead (experiment.py:292-320: mean squared velocity
     error of the ``t_prediction``-step rollout from the last past state), differentiating through every step's
     QP (``simulate`` -> ``dpll_cube_rollout_grad_f64``)."""
@@ -75,7 +81,7 @@ def run(epochs: int = 100, n_pop: int = N_POP, batch_size: int = 256, lr: float 
         data.add_slices_from_trajectory(traj)
 
     # the learned system starts from multiplicatively perturbed parameters of the same URDF
-    learned = MultibodyLearnableSystem({system: URDFS[system]}, DT)
+    learned = MultibodyLearnableSystem({system: (MESH_URDFS if geometry == 'mesh' else URDFS)[system]}, DT)
     gen_p = torch.Generator().manual_seed(seed + 1)
 
     def jitter(n):
@@ -127,11 +133,13 @@ if __name__ == '__main__':
     ap.add_argument('--lr', type=float, default=1e-3)
     ap.add_argument('--perturbation', type=float, default=0.3)
     ap.add_argument('--system', choices=['cube', 'elbow'], default='cube')
+    ap.add_argument('--geometry', choices=['box', 'mesh'], default='box',
+                    help='geometry of the learned system: boxes, or support-function networks initialised from them')
     ap.add_argument('--prediction', action='store_true', help='prediction loss instead of the ContactNets loss')
     ap.add_argument('--t-prediction', type=int, default=1)
     a = ap.parse_args()
     out = run(a.epochs, a.n_pop, a.batch_size, a.lr, perturbation=a.perturbation, contactnets=not a.prediction,
-              t_prediction=a.t_prediction, system=a.system)
+              t_prediction=a.t_prediction, system=a.system, geometry=a.geometry)
     print(f"{out['pairs']} pairs, {a.epochs} epochs in {out['seconds']:.1f} s")
     print('truth  ', out['truth'])
     print('learned', out['learned'])

@@ -44,7 +44,7 @@ extern "C" {
 #define DPLL_EWORKSPACE (-2) /* workspace too small */
 #define DPLL_ECOMM (-3)      /* a peer did not arrive within the exchange's timeout */
 
-#define DPLL_VERSION 213     /* bumped with every change of a signature below; the binding checks it */
+#define DPLL_VERSION 214     /* bumped with every change of a signature below; the binding checks it */
 
 #define DPLL_CUBE_NX 13
 #define DPLL_CUBE_NC 4
@@ -239,6 +239,13 @@ int dpll_elbow_support_directions_f64(const double* q, int64_t q_stride, const d
                                       void* stream);
 
 /*
+ * The same for a single floating body whose learned geometry sits in the link frame: q rows of >= 4 values (the
+ * quaternion first) at stride q_stride, pert (n_query, 3) the geometry's fixed perturbations; dirs (B, n_query, 3).
+ */
+int dpll_body_support_directions_f64(const double* q, int64_t q_stride, const double* pert, int32_t n_query, int64_t B,
+                                     double* dirs, void* stream);
+
+/*
  * Support points on the tensor cores (csrc/cn_icnn_tc.cu; width W = 256 only): HomogeneousICNN.forward
  * (deep_support_function.py:238-266) for all D direction rows in one kernel.  The layer Jacobian d z1 / d d is a
  * (binary mask) x (constant matrix) product, evaluated exactly as int8 digit-plane products by tcgen05.mma with int32
@@ -282,14 +289,21 @@ int dpll_icnn_tc_bwd_f64(const double* gp, const int64_t* n_rows, const double* 
  * points in the direction -R^T e_z -- Sphere: 1 point d r (geometry.py:415-456); Polygon: the top-n_query vertices
  * (geometry.py:220-252, 162-202); Box / DeepSupportConvex likewise -- as pts (B, 4, 3) in the geometry frame, of
  * which the first n_contacts (1..4) rows are used, and gets the loss, the gradient w.r.t. [inertia 10 | mu_pair]
- * (grad, 11) and grad_pts (B, 4, 3) = w_b d loss_b / d pts[b] back (rows >= n_contacts zero).  One sample per
- * thread (these shapes are not on a benchmark configuration; the box keeps its wavefront kernel).
+ * (grad, 11) and grad_pts (B, 4, 3) = w_b d loss_b / d pts[b] back (rows >= n_contacts zero).  The box's wavefront
+ * kernel runs it (its witness-point instance: free-flight triage, Newton visits over shared-memory slots), so per-sample
+ * losses, forces, grad_pts and iteration counts do not depend on `flags`:
+ *   flags     : DPLL_LOSS_DYNAMIC as for dpll_cube_loss_leaf_dp_f64 (32-sample chunks in batch order, for cost-ordered
+ *               batches; the gradient sums are then rounded in a timing-dependent order); other bits are ignored.
+ *   skip_flag : (nullable, device) when *skip_flag != 0 every launch returns at once and writes nothing -- the weighted
+ *               backward pass of a uniform upstream gradient, decided on the device so that the step can be captured
+ *               into a CUDA graph.
  * dpll_body_step_pts_f64: one learnable time step x -> x_next with the same contact set.
  */
 int dpll_body_loss_pts_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
                            const double* mu_pair, const double* pts, int32_t n_contacts, double dt, double eps,
-                           int64_t B, double* loss, double* force, double* grad_pts, int32_t* iters, double* grad,
-                           double* loss_sum, void* workspace, size_t workspace_bytes, void* stream);
+                           int64_t B, int32_t flags, double* loss, double* force, double* grad_pts, int32_t* iters,
+                           double* grad, double* loss_sum, const int32_t* skip_flag, void* workspace,
+                           size_t workspace_bytes, void* stream);
 int dpll_body_step_pts_f64(const double* x, const double* inertia, const double* mu_pair, const double* pts,
                            int32_t n_contacts, double dt, double eps, int64_t B, double* x_next, double* force,
                            void* stream);
