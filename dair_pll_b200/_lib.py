@@ -5,86 +5,49 @@ caller gets an exception.  The library is built in-tree by ``dair_pll_b200.build
 """
 import ctypes
 import os
+import re
 
 from dair_pll_b200 import build as _build
 
 _LIB = None
 ABI_VERSION = 214        # DPLL_VERSION of include/dair_pll_b200.h this binding was written against
+HEADER = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'include', 'dair_pll_b200.h')
 
-_c_void_p = ctypes.c_void_p
-_i64, _i32, _f64, _f32, _sz = ctypes.c_int64, ctypes.c_int32, ctypes.c_double, ctypes.c_float, ctypes.c_size_t
+_SCALARS = {'double': ctypes.c_double, 'float': ctypes.c_float, 'int': ctypes.c_int32, 'int32_t': ctypes.c_int32,
+            'int64_t': ctypes.c_int64, 'uint32_t': ctypes.c_uint32, 'size_t': ctypes.c_size_t}
 
-EXPORTS = {
-    'dpll_version': ([], ctypes.c_int),
-    'dpll_workspace_bytes': ([], _sz),
-    'dpll_set_loss_variant': ([ctypes.c_int], ctypes.c_int),
-    'dpll_cube_loss_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64] + [_c_void_p] * 6 + [_c_void_p, _sz, _c_void_p],
-                           ctypes.c_int),
-    'dpll_cube_loss_f32': ([_c_void_p] * 6 + [_f32, _f32, _i64] + [_c_void_p] * 6 + [_c_void_p, _sz, _c_void_p],
-                           ctypes.c_int),
-    'dpll_cube_loss_leaf_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64] + [_c_void_p] * 6 + [_c_void_p, _sz, _c_void_p],
-                                ctypes.c_int),
-    'dpll_cube_loss_leaf_f32': ([_c_void_p] * 6 + [_f32, _f32, _i64] + [_c_void_p] * 6 + [_c_void_p, _sz, _c_void_p],
-                                ctypes.c_int),
-    'dpll_cube_rollout_f64': ([_c_void_p] * 4 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_cube_rollout_f32': ([_c_void_p] * 4 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_cube_terms_f64': ([_c_void_p] * 5 + [_i64] + [_c_void_p] * 6, ctypes.c_int),
-    'dpll_body_loss_pts_f64': ([_c_void_p] * 6 + [_i32, _f64, _f64, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p],
-                               ctypes.c_int),
-    'dpll_body_step_pts_f64': ([_c_void_p] * 4 + [_i32, _f64, _f64, _i64] + [_c_void_p] * 3, ctypes.c_int),
-    'dpll_chain_loss_f64': ([_i32] + [_c_void_p] * 7 + [_f64, _f64, _i64] + [_c_void_p] * 5 + [_c_void_p, _sz, _c_void_p],
-                            ctypes.c_int),
-    'dpll_chain_rollout_f64': ([_i32] + [_c_void_p] * 5 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 2, ctypes.c_int),
-    'dpll_elbow_terms_f64': ([_c_void_p] * 6 + [_i64] + [_c_void_p] * 6, ctypes.c_int),
-    'dpll_chain_loss_pts_f64': ([ctypes.c_int32] + [_c_void_p] * 7 + [ctypes.c_uint32, ctypes.c_double, ctypes.c_double, _i64]
-                                + [_c_void_p] * 5 + [ctypes.c_size_t, _c_void_p], ctypes.c_int),
-    'dpll_chain_terms_f64': ([ctypes.c_int32] * 2 + [_c_void_p] * 6 + [_i64] + [_c_void_p] * 6, ctypes.c_int),
-    'dpll_cube_rollout_grad_f64': ([_c_void_p] * 4 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_cube_rollout_saved_f64': ([_c_void_p] * 4 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 3, ctypes.c_int),
-    'dpll_cube_rollout_backward_f64': ([_c_void_p] * 5 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_elbow_loss_f64': ([_c_void_p] * 8 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_elbow_loss_f32': ([_c_void_p] * 8 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 7 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_elbow_rollout_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_elbow_rollout_f32': ([_c_void_p] * 6 + [_f32, _f32, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_icnn_input_f64': ([_c_void_p, _c_void_p, _i64, _i32, _f64, _c_void_p, _c_void_p], ctypes.c_int),
-    'dpll_icnn_mask_f64': ([_c_void_p, _i64, _f64, _c_void_p], ctypes.c_int),
-    'dpll_icnn_output_f64': ([_c_void_p] * 5 + [_i64, _i32, _f64, _c_void_p, _c_void_p], ctypes.c_int),
-    'dpll_elbow_support_directions_f64': ([_c_void_p, _i64] + [_c_void_p] * 3 + [_i32, _i64] + [_c_void_p] * 3, ctypes.c_int),
-    'dpll_body_support_directions_f64': ([_c_void_p, _i64, _c_void_p, _i32, _i64, _c_void_p, _c_void_p], ctypes.c_int),
-    'dpll_icnn_tc_image_bytes': ([], ctypes.c_size_t),
-    'dpll_icnn_tc_const_bytes': ([], ctypes.c_size_t),
-    'dpll_icnn_tc_prepare_f64': ([_c_void_p] * 4 + [_i32, _f64, _c_void_p, _c_void_p, _c_void_p], ctypes.c_int),
-    'dpll_icnn_tc_support_f64': ([_c_void_p, _i64, _c_void_p, _c_void_p, _c_void_p, _i32, _f64, _c_void_p, _c_void_p],
-                                 ctypes.c_int),
-    'dpll_icnn_tc_bwd_partial_bytes': ([], ctypes.c_size_t),
-    'dpll_icnn_tc_bwd_planes': ([], ctypes.c_int32),
-    'dpll_icnn_tc_record_f64': ([_c_void_p, _i64, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _i32, _f64, _c_void_p, _c_void_p,
-                                 _i64, _c_void_p], ctypes.c_int),
-    'dpll_icnn_tc_bwd_f64': ([_c_void_p] * 5 + [_i64, _f64] + [_c_void_p] * 5, ctypes.c_int),
-    'dpll_icnn_backward_blocks': ([_i64], ctypes.c_int),
-    'dpll_icnn_backward_f64': ([_c_void_p] * 5 + [_i64, _i32, _f64, _c_void_p, _c_void_p, _c_void_p], ctypes.c_int),
-    'dpll_cube_loss_leaf_dp_f64': ([_c_void_p, _i64, _c_void_p, _i64] + [_c_void_p] * 3 + [_f64, _f64, _i64, _i32] +
-                                   [_c_void_p] * 8 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_cube_loss_leaf_dp_f32': ([_c_void_p, _i64, _c_void_p, _i64] + [_c_void_p] * 3 + [_f32, _f32, _i64, _i32] +
-                                   [_c_void_p] * 8 + [_c_void_p, _sz, _c_void_p], ctypes.c_int),
-    'dpll_comm_handle_bytes': ([], _sz),
-    'dpll_comm_create': ([_i32, _i32, ctypes.POINTER(_c_void_p), _c_void_p], ctypes.c_int),
-    'dpll_comm_connect': ([_c_void_p, _c_void_p], ctypes.c_int),
-    'dpll_comm_destroy': ([_c_void_p], ctypes.c_int),
-    'dpll_comm_device_state': ([_c_void_p], _c_void_p),
-    'dpll_comm_error': ([_c_void_p], ctypes.c_int),
-    'dpll_comm_allreduce_f64': ([_c_void_p, _c_void_p, _i32, _f64, _c_void_p], ctypes.c_int),
-    'dpll_elbow_step_pts_grad_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64] + [_c_void_p] * 5, ctypes.c_int),
-    'dpll_elbow_rollout_saved_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 3, ctypes.c_int),
-    'dpll_elbow_rollout_grad_saved_f64': ([_c_void_p] * 6 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_body_step_pts_grad_f64': ([_c_void_p] * 4 + [_i32, _f64, _f64, _i64] + [_c_void_p] * 5, ctypes.c_int),
-    'dpll_chain_rollout_grad_f64': ([_i32] + [_c_void_p] * 5 + [_f64, _f64, _i64, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_leaf_prepare_f64': ([_c_void_p, _i32, _c_void_p, _c_void_p, _c_void_p, _i32, _c_void_p, _i32] + [_c_void_p] * 4, ctypes.c_int),
-    'dpll_leaf_backward_f64': ([_c_void_p, _i32, _c_void_p, _i32, _c_void_p, _c_void_p, _i32, _c_void_p, _i32] + [_c_void_p] * 7,
-                               ctypes.c_int),
-    'dpll_fma_peak_f64': ([_c_void_p, _i32, _i64, _c_void_p], ctypes.c_int),
-    'dpll_fma_peak_f32': ([_c_void_p, _i32, _i64, _c_void_p], ctypes.c_int),
-}
+
+def _ctype(decl: str, where: str):
+    """ctypes type of a C declaration (``const double* x``, ``void** comm_out``, ``size_t``): any single pointer is a
+    ``c_void_p`` (the binding passes ``data_ptr()`` integers), ``void**`` a pointer to one.  Anything else (arrays,
+    other scalar types, deeper pointers) raises."""
+    stars = decl.count('*')
+    base = decl.replace('*', ' ').replace('const', ' ').split()[0]
+    if '[' not in decl:
+        if stars == 1:
+            return ctypes.c_void_p
+        if stars == 2 and base == 'void':
+            return ctypes.POINTER(ctypes.c_void_p)
+        if stars == 0 and base in _SCALARS:
+            return _SCALARS[base]
+    raise TypeError(f'{where}: no ctypes mapping for C type {decl.strip()!r}')
+
+
+def _signatures(path: str = HEADER) -> dict:
+    """name -> (argtypes, restype) of every ``dpll_*`` prototype of the C header.  The argtypes are positional, so they
+    are read from the header the library is compiled against instead of being restated here."""
+    with open(path) as f:
+        text = re.sub(r'/\*.*?\*/|//[^\n]*', ' ', f.read(), flags=re.S)
+    text = re.sub(r'^\s*#[^\n]*', ' ', text, flags=re.M)
+    out = {}
+    for ret, name, params in re.findall(r'([\w\s*]+?)\b(dpll_\w+)\s*\(([^)]*)\)\s*;', text):
+        params = [p for p in params.split(',') if p.strip() not in ('', 'void')]
+        where = f'{name} in {path}'
+        out[name] = ([_ctype(p, where) for p in params], _ctype(ret, where))
+    return out
+
+
+EXPORTS = _signatures()
 
 
 def lib_path() -> str:

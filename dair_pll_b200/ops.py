@@ -4,6 +4,7 @@ These are the seam between the unchanged Python host API
 (:class:`dair_pll_b200.multibody_learnable_system.MultibodyLearnableSystem`) and the
 sm_100a kernels.  Tensors must be CUDA, contiguous, fp64 or fp32; there is no CPU path.
 """
+from collections import namedtuple
 from typing import Optional, Tuple
 
 import torch
@@ -15,17 +16,9 @@ _SUFFIX = {torch.float64: 'f64', torch.float32: 'f32'}
 _workspaces = {}
 
 
-def _ptr(t: Optional[Tensor]):
-    return None if t is None else t.data_ptr()
-
-
-def _stream() -> int:
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _workspace(device: torch.device) -> Tensor:
+def _workspace(device: torch.device, stream: int) -> Tensor:
     """Per-(device, stream) scratch for the gradient reduction (the library never allocates)."""
-    key = (device.index, _stream())
+    key = (device.index, stream)
     ws = _workspaces.get(key)
     if ws is None:
         ws = torch.empty(_lib.load().dpll_workspace_bytes(), dtype=torch.uint8, device=device)
@@ -33,15 +26,36 @@ def _workspace(device: torch.device) -> Tensor:
     return ws
 
 
+def _call(name: str, device, *args, dtype: Optional[torch.dtype] = None, workspace: bool = False) -> None:
+    """Calls the C entry point ``name`` -- ``name_f64`` / ``name_f32`` when ``dtype`` is given -- on ``device``'s current
+    stream, which every entry point takes last; tensors are passed as their data pointers, ``None`` as NULL.  With
+    ``workspace`` the device's scratch buffer and its size go before the stream.  A non-zero return code raises.
+    ``args`` stays referenced until the entry point has been enqueued: callers pass temporaries (casts, contiguous
+    copies) inline, and the caching allocator must not hand their memory out before the launch is on the stream."""
+    if dtype is not None:
+        name = f'{name}_{_SUFFIX[dtype]}'
+    ptrs = [a.data_ptr() if isinstance(a, Tensor) else a for a in args]
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream().cuda_stream
+        if workspace:
+            ws = _workspace(device, stream)
+            ptrs += [ws.data_ptr(), ws.numel()]
+        _lib.check(getattr(_lib.load(), name)(*ptrs, stream), name)
+
+
 def set_loss_variant(variant: int) -> None:
     """Selects the cube loss kernel: 0 = warp-level wavefront kernel, static sample ranges (default; bitwise
     reproducible), 1 = one sample per thread (A/B measurements), 2 = wavefront kernel with dynamic sample distribution
     (faster by the load imbalance, gradient sums reproducible only to rounding).  The elbow loss always runs its
     wavefront kernel."""
+    # a process-wide setting, not a launch: no device and no stream, so not through _call
     _lib.check(_lib.load().dpll_set_loss_variant(variant), 'dpll_set_loss_variant')
 
 
-def _check_inputs(*tensors: Tensor) -> torch.dtype:
+def _check_inputs(*tensors: Optional[Tensor], f64_only: Optional[str] = None) -> torch.dtype:
+    """The common dtype of the CUDA tensors given (``None`` entries are skipped); ``f64_only``: the message of the
+    TypeError raised when it is not float64."""
+    tensors = [t for t in tensors if t is not None]
     dtype = tensors[0].dtype
     if dtype not in _SUFFIX:
         raise TypeError(f'dair_pll_b200 kernels support float64/float32, got {dtype}')
@@ -50,7 +64,64 @@ def _check_inputs(*tensors: Tensor) -> torch.dtype:
             raise RuntimeError('dair_pll_b200 has no CPU path: tensors must live on a CUDA device')
         if t.dtype != dtype:
             raise TypeError(f'mixed dtypes: {t.dtype} vs {dtype}')
+    if f64_only is not None and dtype != torch.float64:
+        raise TypeError(f64_only)
     return dtype
+
+
+def _check_states(n_x: int, x: Tensor, x_plus: Optional[Tensor] = None) -> None:
+    if x.dim() != 2 or x.shape[1] != n_x or (x_plus is not None and x_plus.shape != x.shape):
+        got = tuple(x.shape) if x_plus is None else f'{tuple(x.shape)} / {tuple(x_plus.shape)}'
+        raise ValueError(f'expected (B,{n_x}) states, got {got}')
+
+
+_Like = namedtuple('_Like', 'shape dtype')      # what _split reads of a tensor
+
+
+def _split(g: Tensor, *like) -> list:
+    """Consecutive pieces of the flat gradient ``g``, one per tensor (or :class:`_Like`) of ``like``, with its shape and
+    dtype."""
+    out, off = [], 0
+    for t in like:
+        n = t.shape.numel()
+        out.append(g[off:off + n].reshape(t.shape).to(t.dtype))
+        off += n
+    return out
+
+
+def _fused_grad(grad: Tensor, grad_loss: Tensor, rerun) -> Tensor:
+    """Parameter gradient of sum_b grad_loss[b] loss_b for a loss whose forward launch already returned
+    ``grad`` = d(sum_b loss_b)/d params (envelope theorem).  A stride-0 upstream gradient (``loss.sum()``) is provably
+    uniform: one scale.  Otherwise (``loss.mean()`` materialises its uniform gradient) uniformity is decided on the
+    DEVICE: ``rerun(weight, skip_flag, grad_out)`` launches the weighted pass, which the kernel skips when the int32
+    ``skip_flag`` is set, and the scaled fused gradient is selected.  No host read, so the backward can be captured
+    into a CUDA graph."""
+    if grad_loss.numel() == 0:
+        return torch.zeros_like(grad)
+    if grad_loss.dim() == 1 and grad_loss.stride(0) == 0:
+        return grad * grad_loss[0]
+    grad_loss = grad_loss.contiguous()
+    lo, hi = torch.aminmax(grad_loss)
+    uniform = lo == hi
+    gw = torch.zeros_like(grad)
+    rerun(grad_loss, uniform.to(torch.int32), gw)
+    return torch.where(uniform, grad * lo, gw)
+
+
+def _f64(t: Optional[Tensor]) -> Optional[Tensor]:
+    return None if t is None else t.detach().to(torch.float64).contiguous()
+
+
+def _summed_backward(name: str, x: Tensor, params, widths, *args, steps: int = 1):
+    """Backward through a rollout or step entry point ``name`` that writes PER-SAMPLE gradients: it is called with
+    ``args`` (tensors cast to contiguous float64) followed by zeroed float64 (B, w) buffers, one per entry of
+    ``widths``, the parameter gradient first; an empty batch or rollout launches nothing.  Returns the parameter
+    gradient summed over the batch and split as ``params``, then the other buffers."""
+    B = x.shape[0]
+    bufs = [torch.zeros((B, w), dtype=torch.float64, device=x.device) for w in widths]
+    if B > 0 and steps > 0:
+        _call(name, x.device, *(_f64(a) if isinstance(a, Tensor) else a for a in args), *bufs)
+    return (*_split(bufs[0].sum(0), *params), *bufs[1:])
 
 
 def cube_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, dt: float,
@@ -62,8 +133,7 @@ def cube_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, h
     dtype = _check_inputs(x, x_plus, inertia, mu_pair, half)
     x, x_plus = x.contiguous(), x_plus.contiguous()
     inertia, mu_pair, half = inertia.contiguous(), mu_pair.contiguous(), half.contiguous()
-    if x.dim() != 2 or x.shape[1] != 13 or x_plus.shape != x.shape:
-        raise ValueError(f'expected (B,13) states, got {tuple(x.shape)} / {tuple(x_plus.shape)}')
+    _check_states(13, x, x_plus)
     if inertia.numel() != 10 or mu_pair.numel() != 1 or half.numel() != 3:
         raise ValueError('cube parameters must be inertia (10), mu_pair (1), half (3)')
     B = x.shape[0]
@@ -75,13 +145,8 @@ def cube_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, h
     iters = torch.empty(B, dtype=torch.int32, device=dev) if want_iters else None
     if weight is not None:
         weight = weight.to(dtype).contiguous()
-    ws = _workspace(dev)
-    fn = getattr(_lib.load(), 'dpll_cube_loss_' + _SUFFIX[dtype])
-    with torch.cuda.device(dev):
-        rc = fn(_ptr(x), _ptr(x_plus), _ptr(weight), _ptr(inertia), _ptr(mu_pair), _ptr(half), dt, eps, B,
-                _ptr(loss), _ptr(force), _ptr(iters), _ptr(grad), _ptr(loss_sum), _ptr(skip_flag), _ptr(ws), ws.numel(),
-                _stream())
-    _lib.check(rc, 'dpll_cube_loss')
+    _call('dpll_cube_loss', dev, x, x_plus, weight, inertia, mu_pair, half, dt, eps, B, loss, force, iters, grad, loss_sum,
+          skip_flag, dtype=dtype, workspace=True)
     return loss, grad, loss_sum, force, iters
 
 
@@ -102,7 +167,6 @@ class CubeContactNetsLoss(torch.autograd.Function):
         need = any(ctx.needs_input_grad[2:5])
         loss, grad, _, _, _ = cube_loss_raw(x, x_plus, inertia, mu_pair, half, dt, eps, want_grad=need)
         ctx.dt, ctx.eps = dt, eps
-        ctx.shapes = (inertia.shape, mu_pair.shape, half.shape)
         if need:
             ctx.save_for_backward(grad, x, x_plus, inertia, mu_pair, half)
         return loss
@@ -110,23 +174,9 @@ class CubeContactNetsLoss(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_loss):
         grad, x, x_plus, inertia, mu_pair, half = ctx.saved_tensors
-        if grad_loss.numel() == 0:
-            g = torch.zeros_like(grad)
-        elif grad_loss.dim() == 1 and grad_loss.stride(0) == 0:
-            g = grad * grad_loss[0]                      # loss.sum(): stride-0 expansion, provably uniform
-        else:
-            # loss.mean() materialises its (uniform) upstream gradient.  Decide on the DEVICE whether
-            # it is uniform: if so the weighted re-evaluation below turns into a no-op (skip flag) and
-            # the fused gradient from the forward launch is scaled; no host synchronisation.
-            grad_loss = grad_loss.contiguous()
-            lo, hi = torch.aminmax(grad_loss)
-            uniform = lo == hi
-            gw = torch.zeros_like(grad)
-            cube_loss_raw(x, x_plus, inertia, mu_pair, half, ctx.dt, ctx.eps, weight=grad_loss, want_grad=True,
-                          want_loss=False, skip_flag=uniform.to(torch.int32), grad_out=gw)
-            g = torch.where(uniform, grad * lo, gw)
-        s_in, s_mu, s_h = ctx.shapes
-        return (None, None, g[0:10].reshape(s_in), g[10:11].reshape(s_mu), g[11:14].reshape(s_h), None, None)
+        g = _fused_grad(grad, grad_loss, lambda w, skip, out: cube_loss_raw(
+            x, x_plus, inertia, mu_pair, half, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip, grad_out=out))
+        return (None, None, *_split(g, inertia, mu_pair, half), None, None)
 
 
 LOSS_DYNAMIC = 1     # DPLL_LOSS_DYNAMIC (include/dair_pll_b200.h)
@@ -154,8 +204,7 @@ def cube_loss_leaf_raw(x: Tensor, x_plus: Tensor, theta: Tensor, friction: Tenso
     dtype = _check_inputs(x, x_plus, theta, friction, length)
     x, x_plus = x.contiguous(), x_plus.contiguous()
     theta, friction, length = theta.contiguous(), friction.contiguous(), length.contiguous()
-    if x.dim() != 2 or x.shape[1] != 13 or x_plus.shape != x.shape:
-        raise ValueError(f'expected (B,13) states, got {tuple(x.shape)} / {tuple(x_plus.shape)}')
+    _check_states(13, x, x_plus)
     if theta.numel() != 10 or friction.numel() != 2 or length.numel() != 3:
         raise ValueError('cube leaves must be theta (10), friction_params (2), length_params (3)')
     B = x.shape[0]
@@ -165,12 +214,8 @@ def cube_loss_leaf_raw(x: Tensor, x_plus: Tensor, theta: Tensor, friction: Tenso
     loss_sum = torch.empty(1, dtype=dtype, device=dev)
     if weight is not None:
         weight = weight.to(dtype).contiguous()
-    ws = _workspace(dev)
-    fn = getattr(_lib.load(), 'dpll_cube_loss_leaf_' + _SUFFIX[dtype])
-    with torch.cuda.device(dev):
-        rc = fn(_ptr(x), _ptr(x_plus), _ptr(weight), _ptr(theta), _ptr(friction), _ptr(length), dt, eps, B,
-                _ptr(loss), None, None, _ptr(grad), _ptr(loss_sum), _ptr(skip_flag), _ptr(ws), ws.numel(), _stream())
-    _lib.check(rc, 'dpll_cube_loss_leaf')
+    _call('dpll_cube_loss_leaf', dev, x, x_plus, weight, theta, friction, length, dt, eps, B, loss, None, None, grad,
+          loss_sum, skip_flag, dtype=dtype, workspace=True)
     return loss, grad, loss_sum
 
 
@@ -202,13 +247,9 @@ def cube_loss_leaf_dp_raw(x: Tensor, x_plus: Tensor, theta: Tensor, friction: Te
     # with a warm start the optima are written back IN PLACE (every sample reads its row before it writes it): a
     # training loop keeps one (B, 6) buffer per batch and nothing is copied between epochs
     u_out = (u_init if u_init is not None else torch.empty((B, 6), dtype=dtype, device=dev)) if want_u else None
-    ws = _workspace(dev)
-    fn = getattr(_lib.load(), 'dpll_cube_loss_leaf_dp_' + _SUFFIX[dtype])
-    with torch.cuda.device(dev):
-        rc = fn(_ptr(x), ldx, _ptr(x_plus), ldxp, _ptr(theta), _ptr(friction), _ptr(length), dt, eps, B, flags,
-                comm.handle if comm is not None else None, _ptr(u_init), _ptr(u_out), _ptr(loss), _ptr(iters),
-                _ptr(sums), _ptr(means), _ptr(local), _ptr(ws), ws.numel(), _stream())
-    _lib.check(rc, 'dpll_cube_loss_leaf_dp')
+    _call('dpll_cube_loss_leaf_dp', dev, x, ldx, x_plus, ldxp, theta, friction, length, dt, eps, B, flags,
+          comm.handle if comm is not None else None, u_init, u_out, loss, iters, sums, means, local, dtype=dtype,
+          workspace=True)
     if want_u:
         return loss, sums, means, local, iters, u_out
     return loss, sums, means, local, iters
@@ -234,7 +275,6 @@ class CubeContactNetsLossLeaf(torch.autograd.Function):
         # (a warm-start buffer is updated in place and not returned through autograd)
         usol = out[5] if (want_u and u_init is None) else torch.empty(0, dtype=loss.dtype, device=loss.device)
         ctx.dt, ctx.eps, ctx.comm = dt, eps, comm
-        ctx.shapes = (theta.shape, friction.shape, length.shape)
         if any(ctx.needs_input_grad[2:5]):
             ctx.save_for_backward(local, x, x_plus, theta, friction, length)
         if iters is None:
@@ -246,24 +286,11 @@ class CubeContactNetsLossLeaf(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_loss, _g_sums, _g_means, _g_iters, _g_u):
         local, x, x_plus, theta, friction, length = ctx.saved_tensors
-        grad = local[:15]
-        if grad_loss.numel() == 0:
-            g = torch.zeros_like(grad)
-        elif grad_loss.dim() == 1 and grad_loss.stride(0) == 0:
-            g = grad * grad_loss[0]
-        else:
-            grad_loss = grad_loss.contiguous()
-            lo, hi = torch.aminmax(grad_loss)
-            uniform = lo == hi
-            gw = torch.zeros_like(grad)
-            cube_loss_leaf_raw(x, x_plus, theta, friction, length, ctx.dt, ctx.eps, weight=grad_loss, want_grad=True,
-                               want_loss=False, skip_flag=uniform.to(torch.int32), grad_out=gw)
-            g = torch.where(uniform, grad * lo, gw)
+        g = _fused_grad(local[:15], grad_loss, lambda w, skip, out: cube_loss_leaf_raw(
+            x, x_plus, theta, friction, length, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip, grad_out=out))
         if ctx.comm is not None:
             g = ctx.comm.all_reduce_sum(g)
-        s_t, s_f, s_l = ctx.shapes
-        return (None, None, g[0:10].reshape(s_t), g[10:12].reshape(s_f), g[12:15].reshape(s_l), None, None, None, None,
-                None, None, None)
+        return (None, None, *_split(g, theta, friction, length), None, None, None, None, None, None, None)
 
 
 class _FusedReduction(torch.autograd.Function):
@@ -276,21 +303,15 @@ class _FusedReduction(torch.autograd.Function):
     def forward(ctx, vec, n, *leaves):
         ctx.save_for_backward(vec)
         ctx.n = n
-        ctx.shapes = [l.shape for l in leaves]
+        # only the leaves' shapes and dtypes are kept: the backward does not hold the leaves themselves (nor trip on
+        # their version counters if they are updated before it runs)
+        ctx.leaves = [_Like(l.shape, l.dtype) for l in leaves]
         return vec[n].clone()
 
     @staticmethod
     def backward(ctx, g):
         (vec,) = ctx.saved_tensors
-        gg = vec[:ctx.n] * g
-        outs, off = [], 0
-        for shape in ctx.shapes:
-            n = 1
-            for s in shape:
-                n *= s
-            outs.append(gg[off:off + n].reshape(shape))
-            off += n
-        return (None, None, *outs)
+        return (None, None, *_split(vec[:ctx.n] * g, *ctx.leaves))
 
 
 _INPLACE_DUNDERS = {'__iadd__', '__isub__', '__imul__', '__itruediv__', '__ifloordiv__', '__ipow__', '__imod__',
@@ -335,16 +356,12 @@ def cube_rollout(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, dt:
     (B,) int32, optional: total Newton iterations of every toss."""
     dtype = _check_inputs(x0, inertia, mu_pair, half)
     x0 = x0.contiguous()
-    if x0.dim() != 2 or x0.shape[1] != 13:
-        raise ValueError(f'expected (B,13) states, got {tuple(x0.shape)}')
+    _check_states(13, x0)
     B = x0.shape[0]
     traj = torch.empty((B, steps + 1, 13), dtype=dtype, device=x0.device)
     force = torch.empty((B, steps, 12), dtype=dtype, device=x0.device) if want_force else None
-    fn = getattr(_lib.load(), 'dpll_cube_rollout_' + _SUFFIX[dtype])
-    with torch.cuda.device(x0.device):
-        rc = fn(_ptr(x0), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()), _ptr(half.contiguous()),
-                dt, eps, B, steps, _ptr(traj), _ptr(force), _ptr(iters_out), _stream())
-    _lib.check(rc, 'dpll_cube_rollout')
+    _call('dpll_cube_rollout', x0.device, x0, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(), dt, eps, B,
+          steps, traj, force, iters_out, dtype=dtype)
     return traj, force
 
 
@@ -356,14 +373,12 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
     """Direct call of ``dpll_elbow_loss_*`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,15); inertia (20), mu_pair (2), half (6) or
     witness points pts (B,8,3), kin (12).  Returns (loss (B,) | None, grad (28,) | None, loss_sum (1,),
     force (B,24) | None, iters (B,) | None[, grad_pts (B,8,3)])."""
-    dtype = _check_inputs(x, x_plus, inertia, mu_pair, kin, *([half] if half is not None else []),
-                          *([pts] if pts is not None else []))
+    dtype = _check_inputs(x, x_plus, inertia, mu_pair, kin, half, pts)
     x, x_plus = x.contiguous(), x_plus.contiguous()
     inertia, mu_pair, kin = inertia.contiguous(), mu_pair.contiguous(), kin.contiguous()
     half = half.contiguous() if half is not None else None
     pts = pts.contiguous() if pts is not None else None
-    if x.dim() != 2 or x.shape[1] != 15 or x_plus.shape != x.shape:
-        raise ValueError(f'expected (B,15) states, got {tuple(x.shape)} / {tuple(x_plus.shape)}')
+    _check_states(15, x, x_plus)
     if inertia.numel() != 20 or mu_pair.numel() != 2 or kin.numel() != 12 or (half is not None and half.numel() != 6):
         raise ValueError('elbow parameters must be inertia (20), mu_pair (2), half (6), kin (12)')
     if half is None and pts is None:
@@ -379,14 +394,9 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
     iters = torch.empty(B, dtype=torch.int32, device=dev) if want_iters else None
     if weight is not None:
         weight = weight.to(dtype).contiguous()
-    ws = _workspace(dev)
     grad_pts = torch.zeros((B, 8, 3), dtype=dtype, device=dev) if (want_grad_pts and want_grad) else None
-    fn = getattr(_lib.load(), 'dpll_elbow_loss_' + _SUFFIX[dtype])
-    with torch.cuda.device(dev):
-        rc = fn(_ptr(x), _ptr(x_plus), _ptr(weight), _ptr(inertia), _ptr(mu_pair), _ptr(half), _ptr(kin), _ptr(pts),
-                dt, eps, B, flags, _ptr(loss), _ptr(force), _ptr(grad_pts), _ptr(iters), _ptr(grad), _ptr(loss_sum),
-                _ptr(skip_flag), _ptr(ws), ws.numel(), _stream())
-    _lib.check(rc, 'dpll_elbow_loss')
+    _call('dpll_elbow_loss', dev, x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, flags, loss, force,
+          grad_pts, iters, grad, loss_sum, skip_flag, dtype=dtype, workspace=True)
     if want_grad_pts:
         return loss, grad, loss_sum, force, iters, grad_pts
     return loss, grad, loss_sum, force, iters
@@ -404,7 +414,6 @@ class ElbowContactNetsLoss(torch.autograd.Function):
         loss, grad, loss_sum, _, iters = elbow_loss_raw(x, x_plus, inertia, mu_pair, half, kin, dt, eps, want_grad=need,
                                                         want_iters=want_iters, flags=flags)
         ctx.dt, ctx.eps = dt, eps
-        ctx.shapes = (inertia.shape, mu_pair.shape, half.shape)
         if need:
             ctx.save_for_backward(grad, x, x_plus, inertia, mu_pair, half, kin)
         else:
@@ -419,21 +428,9 @@ class ElbowContactNetsLoss(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_loss, _g_sums, _g_means, _g_iters):
         grad, x, x_plus, inertia, mu_pair, half, kin = ctx.saved_tensors
-        if grad_loss.numel() == 0:
-            g = torch.zeros_like(grad)
-        elif grad_loss.dim() == 1 and grad_loss.stride(0) == 0:
-            g = grad * grad_loss[0]
-        else:
-            grad_loss = grad_loss.contiguous()
-            lo, hi = torch.aminmax(grad_loss)
-            uniform = lo == hi
-            gw = torch.zeros_like(grad)
-            elbow_loss_raw(x, x_plus, inertia, mu_pair, half, kin, ctx.dt, ctx.eps, weight=grad_loss, want_grad=True,
-                           want_loss=False, skip_flag=uniform.to(torch.int32), grad_out=gw)
-            g = torch.where(uniform, grad * lo, gw)
-        s_in, s_mu, s_h = ctx.shapes
-        return (None, None, g[0:20].reshape(s_in), g[20:22].reshape(s_mu), g[22:28].reshape(s_h), None, None, None,
-                None, None)
+        g = _fused_grad(grad, grad_loss, lambda w, skip, out: elbow_loss_raw(
+            x, x_plus, inertia, mu_pair, half, kin, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip, grad_out=out))
+        return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None, None)
 
 
 class ElbowContactNetsLossPts(torch.autograd.Function):
@@ -449,7 +446,6 @@ class ElbowContactNetsLossPts(torch.autograd.Function):
                              want_grad_pts=True)
         loss, grad, gpts = out[0], out[1], out[5]
         ctx.dt, ctx.eps = dt, eps
-        ctx.shapes = (inertia.shape, mu_pair.shape)
         if need:
             ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts, kin)
         return loss
@@ -457,21 +453,10 @@ class ElbowContactNetsLossPts(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_loss):
         grad, gpts, x, x_plus, inertia, mu_pair, pts, kin = ctx.saved_tensors
-        if grad_loss.numel() == 0:
-            g = torch.zeros_like(grad)
-        elif grad_loss.dim() == 1 and grad_loss.stride(0) == 0:
-            g = grad * grad_loss[0]
-        else:
-            grad_loss = grad_loss.contiguous()
-            lo, hi = torch.aminmax(grad_loss)
-            uniform = lo == hi
-            gw = torch.zeros_like(grad)
-            elbow_loss_raw(x, x_plus, inertia, mu_pair, None, kin, ctx.dt, ctx.eps, weight=grad_loss, want_grad=True,
-                           want_loss=False, skip_flag=uniform.to(torch.int32), grad_out=gw, pts=pts)
-            g = torch.where(uniform, grad * lo, gw)
-        s_in, s_mu = ctx.shapes
-        return (None, None, g[0:20].reshape(s_in), g[20:22].reshape(s_mu), gpts * grad_loss.reshape(-1, 1, 1),
-                None, None, None)
+        g = _fused_grad(grad, grad_loss, lambda w, skip, out: elbow_loss_raw(
+            x, x_plus, inertia, mu_pair, None, kin, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip,
+            grad_out=out, pts=pts))
+        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1), None, None, None)
 
 
 def elbow_rollout_saved(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Optional[Tensor], kin: Tensor, dt: float,
@@ -479,17 +464,11 @@ def elbow_rollout_saved(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Opti
     """``dpll_elbow_rollout_saved_f64``: trajectory (B, steps+1, 15) and every step's QP optimum usol (B, steps, 7), which
     the backward (forward-mode tangents) turns into one evaluation per step instead of a dual-number solve.  float64."""
     _check_inputs(x0, inertia, mu_pair, kin)
-    f64 = torch.float64
-    a = [t.detach().to(f64).contiguous() for t in (x0, inertia, mu_pair, kin)]
-    h = half.detach().to(f64).contiguous() if half is not None else None
-    pt = pts.detach().to(f64).contiguous() if pts is not None else None
     B = x0.shape[0]
-    traj = torch.empty((B, steps + 1, 15), dtype=f64, device=x0.device)
-    usol = torch.empty((B, steps, 7), dtype=f64, device=x0.device)
-    with torch.cuda.device(x0.device):
-        rc = _lib.load().dpll_elbow_rollout_saved_f64(_ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(h), _ptr(a[3]), _ptr(pt), dt, eps,
-                                                      B, steps, _ptr(traj), _ptr(usol), _stream())
-    _lib.check(rc, 'dpll_elbow_rollout_saved')
+    traj = torch.empty((B, steps + 1, 15), dtype=torch.float64, device=x0.device)
+    usol = torch.empty((B, steps, 7), dtype=torch.float64, device=x0.device)
+    _call('dpll_elbow_rollout_saved_f64', x0.device, _f64(x0), _f64(inertia), _f64(mu_pair), _f64(half), _f64(kin), _f64(pts),
+          dt, eps, B, steps, traj, usol)
     return traj, usol
 
 
@@ -500,18 +479,13 @@ def elbow_rollout(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Optional[T
     points ``pts`` (B,8,3) of a learned geometry only a single step is allowed."""
     dtype = _check_inputs(x0, inertia, mu_pair, kin)
     x0 = x0.contiguous()
-    if x0.dim() != 2 or x0.shape[1] != 15:
-        raise ValueError(f'expected (B,15) states, got {tuple(x0.shape)}')
+    _check_states(15, x0)
     B = x0.shape[0]
     traj = torch.empty((B, steps + 1, 15), dtype=dtype, device=x0.device)
     force = torch.empty((B, steps, 24), dtype=dtype, device=x0.device) if want_force else None
-    fn = getattr(_lib.load(), 'dpll_elbow_rollout_' + _SUFFIX[dtype])
-    with torch.cuda.device(x0.device):
-        rc = fn(_ptr(x0), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()),
-                _ptr(half.contiguous() if half is not None else None), _ptr(kin.contiguous()),
-                _ptr(pts.contiguous() if pts is not None else None), dt, eps, B, steps, _ptr(traj), _ptr(force), None,
-                _stream())
-    _lib.check(rc, 'dpll_elbow_rollout')
+    _call('dpll_elbow_rollout', x0.device, x0, inertia.contiguous(), mu_pair.contiguous(),
+          half.contiguous() if half is not None else None, kin.contiguous(), pts.contiguous() if pts is not None else None,
+          dt, eps, B, steps, traj, force, None, dtype=dtype)
     return traj, force
 
 
@@ -527,15 +501,11 @@ class CubeRollout(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x0, inertia, mu_pair, half, dt, steps, eps, forward_mode=False):
-        f64 = torch.float64
         B = x0.shape[0]
-        a = [t.detach().to(f64).contiguous() for t in (x0, inertia, mu_pair, half)]
-        traj = torch.empty((B, steps + 1, 13), dtype=f64, device=x0.device)
-        usol = torch.empty((B, steps, 6), dtype=f64, device=x0.device)
-        with torch.cuda.device(x0.device):
-            rc = _lib.load().dpll_cube_rollout_saved_f64(_ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(a[3]), dt, eps, B, steps,
-                                                         _ptr(traj), _ptr(usol), _stream())
-        _lib.check(rc, 'dpll_cube_rollout_saved')
+        a = [_f64(t) for t in (x0, inertia, mu_pair, half)]
+        traj = torch.empty((B, steps + 1, 13), dtype=torch.float64, device=x0.device)
+        usol = torch.empty((B, steps, 6), dtype=torch.float64, device=x0.device)
+        _call('dpll_cube_rollout_saved_f64', x0.device, *a, dt, eps, B, steps, traj, usol)
         ctx.dt, ctx.steps, ctx.eps, ctx.forward_mode = dt, steps, eps, forward_mode
         ctx.save_for_backward(x0, inertia, mu_pair, half, traj, usol)
         return traj.to(x0.dtype)
@@ -543,28 +513,15 @@ class CubeRollout(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gtraj):
         x0, inertia, mu_pair, half, traj, usol = ctx.saved_tensors
-        B, steps = x0.shape[0], ctx.steps
-        f64 = torch.float64
-        xbar = gtraj[:, 1:, :].to(f64).contiguous()
-        gparams = torch.zeros((B, 14), dtype=f64, device=x0.device)
-        gx0 = torch.zeros((B, 13), dtype=f64, device=x0.device)
-        if B > 0 and steps > 0:
-            args = [t.detach().to(f64).contiguous() for t in (x0, inertia, mu_pair, half)]
-            lib = _lib.load()
-            with torch.cuda.device(x0.device):
-                if ctx.forward_mode:
-                    rc = lib.dpll_cube_rollout_grad_f64(_ptr(args[0]), _ptr(args[1]), _ptr(args[2]), _ptr(args[3]),
-                                                        ctx.dt, ctx.eps, B, steps, _ptr(xbar), _ptr(gparams), _ptr(gx0),
-                                                        _stream())
-                else:
-                    rc = lib.dpll_cube_rollout_backward_f64(_ptr(traj), _ptr(usol), _ptr(args[1]), _ptr(args[2]),
-                                                            _ptr(args[3]), ctx.dt, ctx.eps, B, steps, _ptr(xbar),
-                                                            _ptr(gparams), _ptr(gx0), _stream())
-            _lib.check(rc, 'dpll_cube_rollout_backward')
-        g = gparams.sum(0)
-        gx = (gx0 + gtraj[:, 0, :].to(f64)).to(x0.dtype)
-        return (gx, g[0:10].reshape(inertia.shape).to(inertia.dtype), g[10:11].reshape(mu_pair.shape).to(mu_pair.dtype),
-                g[11:14].reshape(half.shape).to(half.dtype), None, None, None, None)
+        B, steps, params = x0.shape[0], ctx.steps, (inertia, mu_pair, half)
+        if ctx.forward_mode:
+            name, start = 'dpll_cube_rollout_grad_f64', (x0,)
+        else:
+            name, start = 'dpll_cube_rollout_backward_f64', (traj, usol)
+        gi, gm, gh, gx0 = _summed_backward(name, x0, params, (14, 13), *start, *params, ctx.dt, ctx.eps, B, steps,
+                                           gtraj[:, 1:, :], steps=steps)
+        gx = (gx0 + gtraj[:, 0, :].to(torch.float64)).to(x0.dtype)
+        return gx, gi, gm, gh, None, None, None, None
 
 
 class ElbowRollout(torch.autograd.Function):
@@ -583,21 +540,11 @@ class ElbowRollout(torch.autograd.Function):
     def backward(ctx, gtraj):
         x0, inertia, mu_pair, half, kin, usol = ctx.saved_tensors
         B, steps = x0.shape[0], ctx.steps
-        f64 = torch.float64
-        xbar = gtraj[:, 1:, :].to(f64).contiguous()
-        gparams = torch.zeros((B, 28), dtype=f64, device=x0.device)
-        gx0 = torch.zeros((B, 15), dtype=f64, device=x0.device)
-        if B > 0 and steps > 0:
-            a = [t.detach().to(f64).contiguous() for t in (x0, inertia, mu_pair, half, kin)]
-            with torch.cuda.device(x0.device):
-                rc = _lib.load().dpll_elbow_rollout_grad_saved_f64(_ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(a[3]), _ptr(a[4]),
-                                                                   _ptr(usol), ctx.dt, ctx.eps, B, steps, _ptr(xbar),
-                                                                   _ptr(gparams), _ptr(gx0), _stream())
-            _lib.check(rc, 'dpll_elbow_rollout_grad_saved')
-        g = gparams.sum(0)
-        gx = (gx0 + gtraj[:, 0, :].to(f64)).to(x0.dtype)
-        return (gx, g[0:20].reshape(inertia.shape).to(inertia.dtype), g[20:22].reshape(mu_pair.shape).to(mu_pair.dtype),
-                g[22:28].reshape(half.shape).to(half.dtype), None, None, None, None)
+        gi, gm, gh, gx0 = _summed_backward('dpll_elbow_rollout_grad_saved_f64', x0, (inertia, mu_pair, half), (28, 15), x0,
+                                           inertia, mu_pair, half, kin, usol, ctx.dt, ctx.eps, B, steps, gtraj[:, 1:, :],
+                                           steps=steps)
+        gx = (gx0 + gtraj[:, 0, :].to(torch.float64)).to(x0.dtype)
+        return gx, gi, gm, gh, None, None, None, None
 
 
 class ElbowStepPts(torch.autograd.Function):
@@ -616,22 +563,9 @@ class ElbowStepPts(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gnext):
         x, inertia, mu_pair, pts, kin, usol = ctx.saved_tensors
-        B = x.shape[0]
-        f64 = torch.float64
-        gparams = torch.zeros((B, 22), dtype=f64, device=x.device)
-        gpts = torch.zeros((B, 24), dtype=f64, device=x.device)
-        gx = torch.zeros((B, 15), dtype=f64, device=x.device)
-        if B > 0:
-            a = [t.detach().to(f64).contiguous() for t in (x, inertia, mu_pair, kin, pts)]
-            xbar = gnext.to(f64).contiguous()
-            with torch.cuda.device(x.device):
-                rc = _lib.load().dpll_elbow_step_pts_grad_f64(_ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(a[3]), _ptr(a[4]),
-                                                              _ptr(usol), ctx.dt, ctx.eps, B, _ptr(xbar), _ptr(gparams),
-                                                              _ptr(gpts), _ptr(gx), _stream())
-            _lib.check(rc, 'dpll_elbow_step_pts_grad')
-        g = gparams.sum(0)
-        return (gx.to(x.dtype), g[0:20].reshape(inertia.shape).to(inertia.dtype),
-                g[20:22].reshape(mu_pair.shape).to(mu_pair.dtype), gpts.reshape(pts.shape).to(pts.dtype), None, None, None)
+        gi, gm, gpts, gx = _summed_backward('dpll_elbow_step_pts_grad_f64', x, (inertia, mu_pair), (22, 24, 15), x, inertia,
+                                            mu_pair, kin, pts, usol, ctx.dt, ctx.eps, x.shape[0], gnext)
+        return gx.to(x.dtype), gi, gm, gpts.reshape(pts.shape).to(pts.dtype), None, None, None
 
 
 def body_loss_pts_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_contacts: int, dt: float,
@@ -641,13 +575,10 @@ def body_loss_pts_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tenso
     """Direct call of ``dpll_body_loss_pts_f64`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,13), inertia
     (10), mu_pair (1), witness points pts (B,4,3) of which the first ``n_contacts`` rows are used.  Returns (loss (B,) | None,
     grad (11,) | None, loss_sum (1,), grad_pts (B,4,3) | None, iters (B,) | None, force (B,12) | None)."""
-    _check_inputs(x, x_plus, inertia, mu_pair, pts)
-    if x.dtype != torch.float64:
-        raise TypeError('the witness-point kernels are provided in float64')
+    _check_inputs(x, x_plus, inertia, mu_pair, pts, f64_only='the witness-point kernels are provided in float64')
     x, x_plus, pts = x.contiguous(), x_plus.contiguous(), pts.contiguous()
     B, dev = x.shape[0], x.device
-    if x.dim() != 2 or x.shape[1] != 13 or x_plus.shape != x.shape:
-        raise ValueError(f'expected (B,13) states, got {tuple(x.shape)} / {tuple(x_plus.shape)}')
+    _check_states(13, x, x_plus)
     if tuple(pts.shape) != (B, 4, 3):
         raise ValueError(f'pts must be (B,4,3), got {tuple(pts.shape)}')
     loss = torch.empty(B, dtype=x.dtype, device=dev) if want_loss else None
@@ -658,13 +589,8 @@ def body_loss_pts_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tenso
     force = torch.empty((B, 12), dtype=x.dtype, device=dev) if want_force else None
     if weight is not None:
         weight = weight.to(x.dtype).contiguous()
-    ws = _workspace(dev)
-    with torch.cuda.device(dev):
-        rc = _lib.load().dpll_body_loss_pts_f64(_ptr(x), _ptr(x_plus), _ptr(weight), _ptr(inertia.contiguous()),
-                                                _ptr(mu_pair.contiguous()), _ptr(pts), n_contacts, dt, eps, B, flags,
-                                                _ptr(loss), _ptr(force), _ptr(gpts), _ptr(iters), _ptr(grad), _ptr(loss_sum),
-                                                _ptr(skip_flag), _ptr(ws), ws.numel(), _stream())
-    _lib.check(rc, 'dpll_body_loss_pts')
+    _call('dpll_body_loss_pts_f64', dev, x, x_plus, weight, inertia.contiguous(), mu_pair.contiguous(), pts, n_contacts, dt,
+          eps, B, flags, loss, force, gpts, iters, grad, loss_sum, skip_flag, workspace=True)
     return loss, grad, loss_sum, gpts, iters, force
 
 
@@ -681,7 +607,6 @@ class BodyWitnessPointLoss(torch.autograd.Function):
         loss, grad, _, gpts, iters, _ = body_loss_pts_raw(x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, flags=flags,
                                                           want_iters=want_iters)
         ctx.args = (n_contacts, dt, eps, flags)
-        ctx.shapes = (inertia.shape, mu_pair.shape)
         ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts)
         if iters is None:
             iters = torch.empty(0, dtype=torch.int32, device=loss.device)
@@ -692,19 +617,10 @@ class BodyWitnessPointLoss(torch.autograd.Function):
     def backward(ctx, grad_loss, _g_iters):
         grad, gpts, x, x_plus, inertia, mu_pair, pts = ctx.saved_tensors
         n_contacts, dt, eps, flags = ctx.args
-        if grad_loss.dim() == 1 and grad_loss.numel() > 0 and grad_loss.stride(0) == 0:
-            g = grad * grad_loss[0]
-        else:
-            grad_loss = grad_loss.contiguous()
-            lo, hi = torch.aminmax(grad_loss) if grad_loss.numel() > 0 else (grad_loss.new_zeros(()), grad_loss.new_zeros(()))
-            uniform = lo == hi
-            gw = torch.zeros_like(grad)
-            body_loss_pts_raw(x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, weight=grad_loss, want_loss=False,
-                              want_grad_pts=False, flags=flags, skip_flag=uniform.to(torch.int32), grad_out=gw)
-            g = torch.where(uniform, grad * lo, gw)
-        s_in, s_mu = ctx.shapes
-        return (None, None, g[0:10].reshape(s_in), g[10:11].reshape(s_mu), gpts * grad_loss.reshape(-1, 1, 1), None, None,
-                None, None, None)
+        g = _fused_grad(grad, grad_loss, lambda w, skip, out: body_loss_pts_raw(
+            x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, weight=w, want_loss=False, want_grad_pts=False,
+            flags=flags, skip_flag=skip, grad_out=out))
+        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1), None, None, None, None, None)
 
 
 def body_step_pts(x: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_contacts: int, dt: float,
@@ -713,10 +629,8 @@ def body_step_pts(x: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_co
     _check_inputs(x, inertia, mu_pair, pts)
     x, pts = x.contiguous(), pts.contiguous()
     out = torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        rc = _lib.load().dpll_body_step_pts_f64(_ptr(x), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()), _ptr(pts),
-                                                n_contacts, dt, eps, x.shape[0], _ptr(out), None, _stream())
-    _lib.check(rc, 'dpll_body_step_pts')
+    _call('dpll_body_step_pts_f64', x.device, x, inertia.contiguous(), mu_pair.contiguous(), pts, n_contacts, dt, eps,
+          x.shape[0], out, None)
     return out
 
 
@@ -734,22 +648,9 @@ class BodyStepPts(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gnext):
         x, inertia, mu_pair, pts = ctx.saved_tensors
-        B = x.shape[0]
-        f64 = torch.float64
-        gparams = torch.zeros((B, 11), dtype=f64, device=x.device)
-        gpts = torch.zeros((B, 12), dtype=f64, device=x.device)
-        gx = torch.zeros((B, 13), dtype=f64, device=x.device)
-        if B > 0:
-            a = [t.detach().to(f64).contiguous() for t in (x, inertia, mu_pair, pts)]
-            xbar = gnext.to(f64).contiguous()
-            with torch.cuda.device(x.device):
-                rc = _lib.load().dpll_body_step_pts_grad_f64(_ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(a[3]), ctx.n_c, ctx.dt,
-                                                             ctx.eps, B, _ptr(xbar), _ptr(gparams), _ptr(gpts), _ptr(gx),
-                                                             _stream())
-            _lib.check(rc, 'dpll_body_step_pts_grad')
-        g = gparams.sum(0)
-        return (gx.to(x.dtype), g[0:10].reshape(inertia.shape).to(inertia.dtype), g[10:11].reshape(mu_pair.shape).to(mu_pair.dtype),
-                gpts.reshape(pts.shape).to(pts.dtype), None, None, None)
+        gi, gm, gpts, gx = _summed_backward('dpll_body_step_pts_grad_f64', x, (inertia, mu_pair), (11, 12, 13), x, inertia,
+                                            mu_pair, pts, ctx.n_c, ctx.dt, ctx.eps, x.shape[0], gnext)
+        return gx.to(x.dtype), gi, gm, gpts.reshape(pts.shape).to(pts.dtype), None, None, None
 
 
 class ChainContactNetsLoss(torch.autograd.Function):
@@ -758,25 +659,15 @@ class ChainContactNetsLoss(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, x_plus, inertia, mu_pair, half, kin, n, dt, eps):
-        _check_inputs(x, x_plus, inertia, mu_pair, half, kin)
-        if x.dtype != torch.float64:
-            raise TypeError('the generic chain kernels are provided in float64')
-        n_x = 13 + 2 * (n - 1)
+        _check_inputs(x, x_plus, inertia, mu_pair, half, kin, f64_only='the generic chain kernels are provided in float64')
         x, x_plus = x.contiguous(), x_plus.contiguous()
-        if x.dim() != 2 or x.shape[1] != n_x or x_plus.shape != x.shape:
-            raise ValueError(f'expected (B,{n_x}) states, got {tuple(x.shape)} / {tuple(x_plus.shape)}')
+        _check_states(13 + 2 * (n - 1), x, x_plus)
         B, dev = x.shape[0], x.device
         loss = torch.empty(B, dtype=x.dtype, device=dev)
         ctx.args = (n, dt, eps)
-        ctx.shapes = (inertia.shape, mu_pair.shape, half.shape)
         ctx.save_for_backward(x, x_plus, inertia, mu_pair, half, kin)
-        ws = _workspace(dev)
-        with torch.cuda.device(dev):
-            rc = _lib.load().dpll_chain_loss_f64(n, _ptr(x), _ptr(x_plus), None, _ptr(inertia.contiguous()),
-                                                 _ptr(mu_pair.contiguous()), _ptr(half.contiguous()), _ptr(kin.contiguous()),
-                                                 dt, eps, B, _ptr(loss), None, None, None, None, _ptr(ws), ws.numel(),
-                                                 _stream())
-        _lib.check(rc, 'dpll_chain_loss')
+        _call('dpll_chain_loss_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(),
+              kin.contiguous(), dt, eps, B, loss, None, None, None, None, workspace=True)
         return loss
 
     @staticmethod
@@ -786,17 +677,9 @@ class ChainContactNetsLoss(torch.autograd.Function):
         B, dev = x.shape[0], x.device
         g = torch.zeros(14 * n, dtype=x.dtype, device=dev)
         if B > 0:
-            w = grad_loss.contiguous()
-            ws = _workspace(dev)
-            with torch.cuda.device(dev):
-                rc = _lib.load().dpll_chain_loss_f64(n, _ptr(x), _ptr(x_plus), _ptr(w), _ptr(inertia.contiguous()),
-                                                     _ptr(mu_pair.contiguous()), _ptr(half.contiguous()),
-                                                     _ptr(kin.contiguous()), dt, eps, B, None, None, None, _ptr(g), None,
-                                                     _ptr(ws), ws.numel(), _stream())
-            _lib.check(rc, 'dpll_chain_loss')
-        s_in, s_mu, s_h = ctx.shapes
-        return (None, None, g[:10 * n].reshape(s_in), g[10 * n:11 * n].reshape(s_mu), g[11 * n:].reshape(s_h), None, None,
-                None, None)
+            _call('dpll_chain_loss_f64', dev, n, x, x_plus, grad_loss.contiguous(), inertia.contiguous(), mu_pair.contiguous(),
+                  half.contiguous(), kin.contiguous(), dt, eps, B, None, None, None, g, None, workspace=True)
+        return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None)
 
 
 def chain_rollout(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, kin: Tensor, n: int, dt: float,
@@ -806,11 +689,8 @@ def chain_rollout(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, ki
     x0 = x0.contiguous()
     B = x0.shape[0]
     traj = torch.empty((B, steps + 1, x0.shape[1]), dtype=x0.dtype, device=x0.device)
-    with torch.cuda.device(x0.device):
-        rc = _lib.load().dpll_chain_rollout_f64(n, _ptr(x0), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()),
-                                                _ptr(half.contiguous()), _ptr(kin.contiguous()), dt, eps, B, steps,
-                                                _ptr(traj), _stream())
-    _lib.check(rc, 'dpll_chain_rollout')
+    _call('dpll_chain_rollout_f64', x0.device, n, x0, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(),
+          kin.contiguous(), dt, eps, B, steps, traj)
     return traj
 
 
@@ -827,30 +707,18 @@ class ChainRollout(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gtraj):
         x0, inertia, mu_pair, half, kin = ctx.saved_tensors
-        B, n, steps, nx = x0.shape[0], ctx.n, ctx.steps, x0.shape[1]
-        f64 = torch.float64
-        xbar = gtraj[:, 1:, :].to(f64).contiguous()
-        gparams = torch.zeros((B, 14 * n), dtype=f64, device=x0.device)
-        gx0 = torch.zeros((B, nx), dtype=f64, device=x0.device)
-        if B > 0 and steps > 0:
-            a = [t.detach().to(f64).contiguous() for t in (x0, inertia, mu_pair, half, kin)]
-            with torch.cuda.device(x0.device):
-                rc = _lib.load().dpll_chain_rollout_grad_f64(n, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(a[3]), _ptr(a[4]),
-                                                             ctx.dt, ctx.eps, B, steps, _ptr(xbar), _ptr(gparams), _ptr(gx0),
-                                                             _stream())
-            _lib.check(rc, 'dpll_chain_rollout_grad')
-        g = gparams.sum(0)
-        gx = (gx0 + gtraj[:, 0, :].to(f64)).to(x0.dtype)
-        return (gx, g[0:10 * n].reshape(inertia.shape).to(inertia.dtype), g[10 * n:11 * n].reshape(mu_pair.shape).to(mu_pair.dtype),
-                g[11 * n:14 * n].reshape(half.shape).to(half.dtype), None, None, None, None, None)
+        B, n, steps = x0.shape[0], ctx.n, ctx.steps
+        gi, gm, gh, gx0 = _summed_backward('dpll_chain_rollout_grad_f64', x0, (inertia, mu_pair, half), (14 * n, x0.shape[1]),
+                                           n, x0, inertia, mu_pair, half, kin, ctx.dt, ctx.eps, B, steps, gtraj[:, 1:, :],
+                                           steps=steps)
+        gx = (gx0 + gtraj[:, 0, :].to(torch.float64)).to(x0.dtype)
+        return gx, gi, gm, gh, None, None, None, None, None
 
 
 def cube_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor):
     """``dpll_cube_terms_f64``: (delassus (B,12,12), M (B,6,6), J (B,12,6), phi (B,4), acc (B,6)) in the order
     ``MultibodyTerms.forward`` returns them (multibody_terms.py:584-609).  fp64 only, no autograd."""
-    _check_inputs(q, v, inertia, mu_pair, half)
-    if q.dtype != torch.float64:
-        raise TypeError('cube_terms is provided in float64')
+    _check_inputs(q, v, inertia, mu_pair, half, f64_only='cube_terms is provided in float64')
     q, v = q.contiguous(), v.contiguous()
     B, dev = q.shape[0], q.device
     M = torch.empty((B, 6, 6), dtype=q.dtype, device=dev)
@@ -858,20 +726,14 @@ def cube_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Ten
     phi = torch.empty((B, 4), dtype=q.dtype, device=dev)
     acc = torch.empty((B, 6), dtype=q.dtype, device=dev)
     D = torch.empty((B, 12, 12), dtype=q.dtype, device=dev)
-    with torch.cuda.device(dev):
-        rc = _lib.load().dpll_cube_terms_f64(_ptr(q), _ptr(v), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()),
-                                             _ptr(half.contiguous()), B, _ptr(M), _ptr(J), _ptr(phi), _ptr(acc),
-                                             _ptr(D), _stream())
-    _lib.check(rc, 'dpll_cube_terms')
+    _call('dpll_cube_terms_f64', dev, q, v, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(), B, M, J, phi, acc, D)
     return D, M, J, phi, acc
 
 
 def elbow_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, kin: Tensor):
     """``dpll_elbow_terms_f64``: (delassus (B,24,24), M (B,7,7), J (B,24,7), phi (B,8), acc (B,7)) in the order
     ``MultibodyTerms.forward`` returns them (multibody_terms.py:584-609).  fp64 only, no autograd."""
-    _check_inputs(q, v, inertia, mu_pair, half, kin)
-    if q.dtype != torch.float64:
-        raise TypeError('elbow_terms is provided in float64')
+    _check_inputs(q, v, inertia, mu_pair, half, kin, f64_only='elbow_terms is provided in float64')
     q, v = q.contiguous(), v.contiguous()
     B, dev = q.shape[0], q.device
     M = torch.empty((B, 7, 7), dtype=q.dtype, device=dev)
@@ -879,11 +741,8 @@ def elbow_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Te
     phi = torch.empty((B, 8), dtype=q.dtype, device=dev)
     acc = torch.empty((B, 7), dtype=q.dtype, device=dev)
     D = torch.empty((B, 24, 24), dtype=q.dtype, device=dev)
-    with torch.cuda.device(dev):
-        rc = _lib.load().dpll_elbow_terms_f64(_ptr(q), _ptr(v), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()),
-                                              _ptr(half.contiguous()), _ptr(kin.contiguous()), B, _ptr(M), _ptr(J),
-                                              _ptr(phi), _ptr(acc), _ptr(D), _stream())
-    _lib.check(rc, 'dpll_elbow_terms')
+    _call('dpll_elbow_terms_f64', dev, q, v, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(), kin.contiguous(),
+          B, M, J, phi, acc, D)
     return D, M, J, phi, acc
 
 
@@ -895,9 +754,7 @@ class ChainWitnessPointLoss(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, x_plus, inertia, mu_pair, pts, kin, n, n_pts_packed, dt, eps):
-        _check_inputs(x, x_plus, inertia, mu_pair, pts, kin)
-        if x.dtype != torch.float64:
-            raise TypeError('the generic tree kernels are provided in float64')
+        _check_inputs(x, x_plus, inertia, mu_pair, pts, kin, f64_only='the generic tree kernels are provided in float64')
         n_x = 13 + 2 * (n - 1)
         x, x_plus, pts = x.contiguous(), x_plus.contiguous(), pts.contiguous()
         B, dev = x.shape[0], x.device
@@ -905,15 +762,9 @@ class ChainWitnessPointLoss(torch.autograd.Function):
             raise ValueError(f'expected (B,{n_x}) states and (B,{n},4,3) points, got {tuple(x.shape)} / {tuple(pts.shape)}')
         loss = torch.empty(B, dtype=x.dtype, device=dev)
         gpts = torch.empty_like(pts)
-        ws = _workspace(dev)
-        with torch.cuda.device(dev):
-            rc = _lib.load().dpll_chain_loss_pts_f64(n, _ptr(x), _ptr(x_plus), None, _ptr(inertia.contiguous()),
-                                                     _ptr(mu_pair.contiguous()), _ptr(kin.contiguous()), _ptr(pts), n_pts_packed,
-                                                     dt, eps, B, _ptr(loss), _ptr(gpts), None, None, _ptr(ws), ws.numel(),
-                                                     _stream())
-        _lib.check(rc, 'dpll_chain_loss_pts')
+        _call('dpll_chain_loss_pts_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(), kin.contiguous(),
+              pts, n_pts_packed, dt, eps, B, loss, gpts, None, None, workspace=True)
         ctx.args = (n, n_pts_packed, dt, eps)
-        ctx.shapes = (inertia.shape, mu_pair.shape)
         ctx.save_for_backward(gpts, x, x_plus, inertia, mu_pair, pts, kin)
         return loss
 
@@ -924,25 +775,17 @@ class ChainWitnessPointLoss(torch.autograd.Function):
         B, dev = x.shape[0], x.device
         g = torch.zeros(14 * n, dtype=x.dtype, device=dev)
         if B > 0:
-            w = grad_loss.contiguous()
-            ws = _workspace(dev)
-            with torch.cuda.device(dev):
-                rc = _lib.load().dpll_chain_loss_pts_f64(n, _ptr(x), _ptr(x_plus), _ptr(w), _ptr(inertia.contiguous()),
-                                                         _ptr(mu_pair.contiguous()), _ptr(kin.contiguous()), _ptr(pts), packed,
-                                                         dt, eps, B, None, None, _ptr(g), None, _ptr(ws), ws.numel(), _stream())
-            _lib.check(rc, 'dpll_chain_loss_pts')
-        s_in, s_mu = ctx.shapes
-        return (None, None, g[:10 * n].reshape(s_in), g[10 * n:11 * n].reshape(s_mu), gpts * grad_loss.reshape(-1, 1, 1, 1), None,
-                None, None, None, None)
+            _call('dpll_chain_loss_pts_f64', dev, n, x, x_plus, grad_loss.contiguous(), inertia.contiguous(),
+                  mu_pair.contiguous(), kin.contiguous(), pts, packed, dt, eps, B, None, None, g, None, workspace=True)
+        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1, 1), None, None, None, None,
+                None)
 
 
 def chain_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, kin: Tensor, n: int, n_boxes: int):
     """``dpll_chain_terms_f64``: (delassus (B,12g,12g), M (B,nv,nv), J (B,12g,nv), phi (B,4g), acc (B,nv)) of a tree of ``n``
     links with ``g = n_boxes`` boxes, in the order ``MultibodyTerms.forward`` returns them (multibody_terms.py:584-609).
     fp64 only, no autograd."""
-    _check_inputs(q, v, inertia, mu_pair, half, kin)
-    if q.dtype != torch.float64:
-        raise TypeError('chain_terms is provided in float64')
+    _check_inputs(q, v, inertia, mu_pair, half, kin, f64_only='chain_terms is provided in float64')
     q, v = q.contiguous(), v.contiguous()
     B, dev, nv, k = q.shape[0], q.device, 6 + n - 1, 12 * n_boxes
     M = torch.empty((B, nv, nv), dtype=q.dtype, device=dev)
@@ -950,11 +793,8 @@ def chain_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Te
     phi = torch.empty((B, 4 * n_boxes), dtype=q.dtype, device=dev)
     acc = torch.empty((B, nv), dtype=q.dtype, device=dev)
     D = torch.empty((B, k, k), dtype=q.dtype, device=dev)
-    with torch.cuda.device(dev):
-        rc = _lib.load().dpll_chain_terms_f64(n, n_boxes, _ptr(q), _ptr(v), _ptr(inertia.contiguous()), _ptr(mu_pair.contiguous()),
-                                              _ptr(half.contiguous()), _ptr(kin.contiguous()), B, _ptr(M), _ptr(J),
-                                              _ptr(phi), _ptr(acc), _ptr(D), _stream())
-    _lib.check(rc, 'dpll_chain_terms')
+    _call('dpll_chain_terms_f64', dev, n, n_boxes, q, v, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(),
+          kin.contiguous(), B, M, J, phi, acc, D)
     return D, M, J, phi, acc
 
 
@@ -967,20 +807,15 @@ class LeafPrepare(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, theta, friction, pairs, length):
-        _check_inputs(theta, friction, length)
-        if theta.dtype != torch.float64:
-            raise TypeError('dpll_leaf_prepare is provided in float64')
+        _check_inputs(theta, friction, length, f64_only='dpll_leaf_prepare is provided in float64')
         theta, friction, length = theta.contiguous(), friction.contiguous(), length.contiguous()
         assert pairs.dtype == torch.int32 and pairs.is_cuda and pairs.is_contiguous() and pairs.shape[0] == 2
         nb, npair, nlen = theta.shape[0], pairs.shape[1], length.numel()
         inertia = torch.empty_like(theta)
         mu = torch.empty(npair, dtype=theta.dtype, device=theta.device)
         half = torch.empty(nlen, dtype=theta.dtype, device=theta.device)
-        with torch.cuda.device(theta.device):
-            rc = _lib.load().dpll_leaf_prepare_f64(_ptr(theta), nb, _ptr(friction), pairs.data_ptr(),
-                                                   pairs.data_ptr() + 4 * npair, npair, _ptr(length), nlen, _ptr(inertia),
-                                                   _ptr(mu), _ptr(half), _stream())
-        _lib.check(rc, 'dpll_leaf_prepare')
+        _call('dpll_leaf_prepare_f64', theta.device, theta, nb, friction, pairs, pairs.data_ptr() + 4 * npair, npair, length,
+              nlen, inertia, mu, half)
         ctx.save_for_backward(theta, friction, pairs, length)
         return inertia, mu, half
 
@@ -991,48 +826,37 @@ class LeafPrepare(torch.autograd.Function):
         g_theta, g_friction, g_length = torch.empty_like(theta), torch.empty_like(friction), torch.empty_like(length)
         cont = lambda g: None if g is None else g.contiguous()      # noqa: E731
         g_inertia, g_mu, g_half = cont(g_inertia), cont(g_mu), cont(g_half)
-        with torch.cuda.device(theta.device):
-            rc = _lib.load().dpll_leaf_backward_f64(_ptr(theta), nb, _ptr(friction), friction.numel(), pairs.data_ptr(),
-                                                    pairs.data_ptr() + 4 * npair, npair, _ptr(length), nlen, _ptr(g_inertia),
-                                                    _ptr(g_mu), _ptr(g_half), _ptr(g_theta), _ptr(g_friction),
-                                                    _ptr(g_length), _stream())
-        _lib.check(rc, 'dpll_leaf_backward')
+        _call('dpll_leaf_backward_f64', theta.device, theta, nb, friction, friction.numel(), pairs, pairs.data_ptr() + 4 * npair,
+              npair, length, nlen, g_inertia, g_mu, g_half, g_theta, g_friction, g_length)
         return g_theta, g_friction, None, g_length
+
+
+_SUPPORT_F64 = 'the support-network kernels are provided in float64'
 
 
 def elbow_support_directions(q: Tensor, axis: Tensor, pert0: Tensor, pert1: Tensor):
     """``dpll_elbow_support_directions_f64``: q (B, >= 8) rows (any row stride) -> the two links' perturbed, normalised
     support directions (B, n_query, 3) each.  float64, no autograd (directions are data, geometry.py:309-325)."""
-    _check_inputs(q, axis, pert0, pert1)
-    if q.dtype != torch.float64:
-        raise TypeError('the support-network kernels are provided in float64')
+    _check_inputs(q, axis, pert0, pert1, f64_only=_SUPPORT_F64)
     if q.dim() != 2 or q.shape[1] < 8 or q.stride(1) != 1:
         raise ValueError(f'expected (B, >= 8) configuration rows with unit column stride, got {tuple(q.shape)}')
     B, nq = q.shape[0], pert0.shape[0]
     d0 = torch.empty((B, nq, 3), dtype=q.dtype, device=q.device)
     d1 = torch.empty((B, nq, 3), dtype=q.dtype, device=q.device)
-    with torch.cuda.device(q.device):
-        rc = _lib.load().dpll_elbow_support_directions_f64(_ptr(q), q.stride(0) if B > 1 else q.shape[1], _ptr(axis.contiguous()),
-                                                           _ptr(pert0.contiguous()), _ptr(pert1.contiguous()), nq, B,
-                                                           _ptr(d0), _ptr(d1), _stream())
-    _lib.check(rc, 'dpll_elbow_support_directions')
+    _call('dpll_elbow_support_directions_f64', q.device, q, q.stride(0) if B > 1 else q.shape[1], axis.contiguous(),
+          pert0.contiguous(), pert1.contiguous(), nq, B, d0, d1)
     return d0, d1
 
 
 def body_support_directions(q: Tensor, pert: Tensor) -> Tensor:
     """``dpll_body_support_directions_f64``: q (B, >= 4) rows (any row stride, quaternion first) -> the body's perturbed,
     normalised support directions (B, n_query, 3) against the ground.  float64, no autograd (directions are data)."""
-    _check_inputs(q, pert)
-    if q.dtype != torch.float64:
-        raise TypeError('the support-network kernels are provided in float64')
+    _check_inputs(q, pert, f64_only=_SUPPORT_F64)
     if q.dim() != 2 or q.shape[1] < 4 or q.stride(1) != 1:
         raise ValueError(f'expected (B, >= 4) configuration rows with unit column stride, got {tuple(q.shape)}')
     B, nq = q.shape[0], pert.shape[0]
     d = torch.empty((B, nq, 3), dtype=q.dtype, device=q.device)
-    with torch.cuda.device(q.device):
-        rc = _lib.load().dpll_body_support_directions_f64(_ptr(q), q.stride(0) if B > 1 else q.shape[1],
-                                                          _ptr(pert.contiguous()), nq, B, _ptr(d), _stream())
-    _lib.check(rc, 'dpll_body_support_directions')
+    _call('dpll_body_support_directions_f64', q.device, q, q.stride(0) if B > 1 else q.shape[1], pert.contiguous(), nq, B, d)
     return d
 
 
@@ -1046,32 +870,24 @@ def icnn_support_points(d: Tensor, Wd0: Tensor, Wd1: Tensor, Wh: Tensor, wout: T
 
 def icnn_tc_prepare(Wd0: Tensor, Wd1: Tensor, Wh: Tensor, wout: Tensor, slope: float):
     """``dpll_icnn_tc_prepare_f64``: the four weights -> (digit-plane image, epilogue constants) of the tensor-core kernels."""
-    _check_inputs(Wd0, Wd1, Wh, wout)
-    if Wd0.dtype != torch.float64:
-        raise TypeError('the support-network kernels are provided in float64')
+    _check_inputs(Wd0, Wd1, Wh, wout, f64_only=_SUPPORT_F64)
     lib = _lib.load()
     Wd0, Wd1, Wh, wout = (t.contiguous() for t in (Wd0, Wd1, Wh, wout))
     dev = Wd0.device
     image = torch.empty(lib.dpll_icnn_tc_image_bytes(), dtype=torch.uint8, device=dev)
     consts = torch.empty(lib.dpll_icnn_tc_const_bytes() // 8, dtype=torch.float64, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(lib.dpll_icnn_tc_prepare_f64(_ptr(Wd0), _ptr(Wd1), _ptr(Wh), _ptr(wout), Wd0.shape[1], slope, _ptr(image),
-                                                _ptr(consts), _stream()), 'dpll_icnn_tc_prepare')
+    _call('dpll_icnn_tc_prepare_f64', dev, Wd0, Wd1, Wh, wout, Wd0.shape[1], slope, image, consts)
     return image, consts
 
 
 def icnn_support_points_tc(d: Tensor, Wd0: Tensor, Wd1: Tensor, Wh: Tensor, wout: Tensor, slope: float, prepared=None) -> Tensor:
     """``dpll_icnn_tc_support_f64``: support points (D,3) on the tensor cores (``prepared`` = ``icnn_tc_prepare`` output)."""
-    _check_inputs(d, Wh)
-    if d.dtype != torch.float64:
-        raise TypeError('the support-network kernels are provided in float64')
+    _check_inputs(d, Wh, f64_only=_SUPPORT_F64)
     image, consts = prepared if prepared is not None else icnn_tc_prepare(Wd0, Wd1, Wh, wout, slope)
     d, Wh = d.contiguous(), Wh.contiguous()
     D = d.shape[0]
     p = torch.empty((D, 3), dtype=d.dtype, device=d.device)
-    with torch.cuda.device(d.device):
-        _lib.check(_lib.load().dpll_icnn_tc_support_f64(_ptr(d), D, _ptr(image), _ptr(consts), _ptr(Wh), Wh.shape[0], slope,
-                                                        _ptr(p), _stream()), 'dpll_icnn_tc_support')
+    _call('dpll_icnn_tc_support_f64', d.device, d, D, image, consts, Wh, Wh.shape[0], slope, p)
     return p
 
 
@@ -1107,11 +923,8 @@ def icnn_support_backward_tc(d: Tensor, gp: Tensor, Wh: Tensor, slope: float, pr
         partial = torch.empty(lib.dpll_icnn_tc_bwd_partial_bytes() // 4, dtype=torch.int32, device=dev)
         sums = torch.empty(6 * W + 3, dtype=torch.float64, device=dev)
         Cb = torch.empty((3, W, W), dtype=torch.float64, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(lib.dpll_icnn_tc_record_f64(_ptr(d_act), cap, _ptr(n), _ptr(image), _ptr(consts), _ptr(Wh), W, slope,
-                                                   _ptr(m0t), _ptr(m1t), ldk, _stream()), 'dpll_icnn_tc_record')
-            _lib.check(lib.dpll_icnn_tc_bwd_f64(_ptr(g_act), _ptr(n), _ptr(amax), _ptr(m0t), _ptr(m1t), ldk, slope, _ptr(planes),
-                                                _ptr(partial), _ptr(sums), _ptr(Cb), _stream()), 'dpll_icnn_tc_bwd')
+        _call('dpll_icnn_tc_record_f64', dev, d_act, cap, n, image, consts, Wh, W, slope, m0t, m1t, ldk)
+        _call('dpll_icnn_tc_bwd_f64', dev, g_act, n, amax, m0t, m1t, ldk, slope, planes, partial, sums, Cb)
         C += Cb
         R1 += sums[3 * W:6 * W].reshape(3, W)
         S += sums[6 * W:]
@@ -1126,10 +939,7 @@ def icnn_support_forward(d: Tensor, Wd0: Tensor, Wd1: Tensor, Wh: Tensor, wout: 
     """Support points p (D,3) of the depth-2 homogeneous ICNN for unit directions d (D,3), float64, CUDA:
     the ``dpll_icnn_*`` kernels around two FP64 GEMMs.  Returns (p, h0aug, m1, a0) -- the last three are what
     the backward needs."""
-    _check_inputs(d, Wd0, Wd1, Wh, wout)
-    if d.dtype != torch.float64:
-        raise TypeError('the support-network kernels are provided in float64')
-    lib = _lib.load()
+    _check_inputs(d, Wd0, Wd1, Wh, wout, f64_only=_SUPPORT_F64)
     d, Wd0 = d.contiguous(), Wd0.contiguous()
     D, W = d.shape[0], Wd0.shape[1]
     dev = d.device
@@ -1138,31 +948,26 @@ def icnn_support_forward(d: Tensor, Wd0: Tensor, Wd1: Tensor, Wh: Tensor, wout: 
     W_aug = torch.cat((Wh_a, Wd1, torch.zeros((5, W), dtype=d.dtype, device=dev)), 0)
     V1 = (Wd1 * wo).contiguous()
     p = torch.empty((D, 3), dtype=d.dtype, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(lib.dpll_icnn_input_f64(_ptr(d), _ptr(Wd0), D, W, slope, _ptr(h0aug), _stream()), 'dpll_icnn_input')
-        m1 = h0aug @ W_aug                                   # z1 = h0 |Wh| + d Wd1
-        _lib.check(lib.dpll_icnn_mask_f64(_ptr(m1), m1.numel(), slope, _stream()), 'dpll_icnn_mask')
-        a0 = m1 @ (wo[:, None] * Wh_a.t())                   # T, turned into a0 in place below
-        _lib.check(lib.dpll_icnn_output_f64(_ptr(a0), _ptr(h0aug), _ptr(m1), _ptr(Wd0), _ptr(V1), D, W, slope, _ptr(p),
-                                            _stream()), 'dpll_icnn_output')
+    _call('dpll_icnn_input_f64', dev, d, Wd0, D, W, slope, h0aug)
+    m1 = h0aug @ W_aug                                   # z1 = h0 |Wh| + d Wd1
+    _call('dpll_icnn_mask_f64', dev, m1, m1.numel(), slope)
+    a0 = m1 @ (wo[:, None] * Wh_a.t())                   # T, turned into a0 in place below
+    _call('dpll_icnn_output_f64', dev, a0, h0aug, m1, Wd0, V1, D, W, slope, p)
     return p, h0aug, m1, a0
 
 
 def icnn_support_backward(gp: Tensor, h0aug: Tensor, m1: Tensor, a0: Tensor, Wd0: Tensor, slope: float):
     """Returns (g1 = gp^T m1 (3,W), gWd0 = gp^T a0 (3,W), G = t^T m1 (W,W)) with t = (gp Wd0) o m0."""
     _check_inputs(gp, h0aug, m1, a0, Wd0)
-    lib = _lib.load()
     gp, Wd0 = gp.contiguous(), Wd0.contiguous()
     D, W = m1.shape
     dev = gp.device
-    blocks = lib.dpll_icnn_backward_blocks(D)
+    blocks = _lib.load().dpll_icnn_backward_blocks(D)
     t = torch.empty((D, W), dtype=gp.dtype, device=dev)
     part = torch.zeros((max(blocks, 1), 6, W), dtype=gp.dtype, device=dev)   # zeros: D == 0 launches nothing
-    with torch.cuda.device(dev):
-        _lib.check(lib.dpll_icnn_backward_f64(_ptr(gp), _ptr(h0aug), _ptr(m1), _ptr(a0), _ptr(Wd0), D, W, slope, _ptr(t),
-                                              _ptr(part), _stream()), 'dpll_icnn_backward')
-        sums = part.sum(0)
-        G = t.t() @ m1
+    _call('dpll_icnn_backward_f64', dev, gp, h0aug, m1, a0, Wd0, D, W, slope, t, part)
+    sums = part.sum(0)
+    G = t.t() @ m1
     return sums[:3], sums[3:], G
 
 
@@ -1170,16 +975,15 @@ def fma_peak(dtype: torch.dtype, device: torch.device, blocks: int, iters: int, 
     """Measured FMA throughput (FLOP/s) of the CUDA cores for ``dtype`` -- roofline denominator.  Best of
     ``reps`` runs (a peak: a run disturbed by clock ramp-up would understate the denominator)."""
     out = torch.empty(blocks * 256, dtype=dtype, device=device)
-    fn = getattr(_lib.load(), 'dpll_fma_peak_' + _SUFFIX[dtype])
+    stream = torch.cuda.current_stream(out.device)
     best = float('inf')
-    with torch.cuda.device(device):
-        _lib.check(fn(_ptr(out), blocks, iters // 4 + 1, _stream()), 'dpll_fma_peak')   # warm-up
+    _call('dpll_fma_peak', out.device, out, blocks, iters // 4 + 1, dtype=dtype)      # warm-up
+    torch.cuda.synchronize(device)
+    for _ in range(max(1, reps)):
+        start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        start.record(stream)
+        _call('dpll_fma_peak', out.device, out, blocks, iters, dtype=dtype)
+        stop.record(stream)
         torch.cuda.synchronize(device)
-        for _ in range(max(1, reps)):
-            start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            start.record()
-            _lib.check(fn(_ptr(out), blocks, iters, _stream()), 'dpll_fma_peak')
-            stop.record()
-            torch.cuda.synchronize(device)
-            best = min(best, start.elapsed_time(stop))
+        best = min(best, start.elapsed_time(stop))
     return blocks * 256 * iters * 16 * 2 / (best * 1e-3)
