@@ -7,7 +7,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, 'csrc')
 LIB_PATH = os.path.join(_HERE, 'libdair_pll_b200.so')
 SOURCES = ['cn_kernels.cu', 'cn_tangent.cu', 'cn_tangent_elbow.cu', 'cn_icnn.cu', 'cn_comm.cu', 'cn_adjoint.cu', 'cn_elbow_wf.cu', 'cn_chain.cu', 'cn_icnn_tc.cu', 'cn_icnn_tc_bwd.cu', 'cn_leaf.cu', 'cn_tangent_chain.cu']
-HEADERS = ['cn_common.cuh', 'cn_cube.cuh', 'cn_params.cuh', 'cn_elbow.cuh', 'cn_dual.cuh', 'cn_cube_tangent.cuh', 'cn_elbow_tangent.cuh', 'cn_comm.cuh', 'cn_cube_adjoint.cuh', 'cn_elbow_wf.cuh', 'cn_chain.cuh', 'cn_chain_tangent.cuh', 'cn_icnn_tc.cuh', os.path.join('..', '..', 'include', 'dair_pll_b200.h')]
+HEADERS = ['cn_common.cuh', 'cn_cube.cuh', 'cn_params.cuh', 'cn_elbow.cuh', 'cn_dual.cuh', 'cn_cube_tangent.cuh', 'cn_elbow_tangent.cuh', 'cn_comm.cuh', 'cn_cube_adjoint.cuh', 'cn_elbow_wf.cuh', 'cn_chain.cuh', 'cn_chain_tangent.cuh', 'cn_icnn_tc.cuh', 'cn_launch.cuh', 'cn_reduce.cuh', os.path.join('..', '..', 'include', 'dair_pll_b200.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC']
 

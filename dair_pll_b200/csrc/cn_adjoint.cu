@@ -4,6 +4,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_cube_adjoint.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -38,12 +39,9 @@ int dpll_cube_rollout_backward_f64(const double* traj, const double* usol, const
   if (B > 0 && (!traj || !gparams || !gx0 || (steps > 0 && (!usol || !xbar)))) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
   // a toss is one sequential chain: spread the tosses over as many warps as there are (2 per warp at 4,096 tosses)
-  const int threads = 64;
-  const int blocks = (int)((B + threads - 1) / threads);
-  cube_rollout_backward_kernel<double><<<blocks, threads, 0, static_cast<cudaStream_t>(stream)>>>(
+  cube_rollout_backward_kernel<double><<<cn::grid_for(B, 64), 64, 0, static_cast<cudaStream_t>(stream)>>>(
       traj, usol, inertia, mu_pair, half, dt, eps, B, steps, xbar, gparams, gx0);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

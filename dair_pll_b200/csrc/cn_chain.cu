@@ -4,12 +4,14 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_chain.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
 constexpr int kChThreads = 64;
 constexpr int kChNAcc = 96;                 // 14 N parameter gradients + loss sum (N <= 6: 85)
-constexpr int kChMaxBlocks = 148 * 5;       // partials fit the common workspace (dpll_workspace_bytes)
+constexpr int kChMaxBlocks = 148 * 5;
+static_assert((size_t)kChMaxBlocks * kChNAcc * sizeof(double) <= cn::kWsPartialsBytes, "chain partials exceed the workspace");
 
 template <typename T> __device__ __forceinline__ T ch_warp_sum(T v) {
 #pragma unroll
@@ -106,30 +108,17 @@ int launch_chain_loss(const double* x, const double* xp, const double* weight, c
                       int32_t* iters, double* grad, double* loss_sum, void* workspace, size_t workspace_bytes,
                       cudaStream_t st, const double* pts = nullptr, unsigned npts = 0u, double* grad_pts = nullptr) {
   const bool want_red = grad || loss_sum;
-  if (want_red && (!workspace || workspace_bytes < dpll_workspace_bytes())) return DPLL_EWORKSPACE;
+  if (want_red && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
   int64_t need = (B + kChThreads - 1) / kChThreads;
   int blocks = (int)(need < kChMaxBlocks ? need : kChMaxBlocks);
   if (blocks < 1) blocks = 1;
   double* partials = want_red ? static_cast<double*>(workspace) : nullptr;
   chain_loss_kernel<double, N><<<blocks, kChThreads, 0, st>>>(x, xp, weight, inertia, mu, half, kin, dt, eps, B, loss, force,
                                                              iters, partials, grad ? 1 : 0, pts, npts, grad_pts);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return (int)e;
-  if (want_red) {
-    chain_reduce_kernel<double><<<1, 512, 0, st>>>(partials, blocks, 14 * N, grad, loss_sum);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-  }
-  return DPLL_OK;
-}
-
-template <int N>
-int launch_chain_rollout(const double* x0, const double* inertia, const double* mu, const double* half, const double* kin,
-                         double dt, double eps, int64_t B, int steps, double* traj, cudaStream_t st) {
-  const int blocks = (int)((B + kChThreads - 1) / kChThreads);
-  chain_rollout_kernel<double, N><<<blocks, kChThreads, 0, st>>>(x0, inertia, mu, half, kin, dt, eps, B, steps, traj);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  if (int rc = cn::launch_status()) return rc;
+  if (!want_red) return DPLL_OK;
+  chain_reduce_kernel<double><<<1, 512, 0, st>>>(partials, blocks, 14 * N, grad, loss_sum);
+  return cn::launch_status();
 }
 
 // Dense terms export (MultibodyTerms.forward, multibody_terms.py:584-609) for a tree; one sample per thread.
@@ -152,16 +141,6 @@ chain_terms_kernel(const T* __restrict__ q, const T* __restrict__ v, const T* __
                                D ? D + b * kk * kk : (T*)nullptr);
 }
 
-template <int N>
-int launch_chain_terms(const double* q, const double* v, const double* inertia, const double* mu, const double* half,
-                       const double* kin, int n_boxes, int64_t B, double* M, double* J, double* phi, double* acc, double* D,
-                       cudaStream_t st) {
-  const int blocks = (int)((B + kChThreads - 1) / kChThreads);
-  chain_terms_kernel<double, N><<<blocks, kChThreads, 0, st>>>(q, v, inertia, mu, half, kin, n_boxes, B, M, J, phi, acc, D);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
-}
-
 }  // namespace
 
 extern "C" {
@@ -172,20 +151,10 @@ int dpll_chain_loss_f64(int32_t n_links, const double* x, const double* x_plus, 
                         size_t workspace_bytes, void* stream) {
   if (B < 0 || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
   if (B > 0 && (!x || !x_plus)) return DPLL_EINVAL;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  switch (n_links) {
-    case 2: return launch_chain_loss<2>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
-                                        loss_sum, workspace, workspace_bytes, st);
-    case 3: return launch_chain_loss<3>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
-                                        loss_sum, workspace, workspace_bytes, st);
-    case 5: return launch_chain_loss<5>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
-                                        loss_sum, workspace, workspace_bytes, st);
-    case 6: return launch_chain_loss<6>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
-                                        loss_sum, workspace, workspace_bytes, st);
-    case 4: return launch_chain_loss<4>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
-                                        loss_sum, workspace, workspace_bytes, st);
-    default: return DPLL_EINVAL;
-  }
+  return cn::with_links(n_links, [&](auto N) {
+    return launch_chain_loss<N>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
+                                loss_sum, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+  });
 }
 
 int dpll_chain_rollout_f64(int32_t n_links, const double* x0, const double* inertia, const double* mu_pair,
@@ -194,15 +163,11 @@ int dpll_chain_rollout_f64(int32_t n_links, const double* x0, const double* iner
   if (B < 0 || steps < 0 || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
   if (B > 0 && (!x0 || !traj)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  switch (n_links) {
-    case 2: return launch_chain_rollout<2>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, traj, st);
-    case 3: return launch_chain_rollout<3>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, traj, st);
-    case 4: return launch_chain_rollout<4>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, traj, st);
-    case 5: return launch_chain_rollout<5>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, traj, st);
-    case 6: return launch_chain_rollout<6>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, traj, st);
-    default: return DPLL_EINVAL;
-  }
+  return cn::with_links(n_links, [&](auto N) {
+    chain_rollout_kernel<double, N><<<cn::grid_for(B, kChThreads), kChThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        x0, inertia, mu_pair, half, kin, dt, eps, B, steps, traj);
+    return cn::launch_status();
+  });
 }
 
 int dpll_chain_terms_f64(int32_t n_links, int32_t n_boxes, const double* q, const double* v, const double* inertia,
@@ -211,15 +176,11 @@ int dpll_chain_terms_f64(int32_t n_links, int32_t n_boxes, const double* q, cons
   if (B < 0 || n_boxes < 1 || n_boxes > n_links || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
   if (B > 0 && (!q || !v || !M || !J || !phi || !acc)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  switch (n_links) {
-    case 2: return launch_chain_terms<2>(q, v, inertia, mu_pair, half, kin, n_boxes, B, M, J, phi, acc, delassus, st);
-    case 3: return launch_chain_terms<3>(q, v, inertia, mu_pair, half, kin, n_boxes, B, M, J, phi, acc, delassus, st);
-    case 4: return launch_chain_terms<4>(q, v, inertia, mu_pair, half, kin, n_boxes, B, M, J, phi, acc, delassus, st);
-    case 5: return launch_chain_terms<5>(q, v, inertia, mu_pair, half, kin, n_boxes, B, M, J, phi, acc, delassus, st);
-    case 6: return launch_chain_terms<6>(q, v, inertia, mu_pair, half, kin, n_boxes, B, M, J, phi, acc, delassus, st);
-    default: return DPLL_EINVAL;
-  }
+  return cn::with_links(n_links, [&](auto N) {
+    chain_terms_kernel<double, N><<<cn::grid_for(B, kChThreads), kChThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        q, v, inertia, mu_pair, half, kin, n_boxes, B, M, J, phi, acc, delassus);
+    return cn::launch_status();
+  });
 }
 
 int dpll_chain_loss_pts_f64(int32_t n_links, const double* x, const double* x_plus, const double* weight, const double* inertia,
@@ -229,16 +190,11 @@ int dpll_chain_loss_pts_f64(int32_t n_links, const double* x, const double* x_pl
   if (B < 0 || !inertia || !mu_pair || !kin) return DPLL_EINVAL;
   if (B > 0 && (!x || !x_plus || !pts)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-#define DPLL_CHAIN_PTS_CASE(NL)                                                                                               \
-  case NL:                                                                                                                    \
-    return launch_chain_loss<NL>(x, x_plus, weight, inertia, mu_pair, nullptr, kin, dt, eps, B, loss, nullptr, nullptr, grad,  \
-                                 loss_sum, workspace, workspace_bytes, st, pts, n_pts_packed, grad_pts);
-  switch (n_links) {
-    DPLL_CHAIN_PTS_CASE(2) DPLL_CHAIN_PTS_CASE(3) DPLL_CHAIN_PTS_CASE(4) DPLL_CHAIN_PTS_CASE(5) DPLL_CHAIN_PTS_CASE(6)
-    default: return DPLL_EINVAL;
-  }
-#undef DPLL_CHAIN_PTS_CASE
+  return cn::with_links(n_links, [&](auto N) {
+    return launch_chain_loss<N>(x, x_plus, weight, inertia, mu_pair, nullptr, kin, dt, eps, B, loss, nullptr, nullptr, grad,
+                                loss_sum, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), pts, n_pts_packed,
+                                grad_pts);
+  });
 }
 
 }  // extern "C"

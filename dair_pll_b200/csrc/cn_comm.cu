@@ -9,6 +9,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_comm.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -109,8 +110,7 @@ int dpll_comm_allreduce_f64(void* comm, double* buf, int32_t n, double scale, vo
   if (!c || !buf || n < 0 || n > cn::COMM_MAX_ELEMS) return DPLL_EINVAL;
   if (n == 0) return DPLL_OK;
   comm_allreduce_kernel<<<1, 64, 0, static_cast<cudaStream_t>(stream)>>>(c->dev, buf, n, scale);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

@@ -18,6 +18,8 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_elbow_wf.cuh"
+#include "cn_launch.cuh"
+#include "cn_reduce.cuh"
 
 namespace {
 
@@ -36,6 +38,7 @@ constexpr int kEwWarps = CN_EW_WARPS;
 constexpr int kEwQin = 64;
 constexpr int kEwNAcc = 32;       // 28 parameter gradients + loss sum + pad
 constexpr int kEwMaxBlocks = 148 * 16;
+static_assert((size_t)kEwMaxBlocks * kEwNAcc * sizeof(double) <= cn::kWsPartialsBytes, "elbow partials exceed the workspace");
 
 template <typename T> struct EwWarpPool {
   T field[cn::EW_FIELDS][kEwSlots];
@@ -293,39 +296,63 @@ elbow_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const 
   }
 }
 
-}  // namespace
-
-// Launcher used by cn_kernels.cu (launch_elbow_loss): returns the number of blocks launched, or a negative /
-// positive error code through *err.
 template <typename T, typename IO>
-int launch_elbow_loss_wf(const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
-                         const IO* kin, const IO* pts, T dt, T eps, int64_t B, IO* loss, IO* force, IO* grad_pts,
-                         int32_t* iters, T* partials, int want_grad, const int32_t* skip_flag, int sms, cudaStream_t st,
-                         int* err, unsigned long long* dyn) {
+int launch_elbow_loss(const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
+                      const IO* kin, const IO* pts, T dt, T eps, int64_t B, IO* loss, IO* force, IO* grad_pts,
+                      int32_t* iters, IO* grad, IO* loss_sum,
+                      const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream, int flags) {
+  if (B < 0 || !inertia || !mu || (!half && !pts) || !kin || (grad_pts && (!pts || !grad))) return DPLL_EINVAL;
+  if (B > 0 && (!x || !xp)) return DPLL_EINVAL;
+  const bool want_red = grad || loss_sum;
+  if (want_red && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  T* partials = want_red ? static_cast<T*>(workspace) : nullptr;
+  unsigned long long* dyn = nullptr;
+  if (flags & DPLL_LOSS_DYNAMIC) {
+    if (!cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
+    if (int rc = cn::dynamic_counter(workspace, st, &dyn)) return rc;
+  }
   const size_t smem = sizeof(EwWarpPool<T>) * kEwWarps;
   cudaError_t ea = cudaFuncSetAttribute(elbow_loss_wf_kernel<T, IO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (ea != cudaSuccess) { *err = (int)ea; return 0; }
-  int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, elbow_loss_wf_kernel<T, IO>, kEwWarps * 32, smem);
-  if (per_sm < 1) per_sm = 1;
-  int64_t need = (B + kEwWarps * 128 - 1) / (kEwWarps * 128);      // a warp wants >= 128 samples to keep its pool busy
-  int64_t cap = (int64_t)sms * per_sm;
-  if (cap > kEwMaxBlocks) cap = kEwMaxBlocks;
-  int blocks = (int)(need < cap ? need : cap);
-  if (blocks < 1) blocks = 1;
+  if (ea != cudaSuccess) return (int)ea;
+  // at most one resident set; a warp wants >= 128 samples to keep its pool busy
+  int blocks;
+  int64_t cap;
+  if (int rc = cn::resident_blocks(elbow_loss_wf_kernel<T, IO>, kEwWarps * 32, smem, (B + kEwWarps * 128 - 1) / (kEwWarps * 128),
+                                   kEwMaxBlocks, &blocks, &cap))
+    return rc;
   elbow_loss_wf_kernel<T, IO><<<blocks, kEwWarps * 32, smem, st>>>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B,
-                                                                   loss, force, grad_pts, iters, partials, want_grad,
+                                                                   loss, force, grad_pts, iters, partials, grad ? 1 : 0,
                                                                    skip_flag, dyn);
-  cudaError_t e = cudaGetLastError();
-  *err = e == cudaSuccess ? DPLL_OK : (int)e;
-  return blocks;
+  if (int rc = cn::launch_status()) return rc;
+  if (!want_red) return DPLL_OK;
+  reduce_partials_kernel<T, IO, kEwNAcc, DPLL_ELBOW_NPARAM><<<1, 32 * kEwNAcc, 0, st>>>(partials, blocks, grad, loss_sum,
+                                                                                       skip_flag);
+  return cn::launch_status();
 }
 
-template int launch_elbow_loss_wf<double, double>(const double*, const double*, const double*, const double*, const double*,
-                                                  const double*, const double*, const double*, double, double, int64_t,
-                                                  double*, double*, double*, int32_t*, double*, int, const int32_t*, int,
-                                                  cudaStream_t, int*, unsigned long long*);
-template int launch_elbow_loss_wf<double, float>(const float*, const float*, const float*, const float*, const float*,
-                                                 const float*, const float*, const float*, double, double, int64_t, float*,
-                                                 float*, float*, int32_t*, double*, int, const int32_t*, int, cudaStream_t,
-                                                 int*, unsigned long long*);
+}  // namespace
+
+extern "C" {
+
+int dpll_elbow_loss_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
+                        const double* mu_pair, const double* half, const double* kin, const double* pts, double dt,
+                        double eps, int64_t B, int32_t flags, double* loss, double* force, double* grad_pts,
+                        int32_t* iters, double* grad, double* loss_sum, const int32_t* skip_flag, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  return launch_elbow_loss<double, double>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, loss, force,
+                                           grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream,
+                                           flags);
+}
+
+int dpll_elbow_loss_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
+                        const float* mu_pair, const float* half, const float* kin, const float* pts, float dt, float eps,
+                        int64_t B, int32_t flags, float* loss, float* force, float* grad_pts, int32_t* iters, float* grad,
+                        float* loss_sum, const int32_t* skip_flag, void* workspace, size_t workspace_bytes,
+                        void* stream) {
+  return launch_elbow_loss<double, float>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, (double)dt, (double)eps, B,
+                                          loss, force, grad_pts, iters, grad, loss_sum, skip_flag, workspace,
+                                          workspace_bytes, stream, flags);
+}
+
+}  // extern "C"

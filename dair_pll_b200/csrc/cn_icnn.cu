@@ -18,6 +18,7 @@
 #include <cstdint>
 
 #include "../../include/dair_pll_b200.h"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -155,11 +156,6 @@ __global__ void body_support_directions_kernel(const double* __restrict__ q, int
   }
 }
 
-int grid_for(int64_t work, int per_block) {
-  int64_t b = (work + per_block - 1) / per_block;
-  return (int)(b < 1 ? 1 : (b > 2147483647LL ? 2147483647LL : b));
-}
-
 }  // namespace
 
 extern "C" {
@@ -169,9 +165,8 @@ int dpll_icnn_input_f64(const double* d, const double* Wd0, int64_t D, int32_t W
   if (D < 0 || W <= 0 || !Wd0) return DPLL_EINVAL;
   if (D == 0) return DPLL_OK;
   if (!d || !h0aug) return DPLL_EINVAL;
-  icnn_input_kernel<<<grid_for(D, kRowsPerBlock), 288, 0, static_cast<cudaStream_t>(stream)>>>(d, Wd0, D, W, slope, h0aug);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  icnn_input_kernel<<<cn::grid_for(D, kRowsPerBlock), 288, 0, static_cast<cudaStream_t>(stream)>>>(d, Wd0, D, W, slope, h0aug);
+  return cn::launch_status();
 }
 
 int dpll_elbow_support_directions_f64(const double* q, int64_t q_stride, const double* axis, const double* pert0,
@@ -180,10 +175,9 @@ int dpll_elbow_support_directions_f64(const double* q, int64_t q_stride, const d
   if (B < 0 || n_query <= 0 || q_stride < 8 || !axis || !pert0 || !pert1) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
   if (!q || !dirs0 || !dirs1) return DPLL_EINVAL;
-  elbow_support_directions_kernel<<<grid_for(B, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+  elbow_support_directions_kernel<<<cn::grid_for(B, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       q, q_stride, axis, pert0, pert1, n_query, B, dirs0, dirs1);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_body_support_directions_f64(const double* q, int64_t q_stride, const double* pert, int32_t n_query, int64_t B,
@@ -191,21 +185,19 @@ int dpll_body_support_directions_f64(const double* q, int64_t q_stride, const do
   if (B < 0 || n_query <= 0 || q_stride < 4 || !pert) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
   if (!q || !dirs) return DPLL_EINVAL;
-  body_support_directions_kernel<<<grid_for(B, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(q, q_stride, pert, n_query,
+  body_support_directions_kernel<<<cn::grid_for(B, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(q, q_stride, pert, n_query,
                                                                                                   B, dirs);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_icnn_mask_f64(double* z, int64_t n, double slope, void* stream) {
   if (n < 0) return DPLL_EINVAL;
   if (n == 0) return DPLL_OK;
   if (!z) return DPLL_EINVAL;
-  int blocks = grid_for(n, 256 * 8);
+  int blocks = cn::grid_for(n, 256 * 8);
   if (blocks > 148 * 16) blocks = 148 * 16;
   icnn_mask_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(z, n, slope);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_icnn_output_f64(double* T, const double* h0aug, const double* m1, const double* Wd0, const double* V1, int64_t D,
@@ -213,11 +205,10 @@ int dpll_icnn_output_f64(double* T, const double* h0aug, const double* m1, const
   if (D < 0 || W <= 0 || !Wd0 || !V1) return DPLL_EINVAL;
   if (D == 0) return DPLL_OK;
   if (!T || !h0aug || !m1 || !p) return DPLL_EINVAL;
-  int blocks = grid_for(D, 8);                 // 8 warps (rows) per block of 256 threads
+  int blocks = cn::grid_for(D, 8);                 // 8 warps (rows) per block of 256 threads
   if (blocks > 148 * 8) blocks = 148 * 8;
   icnn_output_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(T, h0aug, m1, Wd0, V1, D, W, slope, p);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 // rows per block: 512 for large batches; small batches (the active rows of a step) still get ~4 blocks per SM
@@ -227,7 +218,7 @@ static int backward_rows_per_block(int64_t D) {
   return rows;
 }
 
-int dpll_icnn_backward_blocks(int64_t D) { return grid_for(D, backward_rows_per_block(D)); }
+int dpll_icnn_backward_blocks(int64_t D) { return cn::grid_for(D, backward_rows_per_block(D)); }
 
 int dpll_icnn_backward_f64(const double* gp, const double* h0aug, const double* m1, const double* a0, const double* Wd0,
                            int64_t D, int32_t W, double slope, double* t, double* part, void* stream) {
@@ -236,8 +227,7 @@ int dpll_icnn_backward_f64(const double* gp, const double* h0aug, const double* 
   if (!gp || !h0aug || !m1 || !a0 || !t || !part) return DPLL_EINVAL;
   icnn_backward_kernel<<<dpll_icnn_backward_blocks(D), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       gp, h0aug, m1, a0, Wd0, D, W, slope, backward_rows_per_block(D), t, part);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

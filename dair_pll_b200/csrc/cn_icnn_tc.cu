@@ -21,6 +21,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_icnn_tc.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -463,13 +464,6 @@ icnn_tc_prepare_kernel(const double* __restrict__ Wd0, const double* __restrict_
   }
 }
 
-int sm_count() {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return sms;
-}
-
 }  // namespace
 
 extern "C" {
@@ -482,8 +476,7 @@ int dpll_icnn_tc_prepare_f64(const double* Wd0, const double* Wd1, const double*
   if (W != cn::TC_W || !Wd0 || !Wd1 || !Wh || !wout || !image || !consts) return DPLL_EINVAL;
   icnn_tc_prepare_kernel<<<cn::TC_W, cn::TC_W, 0, static_cast<cudaStream_t>(stream)>>>(
       Wd0, Wd1, Wh, wout, slope, static_cast<uint8_t*>(image), consts);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_icnn_tc_support_f64(const double* d, int64_t D, const void* image, const double* consts, const double* Wh,
@@ -494,12 +487,12 @@ int dpll_icnn_tc_support_f64(const double* d, int64_t D, const void* image, cons
   cudaError_t e = cudaFuncSetAttribute(icnn_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e != cudaSuccess) return (int)e;
   const int64_t ntiles = (D + kTileRows - 1) / kTileRows;
-  const int sms = sm_count();
+  int sms = 0;
+  if (int rc = cn::sm_count(&sms)) return rc;
   const int grid = (int)(ntiles < sms ? ntiles : sms);
   icnn_tc_kernel<false><<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
       d, D, nullptr, static_cast<const uint8_t*>(image), consts, Wh, slope, p, nullptr, nullptr, 0);
-  e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_icnn_tc_record_f64(const double* d, int64_t capacity, const int64_t* n_rows, const void* image, const double* consts,
@@ -510,12 +503,12 @@ int dpll_icnn_tc_record_f64(const double* d, int64_t capacity, const int64_t* n_
   cudaError_t e = cudaFuncSetAttribute(icnn_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e != cudaSuccess) return (int)e;
   const int64_t ntiles = (capacity + kTileRows - 1) / kTileRows;
-  const int sms = sm_count();
+  int sms = 0;
+  if (int rc = cn::sm_count(&sms)) return rc;
   const int grid = (int)(ntiles < sms ? ntiles : sms);
   icnn_tc_kernel<true><<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
       d, capacity, n_rows, static_cast<const uint8_t*>(image), consts, Wh, slope, nullptr, m0t, m1t, ldk);
-  e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

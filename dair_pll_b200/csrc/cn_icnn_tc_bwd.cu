@@ -25,6 +25,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_icnn_tc.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -313,8 +314,7 @@ int dpll_icnn_tc_bwd_f64(const double* gp, const int64_t* n_rows, const double* 
   if (e != cudaSuccess) return (int)e;
   bwd_gram_kernel<<<TCB_BLOCKS * TCB_CHUNKS, kGramThreads, kGramSmem, st>>>(n_rows, m0t, m1t, planes, ldk, partial);
   bwd_finish_kernel<<<3 * TC_W, TC_W, 0, st>>>(partial, sums, amax, slope, C);
-  e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

@@ -13,34 +13,15 @@
 #include "cn_elbow.cuh"
 #include "cn_elbow_wf.cuh"
 #include "cn_comm.cuh"
-
-// wavefront kernel of the two-body system (cn_elbow_wf.cu)
-template <typename T, typename IO>
-int launch_elbow_loss_wf(const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
-                         const IO* kin, const IO* pts, T dt, T eps, int64_t B, IO* loss, IO* force, IO* grad_pts,
-                         int32_t* iters, T* partials, int want_grad, const int32_t* skip_flag, int sms, cudaStream_t st,
-                         int* err, unsigned long long* dyn);
+#include "cn_launch.cuh"
+#include "cn_reduce.cuh"
 
 namespace {
 
 constexpr int kLossThreads = 128;
 constexpr int kNAcc = 16;            // 14 parameter gradients + loss sum + pad
-constexpr int kMaxBlocks = 148 * 16; // upper bound used to size the workspace
-// workspace: [per-block partials kMaxBlocks x 32 doubles | 16 prepared parameters | chunk counter of the dynamic schedule]
-constexpr size_t kWsQueueOffset = ((size_t)kMaxBlocks * 32 + 16) * sizeof(double);
-constexpr size_t kWsQueueBytes = 2 * sizeof(unsigned long long);
-
-struct DeviceInfo { int sms; int device; };
-inline DeviceInfo device_info() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  static int cached_dev = -1, cached_sms = 0;
-  if (cached_dev != dev) {
-    cudaDeviceGetAttribute(&cached_sms, cudaDevAttrMultiProcessorCount, dev);
-    cached_dev = dev;
-  }
-  return {cached_sms, dev};
-}
+constexpr int kMaxBlocks = 148 * 16; // most blocks of a loss launch (box and witness points)
+static_assert((size_t)kMaxBlocks * kNAcc * sizeof(double) <= cn::kWsPartialsBytes, "box partials exceed the workspace");
 
 // Tosses per warp of a rollout launch.  A toss is a chain of dependent steps, so a warp is issue-bound by its own
 // instruction stream whatever its number of active lanes (ncu, 4,096 x 80 at four tosses per warp: 2.2 lanes per instruction
@@ -55,12 +36,6 @@ inline int rollout_tosses_per_warp(int64_t B, int sms, int64_t resident_warps) {
   if (lpw < 1) lpw = 1;
   if (lpw > 32) lpw = 32;
   return (int)lpw;
-}
-
-template <typename T> __device__ __forceinline__ T warp_sum(T v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
 }
 
 // load the callable-level parameters (stored as IO) into the compute type
@@ -531,23 +506,6 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
   }
 }
 
-// Fixed-order reduction of the per-block partials: warp w owns accumulator w.
-// NACC accumulators per block: [0, NPARAM) parameter gradients, slot NPARAM = loss sum.
-template <typename T, typename IO, int NACC, int NPARAM>
-__global__ void reduce_partials_kernel(const T* __restrict__ partials, int nblocks, IO* __restrict__ grad,
-                                       IO* __restrict__ loss_sum, const int32_t* __restrict__ skip_flag) {
-  if (skip_flag && *skip_flag) return;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  if (w >= NACC) return;
-  T s = T(0);
-  for (int b = lane; b < nblocks; b += 32) s += partials[(int64_t)b * NACC + w];
-  s = warp_sum(s);
-  if (lane == 0) {
-    if (w < NPARAM) { if (grad) grad[w] = IO(s); }
-    else if (w == NPARAM) { if (loss_sum) *loss_sum = IO(s); }
-  }
-}
-
 // ---- leaf-level parameter preparation / chain rule (cube: theta 10, friction 2 [box, ground], length 3) ----
 
 template <typename T, typename IO>
@@ -715,8 +673,6 @@ cube_terms_kernel(const IO* __restrict__ q, const IO* __restrict__ v, const IO* 
 // Elbow (floating base + hinge, 8 contacts): the loss kernel is the wavefront kernel in cn_elbow_wf.cu; rollout
 // and terms run one sample per thread, problem in thread-local arrays.
 // ---------------------------------------------------------------------------
-constexpr int kNAccE = 32;   // 28 parameter gradients + loss sum + pad
-
 template <typename T, typename IO>
 __device__ __forceinline__ void load_elbow_params(cn::ElbowParams<T>& P, const IO* inertia, const IO* mu, const IO* half,
                                                   const IO* kin, T dt, T eps) {
@@ -782,66 +738,6 @@ elbow_terms_kernel(const IO* __restrict__ q, const IO* __restrict__ v, const IO*
   for (int i = 0; i < 7; ++i) acc[b * 7 + i] = IO(ao[i]);
 }
 
-template <typename T, typename IO>
-int launch_elbow_loss(const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
-                      const IO* kin, const IO* pts, T dt, T eps, int64_t B, IO* loss, IO* force, IO* grad_pts,
-                      int32_t* iters, IO* grad, IO* loss_sum,
-                      const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream, int flags) {
-  if (B < 0 || !inertia || !mu || (!half && !pts) || !kin || (grad_pts && (!pts || !grad))) return DPLL_EINVAL;
-  if (B > 0 && (!x || !xp)) return DPLL_EINVAL;
-  const bool want_red = grad || loss_sum;
-  if (want_red && (!workspace || workspace_bytes < dpll_workspace_bytes())) return DPLL_EWORKSPACE;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const DeviceInfo di = device_info();
-  T* partials = want_red ? static_cast<T*>(workspace) : nullptr;
-  // wavefront kernel: per-visit scheduling over shared-memory records
-  int err = DPLL_OK;
-  unsigned long long* dyn = nullptr;
-  if (flags & DPLL_LOSS_DYNAMIC) {
-    if (!workspace || workspace_bytes < dpll_workspace_bytes()) return DPLL_EWORKSPACE;
-    dyn = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + kWsQueueOffset);
-    cudaError_t em = cudaMemsetAsync(dyn, 0, kWsQueueBytes, st);
-    if (em != cudaSuccess) return (int)em;
-  }
-  const int blocks = ::launch_elbow_loss_wf<T, IO>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B, loss, force,
-                                                   grad_pts, iters, partials, grad ? 1 : 0, skip_flag, di.sms, st, &err,
-                                                   dyn);
-  if (err != DPLL_OK) return err;
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return (int)e;
-  if (want_red) {
-    reduce_partials_kernel<T, IO, kNAccE, DPLL_ELBOW_NPARAM><<<1, 32 * kNAccE, 0, st>>>(partials, blocks, grad, loss_sum,
-                                                                                         skip_flag);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-  }
-  return DPLL_OK;
-}
-
-template <typename T, typename IO>
-int launch_elbow_rollout(const IO* x0, const IO* inertia, const IO* mu, const IO* half, const IO* kin, const IO* pts,
-                         T dt, T eps, int64_t B, int32_t steps, IO* traj, IO* force, int32_t* iters, void* stream,
-                         IO* usol = nullptr) {
-  if (B < 0 || steps < 0 || !inertia || !mu || (!half && !pts) || !kin || (pts && steps > 1)) return DPLL_EINVAL;
-  if (B > 0 && (!x0 || !traj)) return DPLL_EINVAL;
-  if (B == 0) return DPLL_OK;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const DeviceInfo di = device_info();
-  int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, elbow_rollout_kernel<T, IO>, kLossThreads, 0);
-  if (per_sm < 1) per_sm = 1;
-  const int64_t cap = (int64_t)di.sms * per_sm;
-  const int64_t warps = cap * (kLossThreads / 32);
-  const int lpw = rollout_tosses_per_warp(B, di.sms, warps);
-  const int64_t per_block = (int64_t)lpw * (kLossThreads / 32);
-  const int64_t need = (B + per_block - 1) / per_block;
-  const int blocks = (int)(need < cap ? need : cap);
-  elbow_rollout_kernel<T, IO><<<blocks, kLossThreads, 0, st>>>(x0, inertia, mu, half, kin, pts, dt, eps, B, steps, traj,
-                                                              force, iters, lpw, usol);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
-}
-
 template <typename T>
 __global__ void __launch_bounds__(256) fma_peak_kernel(T* out, int64_t iters) {
   T a[16];
@@ -858,23 +754,87 @@ __global__ void __launch_bounds__(256) fma_peak_kernel(T* out, int64_t iters) {
   out[(int64_t)blockIdx.x * blockDim.x + threadIdx.x] = s;
 }
 
-// Grid of a wavefront loss launch: at most one resident set of blocks (*cap), fewer for small batches -- a warp needs a
-// few hundred samples to keep its pool full; with fewer, every SM would run many mostly-empty warps at the issue rate of
-// full ones.
+// Grid and tosses per warp of a rollout launch (rollout_tosses_per_warp): at most one resident set of blocks.
 template <typename K>
-int wf_blocks(int64_t B, K kernel, size_t smem, int sms, int64_t* cap) {
-  int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kWfWarps * 32, smem);
-  if (per_sm < 1) per_sm = 1;
-  const int64_t need = (B + kWfWarps * kWfMinPerWarp - 1) / (kWfWarps * kWfMinPerWarp);
-  *cap = (int64_t)sms * per_sm;
-  if (*cap > kMaxBlocks) *cap = kMaxBlocks;
-  const int blocks = (int)(need < *cap ? need : *cap);
-  return blocks < 1 ? 1 : blocks;
+int rollout_grid(K kernel, int64_t B, int* blocks, int* lpw) {
+  int sms = 0;
+  int64_t cap;
+  if (int rc = cn::sm_count(&sms)) return rc;
+  if (int rc = cn::resident_cap(kernel, kLossThreads, 0, INT64_MAX, &cap)) return rc;
+  *lpw = rollout_tosses_per_warp(B, sms, cap * (kLossThreads / 32));
+  const int64_t per_block = (int64_t)*lpw * (kLossThreads / 32);
+  const int64_t need = (B + per_block - 1) / per_block;
+  *blocks = (int)(need < cap ? need : cap);
+  return DPLL_OK;
 }
 
 constexpr int64_t kRaceMaxBatch = 300000;     // larger launches are bound by throughput, not by their longest chain
 constexpr int64_t kRaceMaxHead = 2048;
+
+// Wavefront loss launch of the single body: box corners, or witness points (PTS; the arguments are packed as
+// cube_loss_wf_kernel describes).  Sets the shared-memory size of every instance it may launch, picks the grid and the
+// instance by batch size, resets the chunk counter of the dynamic schedule and launches.  *rows = the number of blocks
+// that write partials.
+template <typename T, typename IO, bool PTS>
+int launch_cube_wf(bool dynamic, int flags, const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu,
+                   const IO* half, T dt, T eps, int64_t B, IO* loss, IO* force, int32_t* iters, T* partials,
+                   int want_grad, const int32_t* skip_flag, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                   int64_t ldx, int64_t ldxp, const IO* u_init, IO* u_out, int* rows) {
+  const size_t smem = sizeof(WfWarpPool<T>) * kWfWarps;
+  cudaError_t ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, kWfUnr, false, PTS>,
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (ea == cudaSuccess)
+    ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, 4, false, PTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              (int)smem);
+  if constexpr (!PTS) {
+    if (ea == cudaSuccess)
+      ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  }
+  if (ea != cudaSuccess) return (int)ea;
+  // at most one resident set of blocks, fewer for small batches -- a warp needs a few hundred samples to keep its pool
+  // full; with fewer, every SM would run many mostly-empty warps at the issue rate of full ones
+  int blocks;
+  int64_t cap;
+  if (int rc = cn::resident_blocks(cube_loss_wf_kernel<T, IO, kWfUnr, false, PTS>, kWfWarps * 32, smem,
+                                   (B + kWfWarps * kWfMinPerWarp - 1) / (kWfWarps * kWfMinPerWarp), kMaxBlocks,
+                                   &blocks, &cap))
+    return rc;
+  unsigned long long* dyn = nullptr;
+  if (dynamic) {
+    if (!cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
+    if (int rc = cn::dynamic_counter(workspace, st, &dyn)) return rc;
+  }
+  // Up to ~320 samples per warp (crossover measured around 400) the launch is a few long Newton chains per warp: the
+  // instance with the per-contact loop of the Newton visit unrolled overlaps the four contacts (measured -8% at
+  // 65,536 pairs, -5% at 262,144).  Larger batches keep every warp's pool full and run the rolled instance,
+  // which is smaller in the instruction cache (the unrolled one is +5% at 1M pairs, +15% at 4M).
+  const bool small = B <= cap * kWfWarps * 320;
+  if constexpr (!PTS) {
+    // DPLL_LOSS_RACE: the head of a cost-ordered batch goes to racing blocks at the front of the same grid, the
+    // wavefront blocks take the rest.  Only for launches bounded by their longest chain (small shards), and only for
+    // cold solves.
+    if ((flags & DPLL_LOSS_RACE) && dynamic && small && !u_init && B >= 4096 && B <= kRaceMaxBatch) {
+      int64_t head = B / 64;
+      if (head > kRaceMaxHead) head = kRaceMaxHead;
+      head -= head % (kWfWarps * kRaceSamples);
+      const int race_blocks = (int)(head / (kWfWarps * kRaceSamples));
+      // an SM holds two blocks: leave the racing blocks their share of the resident set
+      if (blocks > cap - race_blocks) blocks = (int)(cap - race_blocks > 1 ? cap - race_blocks : 1);
+      if (race_blocks > 0) {
+        cube_loss_wf_kernel<T, IO, 4, true><<<race_blocks + blocks, kWfWarps * 32, smem, st>>>(
+            x, xp, weight, inertia, mu, half, dt, eps, B, loss, force, iters, partials, want_grad, skip_flag, dyn, ldx,
+            ldxp, u_init, u_out, race_blocks, head);
+        *rows = race_blocks + blocks;
+        return cn::launch_status();
+      }
+    }
+  }
+  auto kernel = small ? cube_loss_wf_kernel<T, IO, 4, false, PTS> : cube_loss_wf_kernel<T, IO, kWfUnr, false, PTS>;
+  kernel<<<blocks, kWfWarps * 32, smem, st>>>(x, xp, weight, inertia, mu, half, dt, eps, B, loss, force, iters, partials,
+                                              want_grad, skip_flag, dyn, ldx, ldxp, u_init, u_out, 0, 0);
+  *rows = blocks;
+  return cn::launch_status();
+}
 
 template <typename T, typename IO>
 int launch_cube_loss(int variant, const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu,
@@ -891,89 +851,38 @@ int launch_cube_loss(int variant, const IO* x, const IO* xp, const IO* weight, c
   if (B < 0 || (leaf ? (!friction || !length) : (!inertia || !mu || !half))) return DPLL_EINVAL;
   if (B > 0 && (!x || !xp)) return DPLL_EINVAL;
   const bool want_red = grad || loss_sum || comm || sums || means;
-  if ((want_red || leaf) && (!workspace || workspace_bytes < dpll_workspace_bytes())) return DPLL_EWORKSPACE;
+  if ((want_red || leaf) && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const DeviceInfo di = device_info();
   T* partials = want_red ? static_cast<T*>(workspace) : nullptr;
   if (leaf) {
     // callable-level parameters are produced on the device, behind the partials in the workspace
-    IO* params = reinterpret_cast<IO*>(static_cast<T*>(workspace) + (size_t)kMaxBlocks * 32);
+    IO* params = reinterpret_cast<IO*>(static_cast<char*>(workspace) + cn::kWsParamsOffset);
     cube_prep_kernel<T, IO><<<1, 32, 0, st>>>(theta, friction, length, params, skip_flag);
     inertia = params; mu = params + 10; half = params + 11;
   }
-  int blocks, race_rows = 0;
+  const int want_grad = (grad || sums || means) ? 1 : 0;
+  int rows;
   if (variant == 0 || variant == 2) {
-    // wavefront kernel: persistent, one resident set of blocks
-    const size_t smem = sizeof(WfWarpPool<T>) * kWfWarps;
-    cudaError_t ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, kWfUnr>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (ea == cudaSuccess)
-      ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (ea == cudaSuccess)
-      ea = cudaFuncSetAttribute(cube_loss_wf_kernel<T, IO, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (ea != cudaSuccess) return (int)ea;
-    int64_t cap;
-    blocks = wf_blocks(B, cube_loss_wf_kernel<T, IO, kWfUnr>, smem, di.sms, &cap);
-    unsigned long long* dyn = nullptr;
-    if (variant == 2) {
-      if (!workspace || workspace_bytes < dpll_workspace_bytes()) return DPLL_EWORKSPACE;
-      dyn = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + kWsQueueOffset);
-      cudaError_t em = cudaMemsetAsync(dyn, 0, kWsQueueBytes, st);
-      if (em != cudaSuccess) return (int)em;
-    }
-    // Up to ~320 samples per warp (crossover measured around 400) the launch is a few long Newton chains per warp: the
-    // instance with the per-contact loop of the Newton visit unrolled overlaps the four contacts (measured -8% at
-    // 65,536 pairs, -5% at 262,144).  Larger batches keep every warp's pool full and run the rolled instance,
-    // which is smaller in the instruction cache (the unrolled one is +5% at 1M pairs, +15% at 4M).
-    // DPLL_LOSS_RACE: the head of a cost-ordered batch goes to racing blocks at the front of the same grid, the wavefront
-    // blocks take the rest.  Only for launches bounded by their longest chain (small shards), and only for cold solves.
-    int64_t head = 0;
-    int race_blocks = 0;
-    const bool small = B <= cap * kWfWarps * 320;
-    if ((flags & DPLL_LOSS_RACE) && variant == 2 && small && !u_init && B >= 4096 && B <= kRaceMaxBatch) {
-      head = B / 64;
-      if (head > kRaceMaxHead) head = kRaceMaxHead;
-      head -= head % (kWfWarps * kRaceSamples);
-      race_blocks = (int)(head / (kWfWarps * kRaceSamples));
-      // an SM holds two blocks: leave the racing blocks their share of the resident set
-      if (blocks > cap - race_blocks) blocks = (int)(cap - race_blocks > 1 ? cap - race_blocks : 1);
-    }
-    if (race_blocks > 0)
-      cube_loss_wf_kernel<T, IO, 4, true><<<race_blocks + blocks, kWfWarps * 32, smem, st>>>(
-          x, xp, weight, inertia, mu, half, dt, eps, B, loss, force, iters, partials, (grad || sums || means) ? 1 : 0,
-          skip_flag, dyn, ldx, ldxp, u_init, u_out, race_blocks, head);
-    else if (small)
-      cube_loss_wf_kernel<T, IO, 4><<<blocks, kWfWarps * 32, smem, st>>>(
-          x, xp, weight, inertia, mu, half, dt, eps, B, loss, force, iters, partials, (grad || sums || means) ? 1 : 0,
-          skip_flag, dyn, ldx, ldxp, u_init, u_out, 0, 0);
-    else
-      cube_loss_wf_kernel<T, IO, kWfUnr><<<blocks, kWfWarps * 32, smem, st>>>(
-          x, xp, weight, inertia, mu, half, dt, eps, B, loss, force, iters, partials, (grad || sums || means) ? 1 : 0,
-          skip_flag, dyn, ldx, ldxp, u_init, u_out, 0, 0);
-    race_rows = race_blocks;
+    if (int rc = launch_cube_wf<T, IO, false>(variant == 2, flags, x, xp, weight, inertia, mu, half, dt, eps, B, loss,
+                                              force, iters, partials, want_grad, skip_flag, workspace, workspace_bytes,
+                                              st, ldx, ldxp, u_init, u_out, &rows))
+      return rc;
   } else {
-    int per_sm = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cube_loss_kernel<T, IO>, kLossThreads, 0);
-    if (per_sm < 1) per_sm = 1;
-    int64_t need = (B + kLossThreads - 1) / kLossThreads;
-    int64_t cap = (int64_t)di.sms * per_sm;
-    if (cap > kMaxBlocks) cap = kMaxBlocks;
-    blocks = (int)(need < cap ? need : cap);
-    if (blocks < 1) blocks = 1;
-    cube_loss_kernel<T, IO><<<blocks, kLossThreads, 0, st>>>(x, xp, weight, inertia, mu, half, dt, eps, B, loss, force,
-                                                         iters, partials, (grad || sums || means) ? 1 : 0, skip_flag, ldx, ldxp);
+    int64_t cap;
+    if (int rc = cn::resident_blocks(cube_loss_kernel<T, IO>, kLossThreads, 0, (B + kLossThreads - 1) / kLossThreads,
+                                     kMaxBlocks, &rows, &cap))
+      return rc;
+    cube_loss_kernel<T, IO><<<rows, kLossThreads, 0, st>>>(x, xp, weight, inertia, mu, half, dt, eps, B, loss, force,
+                                                           iters, partials, want_grad, skip_flag, ldx, ldxp);
+    if (int rc = cn::launch_status()) return rc;
   }
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return (int)e;
-  if (want_red) {
-    if (leaf) reduce_partials_leaf_kernel<T, IO><<<1, 32 * kNAcc, 0, st>>>(partials, blocks + race_rows, theta, friction, length, grad,
-                                                                     loss_sum, skip_flag, comm, (double)B, sums, means,
-                                                                     local_out);
-    else reduce_partials_kernel<T, IO, kNAcc, DPLL_CUBE_NPARAM><<<1, 32 * kNAcc, 0, st>>>(partials, blocks + race_rows, grad, loss_sum,
-                                                                                        skip_flag);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-  }
-  return DPLL_OK;
+  if (!want_red) return DPLL_OK;
+  if (leaf) reduce_partials_leaf_kernel<T, IO><<<1, 32 * kNAcc, 0, st>>>(partials, rows, theta, friction, length, grad,
+                                                                        loss_sum, skip_flag, comm, (double)B, sums, means,
+                                                                        local_out);
+  else reduce_partials_kernel<T, IO, kNAcc, DPLL_CUBE_NPARAM><<<1, 32 * kNAcc, 0, st>>>(partials, rows, grad, loss_sum,
+                                                                                       skip_flag);
+  return cn::launch_status();
 }
 
 template <typename T, typename IO>
@@ -982,21 +891,25 @@ int launch_cube_rollout(const IO* x0, const IO* inertia, const IO* mu, const IO*
   if (B < 0 || steps < 0 || !inertia || !mu || !half) return DPLL_EINVAL;
   if (B > 0 && (!x0 || !traj)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const DeviceInfo di = device_info();
-  int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cube_rollout_kernel<T, IO>, kLossThreads, 0);
-  if (per_sm < 1) per_sm = 1;
-  const int64_t cap = (int64_t)di.sms * per_sm;                      // resident blocks
-  const int64_t warps = cap * (kLossThreads / 32);
-  const int lpw = rollout_tosses_per_warp(B, di.sms, warps);
-  const int64_t per_block = (int64_t)lpw * (kLossThreads / 32);
-  const int64_t need = (B + per_block - 1) / per_block;
-  const int blocks = (int)(need < cap ? need : cap);
-  cube_rollout_kernel<T, IO><<<blocks, kLossThreads, 0, st>>>(x0, inertia, mu, half, dt, eps, B, steps, traj, force,
-                                                          iters, lpw, usol);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  int blocks, lpw;
+  if (int rc = rollout_grid(cube_rollout_kernel<T, IO>, B, &blocks, &lpw)) return rc;
+  cube_rollout_kernel<T, IO><<<blocks, kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      x0, inertia, mu, half, dt, eps, B, steps, traj, force, iters, lpw, usol);
+  return cn::launch_status();
+}
+
+template <typename T, typename IO>
+int launch_elbow_rollout(const IO* x0, const IO* inertia, const IO* mu, const IO* half, const IO* kin, const IO* pts,
+                         T dt, T eps, int64_t B, int32_t steps, IO* traj, IO* force, int32_t* iters, void* stream,
+                         IO* usol = nullptr) {
+  if (B < 0 || steps < 0 || !inertia || !mu || (!half && !pts) || !kin || (pts && steps > 1)) return DPLL_EINVAL;
+  if (B > 0 && (!x0 || !traj)) return DPLL_EINVAL;
+  if (B == 0) return DPLL_OK;
+  int blocks, lpw;
+  if (int rc = rollout_grid(elbow_rollout_kernel<T, IO>, B, &blocks, &lpw)) return rc;
+  elbow_rollout_kernel<T, IO><<<blocks, kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      x0, inertia, mu, half, kin, pts, dt, eps, B, steps, traj, force, iters, lpw, usol);
+  return cn::launch_status();
 }
 
 }  // namespace
@@ -1015,7 +928,7 @@ int dpll_set_loss_variant(int variant) {
 
 int dpll_version(void) { return DPLL_VERSION; }
 
-size_t dpll_workspace_bytes(void) { return kWsQueueOffset + kWsQueueBytes; }
+size_t dpll_workspace_bytes(void) { return cn::kWsBytes; }
 
 int dpll_cube_loss_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
                        const double* mu_pair, const double* half, double dt, double eps, int64_t B, double* loss,
@@ -1111,40 +1024,20 @@ int dpll_body_loss_pts_f64(const double* x, const double* x_plus, const double* 
   if (B > 0 && (!x || !x_plus || !pts)) return DPLL_EINVAL;
   const bool want_red = grad || loss_sum;
   const bool dynamic = (flags & DPLL_LOSS_DYNAMIC) != 0;
-  if ((want_red || dynamic) && (!workspace || workspace_bytes < dpll_workspace_bytes())) return DPLL_EWORKSPACE;
+  if ((want_red || dynamic) && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const DeviceInfo di = device_info();
-  // the box's wavefront kernel, witness-point instance; the same grid and the same choice of instance by batch size
-  const size_t smem = sizeof(WfWarpPool<double>) * kWfWarps;
-  cudaError_t ea = cudaFuncSetAttribute(cube_loss_wf_kernel<double, double, kWfUnr, false, true>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (ea == cudaSuccess)
-    ea = cudaFuncSetAttribute(cube_loss_wf_kernel<double, double, 4, false, true>,
-                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (ea != cudaSuccess) return (int)ea;
-  int64_t cap;
-  const int blocks = wf_blocks(B, cube_loss_wf_kernel<double, double, kWfUnr, false, true>, smem, di.sms, &cap);
-  unsigned long long* dyn = nullptr;
-  if (dynamic) {
-    dyn = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + kWsQueueOffset);
-    cudaError_t em = cudaMemsetAsync(dyn, 0, kWsQueueBytes, st);
-    if (em != cudaSuccess) return (int)em;
-  }
   double* partials = want_red ? static_cast<double*>(workspace) : nullptr;
-  auto kernel = B <= cap * kWfWarps * 320 ? cube_loss_wf_kernel<double, double, 4, false, true>
-                                          : cube_loss_wf_kernel<double, double, kWfUnr, false, true>;
-  // (the points travel in `half`, grad_pts in `u_out`, n_contacts in the upper bits of `want_grad`: see the kernel)
-  kernel<<<blocks, kWfWarps * 32, smem, st>>>(x, x_plus, weight, inertia, mu_pair, pts, dt, eps, B, loss, force, iters,
-                                              partials, (grad ? 1 : 0) | (n_contacts << 1), skip_flag, dyn, 13, 13, nullptr,
-                                              grad_pts, 0, 0);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return (int)e;
-  if (want_red) {
-    reduce_partials_kernel<double, double, kNAcc, 11><<<1, 32 * kNAcc, 0, st>>>(partials, blocks, grad, loss_sum, skip_flag);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-  }
-  return DPLL_OK;
+  // the box's wavefront launch, witness-point instance: the points travel in `half`, grad_pts in `u_out`, n_contacts
+  // in the upper bits of `want_grad` (see the kernel)
+  int rows;
+  if (int rc = launch_cube_wf<double, double, true>(dynamic, flags, x, x_plus, weight, inertia, mu_pair, pts, dt, eps, B,
+                                                    loss, force, iters, partials, (grad ? 1 : 0) | (n_contacts << 1),
+                                                    skip_flag, workspace, workspace_bytes, st, 13, 13, nullptr, grad_pts,
+                                                    &rows))
+    return rc;
+  if (!want_red) return DPLL_OK;
+  reduce_partials_kernel<double, double, kNAcc, 11><<<1, 32 * kNAcc, 0, st>>>(partials, rows, grad, loss_sum, skip_flag);
+  return cn::launch_status();
 }
 
 int dpll_body_step_pts_f64(const double* x, const double* inertia, const double* mu_pair, const double* pts,
@@ -1153,11 +1046,9 @@ int dpll_body_step_pts_f64(const double* x, const double* inertia, const double*
   if (B < 0 || !inertia || !mu_pair || n_contacts < 1 || n_contacts > DPLL_CUBE_NC) return DPLL_EINVAL;
   if (B > 0 && (!x || !pts || !x_next)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int blocks = (int)((B + kLossThreads - 1) / kLossThreads);
-  body_pts_step_kernel<double, double><<<blocks, kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  body_pts_step_kernel<double, double><<<cn::grid_for(B, kLossThreads), kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x, inertia, mu_pair, pts, n_contacts, dt, eps, B, x_next, force);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_cube_terms_f64(const double* q, const double* v, const double* inertia, const double* mu_pair,
@@ -1166,11 +1057,9 @@ int dpll_cube_terms_f64(const double* q, const double* v, const double* inertia,
   if (B < 0 || !inertia || !mu_pair || !half) return DPLL_EINVAL;
   if (B > 0 && (!q || !v || !M || !J || !phi || !acc)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int blocks = (int)((B + kLossThreads - 1) / kLossThreads);
-  cube_terms_kernel<double, double><<<blocks, kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+  cube_terms_kernel<double, double><<<cn::grid_for(B, kLossThreads), kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       q, v, inertia, mu_pair, half, B, M, J, phi, acc, delassus);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_elbow_terms_f64(const double* q, const double* v, const double* inertia, const double* mu_pair,
@@ -1179,31 +1068,9 @@ int dpll_elbow_terms_f64(const double* q, const double* v, const double* inertia
   if (B < 0 || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
   if (B > 0 && (!q || !v || !M || !J || !phi || !acc)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int blocks = (int)((B + 63) / 64);
-  elbow_terms_kernel<double, double><<<blocks, 64, 0, static_cast<cudaStream_t>(stream)>>>(
+  elbow_terms_kernel<double, double><<<cn::grid_for(B, 64), 64, 0, static_cast<cudaStream_t>(stream)>>>(
       q, v, inertia, mu_pair, half, kin, B, M, J, phi, acc, delassus);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
-}
-
-int dpll_elbow_loss_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
-                        const double* mu_pair, const double* half, const double* kin, const double* pts, double dt,
-                        double eps, int64_t B, int32_t flags, double* loss, double* force, double* grad_pts,
-                        int32_t* iters, double* grad, double* loss_sum, const int32_t* skip_flag, void* workspace,
-                        size_t workspace_bytes, void* stream) {
-  return launch_elbow_loss<double, double>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, loss, force,
-                                           grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream,
-                                           flags);
-}
-
-int dpll_elbow_loss_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
-                        const float* mu_pair, const float* half, const float* kin, const float* pts, float dt, float eps,
-                        int64_t B, int32_t flags, float* loss, float* force, float* grad_pts, int32_t* iters, float* grad,
-                        float* loss_sum, const int32_t* skip_flag, void* workspace, size_t workspace_bytes,
-                        void* stream) {
-  return launch_elbow_loss<double, float>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, (double)dt, (double)eps, B,
-                                          loss, force, grad_pts, iters, grad, loss_sum, skip_flag, workspace,
-                                          workspace_bytes, stream, flags);
+  return cn::launch_status();
 }
 
 int dpll_elbow_rollout_f64(const double* x0, const double* inertia, const double* mu_pair, const double* half,
@@ -1231,15 +1098,13 @@ int dpll_elbow_rollout_f32(const float* x0, const float* inertia, const float* m
 int dpll_fma_peak_f64(double* out, int32_t blocks, int64_t iters, void* stream) {
   if (!out || blocks <= 0 || iters < 0) return DPLL_EINVAL;
   fma_peak_kernel<double><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(out, iters);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_fma_peak_f32(float* out, int32_t blocks, int64_t iters, void* stream) {
   if (!out || blocks <= 0 || iters < 0) return DPLL_EINVAL;
   fma_peak_kernel<float><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(out, iters);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

@@ -10,6 +10,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_params.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -75,8 +76,7 @@ int dpll_leaf_prepare_f64(const double* theta, int32_t n_bodies, const double* f
     return DPLL_EINVAL;
   leaf_prepare_kernel<<<1, 64, 0, static_cast<cudaStream_t>(stream)>>>(theta, n_bodies, friction, pair_a, pair_b, n_pairs,
                                                                      length, n_len, inertia, mu, half);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_leaf_backward_f64(const double* theta, int32_t n_bodies, const double* friction, int32_t n_geoms,
@@ -90,8 +90,7 @@ int dpll_leaf_backward_f64(const double* theta, int32_t n_bodies, const double* 
   leaf_backward_kernel<<<1, 64, 0, static_cast<cudaStream_t>(stream)>>>(theta, n_bodies, friction, n_geoms, pair_a, pair_b,
                                                                       n_pairs, length, n_len, g_inertia, g_mu, g_half,
                                                                       g_theta, g_friction, g_length);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"

@@ -5,6 +5,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_cube_tangent.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -35,12 +36,9 @@ int launch_cube_rollout_grad(const T* x0, const T* inertia, const T* mu, const T
   if (B < 0 || steps < 0 || !inertia || !mu || !half) return DPLL_EINVAL;
   if (B > 0 && (!x0 || !xbar || !gparams || !gx0)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int64_t threads = B * cn::CUBE_NTAN;
-  const int blocks = (int)((threads + 127) / 128);
-  cube_rollout_grad_kernel<T><<<blocks, 128, 0, static_cast<cudaStream_t>(stream)>>>(x0, inertia, mu, half, dt, eps, B, steps,
+  cube_rollout_grad_kernel<T><<<cn::grid_for(B * cn::CUBE_NTAN, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(x0, inertia, mu, half, dt, eps, B, steps,
                                                                                   xbar, gparams, gx0);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 // backward of one witness-point step: one (sample, direction) pair per thread; gparams (B, 11), gpts (B, 12), gx (B, 13)
@@ -74,12 +72,9 @@ int dpll_body_step_pts_grad_f64(const double* x, const double* inertia, const do
   if (B < 0 || !inertia || !mu_pair || n_contacts < 0 || n_contacts > 4) return DPLL_EINVAL;
   if (B > 0 && (!x || !pts || !xbar || !gparams || !gpts || !gx)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int64_t threads = B * cn::BODY_PTS_NTAN;
-  const int blocks = (int)((threads + 127) / 128);
-  body_step_pts_grad_kernel<double><<<blocks, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+  body_step_pts_grad_kernel<double><<<cn::grid_for(B * cn::BODY_PTS_NTAN, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
       x, inertia, mu_pair, pts, n_contacts, dt, eps, B, xbar, gparams, gpts, gx);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 int dpll_cube_rollout_grad_f64(const double* x0, const double* inertia, const double* mu_pair, const double* half,

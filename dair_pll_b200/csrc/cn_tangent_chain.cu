@@ -3,6 +3,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_chain_tangent.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -23,17 +24,6 @@ chain_rollout_grad_kernel(const T* __restrict__ x0, const T* __restrict__ inerti
   else gx0[b * NX + (dir - NP)] = g;
 }
 
-template <int N>
-int launch(const double* x0, const double* inertia, const double* mu, const double* half, const double* kin, double dt,
-           double eps, int64_t B, int steps, const double* xbar, double* gparams, double* gx0, cudaStream_t st) {
-  constexpr int NTAN = 14 * N + 13 + 2 * (N - 1);
-  const int64_t threads = B * NTAN;
-  const int blocks = (int)((threads + 63) / 64);
-  chain_rollout_grad_kernel<double, N><<<blocks, 64, 0, st>>>(x0, inertia, mu, half, kin, dt, eps, B, steps, xbar, gparams, gx0);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
-}
-
 }  // namespace
 
 extern "C" {
@@ -44,15 +34,12 @@ int dpll_chain_rollout_grad_f64(int32_t n_links, const double* x0, const double*
   if (B < 0 || steps < 0 || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
   if (B > 0 && (!x0 || !xbar || !gparams || !gx0)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  switch (n_links) {
-    case 2: return launch<2>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0, st);
-    case 3: return launch<3>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0, st);
-    case 4: return launch<4>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0, st);
-    case 5: return launch<5>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0, st);
-    case 6: return launch<6>(x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0, st);
-    default: return DPLL_EINVAL;
-  }
+  return cn::with_links(n_links, [&](auto N) {
+    constexpr int NTAN = 14 * N + 13 + 2 * (N - 1);       // (toss, direction) pairs per toss
+    chain_rollout_grad_kernel<double, N><<<cn::grid_for(B * NTAN, 64), 64, 0, static_cast<cudaStream_t>(stream)>>>(
+        x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0);
+    return cn::launch_status();
+  });
 }
 
 }  // extern "C"

@@ -3,6 +3,7 @@
 
 #include "../../include/dair_pll_b200.h"
 #include "cn_elbow_tangent.cuh"
+#include "cn_launch.cuh"
 
 namespace {
 
@@ -61,12 +62,9 @@ int dpll_elbow_step_pts_grad_f64(const double* x, const double* inertia, const d
   if (B < 0 || !inertia || !mu_pair || !kin) return DPLL_EINVAL;
   if (B > 0 && (!x || !pts || !xbar || !gparams || !gpts || !gx)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int64_t threads = B * cn::ELBOW_PTS_NTAN;
-  const int blocks = (int)((threads + 127) / 128);
-  elbow_step_pts_grad_kernel<double><<<blocks, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+  elbow_step_pts_grad_kernel<double><<<cn::grid_for(B * cn::ELBOW_PTS_NTAN, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
       x, inertia, mu_pair, kin, pts, dt, eps, B, xbar, gparams, gpts, gx, usol);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 
@@ -76,12 +74,9 @@ int dpll_elbow_rollout_grad_saved_f64(const double* x0, const double* inertia, c
   if (B < 0 || steps < 0 || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
   if (B > 0 && (!x0 || !xbar || !gparams || !gx0)) return DPLL_EINVAL;
   if (B == 0) return DPLL_OK;
-  const int64_t threads = B * cn::ELBOW_NTAN;
-  const int blocks = (int)((threads + 127) / 128);
-  elbow_rollout_grad_kernel<double><<<blocks, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+  elbow_rollout_grad_kernel<double><<<cn::grid_for(B * cn::ELBOW_NTAN, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
       x0, inertia, mu_pair, half, kin, dt, eps, B, steps, xbar, gparams, gx0, usol);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? DPLL_OK : (int)e;
+  return cn::launch_status();
 }
 
 }  // extern "C"
