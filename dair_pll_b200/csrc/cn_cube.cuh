@@ -210,10 +210,10 @@ template <typename T>
 CN_HD void cube_contact_residual(const CubeParams<T>& P, const CubeProb<T>& S, int c, const T* u, T* rho, T* r) {
   rho[0] = S.rho(3 * c); rho[1] = S.rho(3 * c + 1); rho[2] = S.rho(3 * c + 2);
   T e[3];
-  cross3(u, rho, e);
-  r[0] = P.mu * (e[0] + u[3]) + S.q(3 * c);
-  r[1] = P.mu * (e[1] + u[4]) + S.q(3 * c + 1);
-  r[2] = (e[2] + u[5]) + S.q(3 * c + 2);
+  cross3_add(u, rho, u + 3, e);
+  r[0] = P.mu * e[0] + S.q(3 * c);
+  r[1] = P.mu * e[1] + S.q(3 * c + 1);
+  r[2] = e[2] + S.q(3 * c + 2);
 }
 
 // Gradient (and optionally Hessian) of the primal objective at u (world twist).
@@ -240,10 +240,9 @@ CN_HD void cube_eval(const CubeParams<T>& P, const CubeProb<T>& S, const T* u, T
     cube_contact_residual(P, S, c, u, rho, r);
     cone_eval<T, WANT_H>(r, P.inv_eps, P.mu, f, K);
     const T ft[3] = {P.mu * f[0], P.mu * f[1], f[2]};
-    T tq[3];
-    cross3(rho, ft, tq);
+    cross3_add(rho, ft, z, z);
 #pragma unroll
-    for (int i = 0; i < 3; ++i) { z[i] += tq[i]; z[3 + i] += ft[i]; }
+    for (int i = 0; i < 3; ++i) z[3 + i] += ft[i];
     if (WANT_H) {
       const T K0[3] = {K[0], K[1], K[2]}, K1[3] = {K[1], K[3], K[4]}, K2[3] = {K[2], K[4], K[5]};
       // Pm = S(rho) K : column j = rho x K_j  (K symmetric)
@@ -252,11 +251,15 @@ CN_HD void cube_eval(const CubeParams<T>& P, const CubeProb<T>& S, const T* u, T
       // H_vw (rows 3+j, cols i) += Pm^T
 #pragma unroll
       for (int i = 0; i < 3; ++i) { H[18 + i] += P0[i]; H[24 + i] += P1[i]; H[30 + i] += P2[i]; }
-      // H_ww += -Pm S(rho): row i = rho x (row i of Pm)
-      const T r0[3] = {P0[0], P1[0], P2[0]}, r1[3] = {P0[1], P1[1], P2[1]}, r2[3] = {P0[2], P1[2], P2[2]};
-      T w0[3], w1[3], w2[3];
-      cross3(rho, r0, w0); cross3(rho, r1, w1); cross3(rho, r2, w2);
-      H[0] += w0[0]; H[6] += w1[0]; H[7] += w1[1]; H[12] += w2[0]; H[13] += w2[1]; H[14] += w2[2];
+      // H_ww += -Pm S(rho) = S(rho) K S(rho)^T: row i = rho x (row i of Pm); only the lower triangle, each entry one
+      // FMA chain ending on H
+      const T a = rho[0], b = rho[1], cz = rho[2];
+      H[0] = H[0] + b * P2[0] - cz * P1[0];
+      H[6] = H[6] + b * P2[1] - cz * P1[1];
+      H[7] = H[7] + cz * P0[1] - a * P2[1];
+      H[12] = H[12] + b * P2[2] - cz * P1[2];
+      H[13] = H[13] + cz * P0[2] - a * P2[2];
+      H[14] = H[14] + a * P1[2] - b * P0[2];
       // H_vv += K
       H[21] += K[0]; H[27] += K[1]; H[28] += K[3]; H[33] += K[2]; H[34] += K[4]; H[35] += K[5];
     }
@@ -437,36 +440,37 @@ CN_HD void cube_loss_prologue(const CubeParams<T>& P, const T* x, const T* xp, c
   rot3(A.R, A.dv, dvW); rot3(A.R, A.vp, vW);
 #pragma unroll
   for (int i = 0; i < 3; ++i) { dvW[3 + i] = A.dv[3 + i]; vW[3 + i] = A.vp[3 + i]; }
-  T pen = T(0), a_min = T(2);
+  T pen4 = T(0), a_min = T(2);
 #pragma unroll UNR
   for (int c = 0; c < CUBE_NC; ++c) {
     const T rho[3] = {S.rho(3 * c), S.rho(3 * c + 1), S.rho(3 * c + 2)};
     T ed[3], ev[3];
-    cross3(dvW, rho, ed); cross3(vW, rho, ev);
-#pragma unroll
-    for (int i = 0; i < 3; ++i) { ed[i] += dvW[3 + i]; ev[i] += vW[3 + i]; }
+    cross3_add(dvW, rho, dvW + 3, ed); cross3_add(vW, rho, vW + 3, ev);
     const T sx = P.mu * ev[0], sy = P.mu * ev[1];
     const T speed2 = sx * sx + sy * sy;
-    const T speed = speed2 * t_rsqrt(t_max(speed2, t_tiny<T>()));
+    const T speed = speed2 * t_rsqrt0(speed2);
     const T phic = rho[2] + A.pos_z;
     const T s0 = P.dt * sx, s1 = P.dt * sy, s2 = t_abs(phic) + P.dt * speed;
     const T e0 = -P.mu * ed[0], e1 = -P.mu * ed[1], e2 = -ed[2];
     S.q(3 * c) = e0 + s0;                                          // :158-161
     S.q(3 * c + 1) = e1 + s1;
     S.q(3 * c + 2) = e2 + s2;
-    const T pneg = t_max(-phic, T(0));
-    pen += pneg * pneg;
+    const T pneg2 = t_abs(phic) - phic;                            // 2 max(-phi_c, 0), exactly
+    pen4 += pneg2 * pneg2;
     if (CN_LOSS_START_FACTOR > 0) {
-      // |s_t + a e_t|^2 = (s_n + a e_n)^2: smallest positive root, in the cancellation-free form -2 C / (B + sqrt(disc))
-      const T Aq = e0 * e0 + e1 * e1 - e2 * e2, Bq = T(2) * (s0 * e0 + s1 * e1 - s2 * e2);
-      const T Cq = t_min(s0 * s0 + s1 * s1 - s2 * s2, T(0));
-      const T disc = Bq * Bq - T(4) * Aq * Cq;
-      const T dpos = t_max(disc, T(0));
-      const T den = Bq + dpos * t_rsqrt(t_max(dpos, t_tiny<T>()));
-      const T a_c = (disc >= T(0) && den > T(0)) ? T(-2) * Cq * t_rcp(den) : T(2);
-      a_min = t_min(a_min, a_c);
+      // |s_t + a e_t|^2 = (s_n + a e_n)^2, i.e. Aq a^2 + 2 Bh a + Cq = 0: smallest positive root, in the cancellation-free
+      // form -Cq / (Bh + sqrt(disc)).  Cq = min(cs, 0) = (cs - |cs|) / 2, exactly.  disc < 0 (no root) makes den NaN, so
+      // den > 0 alone selects the samples with a root.
+      const T Aq = e0 * e0 + e1 * e1 - e2 * e2, Bh = s0 * e0 + s1 * e1 - s2 * e2;
+      const T cs = s0 * s0 + s1 * s1 - s2 * s2;
+      const T Cq = T(0.5) * (cs - t_abs(cs));
+      const T disc = Bh * Bh - Aq * Cq;
+      const T den = Bh + disc * t_rsqrt0(disc);
+      const T a_c = den > T(0) ? -Cq * t_rcp(den) : T(2);
+      a_min = a_c < a_min ? a_c : a_min;
     }
   }
+  const T pen = T(0.25) * pen4;
   A.a_min = a_min;
 #pragma unroll
   for (int i = 0; i < 6; ++i) A.dvW[i] = dvW[i];
@@ -551,21 +555,20 @@ CN_HD T cube_loss_epilogue(const CubeParams<T>& P, const CubeProb<T>& S, const C
   const T* R = A.R;
   // pass 1: forces f_c = Pi(-(D_mu J_c u + q_c)/eps), z = J^T f (world twist), q.f, f.f, validity
   T zW[6] = {T(0), T(0), T(0), T(0), T(0), T(0)};
-  T qf = T(0), ff = T(0), fmax = T(0);
+  T qf = T(0), ff = T(0);
+  bool fok = true;                         // every |f_i| <= 1e3 (false for NaN)
 #pragma unroll UNR
   for (int c = 0; c < CUBE_NC; ++c) {
     T rho[3], r[3], f[3];
     cube_contact_residual(P, S, c, u, rho, r);
     cone_eval<T, false>(r, P.inv_eps, P.mu, f, (T*)nullptr);
     const T ft[3] = {P.mu * f[0], P.mu * f[1], f[2]};
-    T tq[3];
-    cross3(rho, ft, tq);
+    cross3_add(rho, ft, zW, zW);
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
-      zW[i] += tq[i]; zW[3 + i] += ft[i];
+      zW[3 + i] += ft[i];
       qf += S.q(3 * c + i) * f[i]; ff += f[i] * f[i];
-      const T af = t_abs(f[i]);
-      fmax = (af > fmax || af != af) ? af : fmax;     // NaN-propagating max
+      fok = fok && t_abs(f[i]) <= T(1e3);
     }
     if (PARK) {
 #pragma unroll
@@ -573,7 +576,7 @@ CN_HD T cube_loss_epilogue(const CubeParams<T>& P, const CubeProb<T>& S, const C
     }
     if (force_out) { force_out[c] = f[2]; force_out[4 + 2 * c] = f[0]; force_out[4 + 2 * c + 1] = f[1]; }
   }
-  if (!(fmax <= T(1e3))) {                 // |f| > 1e3, NaN or Inf: force := 0, constant := 0 (:186-192)
+  if (!fok) {                              // |f| > 1e3, NaN or Inf: force := 0, constant := 0 (:186-192)
     if (force_out) for (int i = 0; i < 12; ++i) force_out[i] = T(0);
     return T(0);
   }
@@ -620,26 +623,26 @@ CN_HD T cube_loss_epilogue(const CubeParams<T>& P, const CubeProb<T>& S, const C
       cone_eval<T, false>(r, P.inv_eps, P.mu, f, (T*)nullptr);
     }
     T eb[3], ev[3];
-    cross3(bW, rho, eb); cross3(wW, rho, ev);
-#pragma unroll
-    for (int i = 0; i < 3; ++i) { eb[i] += b[3 + i]; ev[i] += A.vp[3 + i]; }
+    cross3_add(bW, rho, b + 3, eb); cross3_add(wW, rho, A.vp + 3, ev);
     const T ftx = f[0], fty = f[1], fn = f[2];
     const T sx = P.mu * ev[0], sy = P.mu * ev[1];
-    const T speed2 = sx * sx + sy * sy;
-    const T sinv = t_rsqrt(t_max(speed2, t_tiny<T>()));            // speed 0: sx = sy = 0, so ux = uy = 0
+    const T sinv = t_rsqrt0(sx * sx + sy * sy);                     // speed 0: sx = sy = 0, so ux = uy = 0
     const T ux = sx * sinv, uy = sy * sinv;
     const T gx = P.dt * (fn * ux + ftx), gy = P.dt * (fn * uy + fty);
-    gmu += ftx * eb[0] + fty * eb[1] + gx * ev[0] + gy * ev[1];
+    gmu = gmu + ftx * eb[0] + fty * eb[1] + gx * ev[0] + gy * ev[1];
+    const T phic = rho[2] + A.pos_z;
+    const T phibar = (phic > T(0) ? fn : (phic < T(0) ? -fn : T(0))) - (t_abs(phic) - phic);
+    // (R^T ft) x b + (R^T gt) x w + phibar R^T e_z = R^T (ft x bW + gt x wW + phibar e_z)
     const T ft[3] = {P.mu * ftx, P.mu * fty, fn};
     const T gt[3] = {P.mu * gx, P.mu * gy, T(0)};
-    T ftB[3], gtB[3], p1[3], p2[3];
-    rot3t(R, ft, ftB); rot3t(R, gt, gtB);
-    cross3(ftB, b, p1); cross3(gtB, w, p2);
-    const T phic = rho[2] + A.pos_z;
-    const T phibar = (phic > T(0) ? fn : (phic < T(0) ? -fn : T(0))) - T(2) * t_max(-phic, T(0));
-    gh0 += sgn_bit<T>(A.sel, cidx, 0) * (p1[0] + p2[0] + phibar * R[6]);
-    gh1 += sgn_bit<T>(A.sel, cidx, 1) * (p1[1] + p2[1] + phibar * R[7]);
-    gh2 += sgn_bit<T>(A.sel, cidx, 2) * (p1[2] + p2[2] + phibar * R[8]);
+    T p[3], pB[3];
+    cross3(ft, bW, p);
+    cross3_add(gt, wW, p, p);
+    p[2] += phibar;
+    rot3t(R, p, pB);
+    gh0 += sgn_bit<T>(A.sel, cidx, 0) * pB[0];
+    gh1 += sgn_bit<T>(A.sel, cidx, 1) * pB[1];
+    gh2 += sgn_bit<T>(A.sel, cidx, 2) * pB[2];
   }
   grad[10] += gmu;
   grad[11] += gh0; grad[12] += gh1; grad[13] += gh2;
@@ -670,29 +673,28 @@ CN_HD bool cube_loss_free_flight(const CubeParams<T>& P, const T* x, const T* xp
 #pragma unroll
     for (int k = 0; k < 3; ++k) Rh[3 * i + k] = R[3 * i + k] * P.h[k];
   bool open = true;
-  T pen = T(0), gh[3] = {T(0), T(0), T(0)};
+  T pen4 = T(0), gs[3] = {T(0), T(0), T(0)};
 #pragma unroll 1
   for (int c = 0; c < CUBE_NC; ++c) {
     const T sx = sgn_bit<T>(sel, c, 0), sy = sgn_bit<T>(sel, c, 1), sz = sgn_bit<T>(sel, c, 2);
     T rho[3], ed[3], ev[3];
 #pragma unroll
     for (int i = 0; i < 3; ++i) rho[i] = sx * Rh[3 * i] + sy * Rh[3 * i + 1] + sz * Rh[3 * i + 2];
-    cross3(dvW, rho, ed); cross3(vW, rho, ev);
-#pragma unroll
-    for (int i = 0; i < 3; ++i) { ed[i] += dv[3 + i]; ev[i] += vp[3 + i]; }
+    cross3_add(dvW, rho, dv + 3, ed); cross3_add(vW, rho, vp + 3, ev);
     const T tx = P.mu * ev[0], ty = P.mu * ev[1];
     const T speed2 = tx * tx + ty * ty;
-    const T speed = speed2 * t_rsqrt(t_max(speed2, t_tiny<T>()));
+    const T speed = speed2 * t_rsqrt0(speed2);
     const T phic = rho[2] + xp[6];
     const T q0 = -P.mu * ed[0] + P.dt * tx, q1 = -P.mu * ed[1] + P.dt * ty;
     const T qn = -ed[2] + t_abs(phic) + P.dt * speed;
     open = open && (qn >= T(0)) && (q0 * q0 + q1 * q1 <= qn * qn);
-    const T pneg = t_max(-phic, T(0));
-    pen += pneg * pneg;
-    const T phibar = T(-2) * pneg;                   // d loss / d phi_c at f = 0
-    gh[0] += sx * phibar * R[6]; gh[1] += sy * phibar * R[7]; gh[2] += sz * phibar * R[8];
+    const T pneg2 = t_abs(phic) - phic;              // 2 max(-phi_c, 0) = -d loss / d phi_c at f = 0, exactly
+    pen4 += pneg2 * pneg2;
+    gs[0] -= sx * pneg2; gs[1] -= sy * pneg2; gs[2] -= sz * pneg2;
   }
   if (!open) return false;
+  const T pen = T(0.25) * pen4;
+  const T gh[3] = {gs[0] * R[6], gs[1] * R[7], gs[2] * R[8]};
   // 1/2 dv^T M dv in state coordinates: w^T Io w + 2 m w . (c x R^T v) + m v . v
   T vB[3], Iw[3], cxv[3];
   rot3t(R, dv + 3, vB);
@@ -1028,25 +1030,24 @@ CN_HD bool body_loss_free_flight_pts(const CubeParams<T>& P, const T* x, const T
   T dvW[3], vW[3];
   rot3(R, dv, dvW); rot3(R, vp, vW);
   bool open = true;
-  T pen = T(0);
+  T pen4 = T(0);
 #pragma unroll 1
   for (int c = 0; c < n_c; ++c) {
     T rho[3], ed[3], ev[3];
     rot3(R, pts + 3 * c, rho);
-    cross3(dvW, rho, ed); cross3(vW, rho, ev);
-#pragma unroll
-    for (int i = 0; i < 3; ++i) { ed[i] += dv[3 + i]; ev[i] += vp[3 + i]; }
+    cross3_add(dvW, rho, dv + 3, ed); cross3_add(vW, rho, vp + 3, ev);
     const T tx = P.mu * ev[0], ty = P.mu * ev[1];
     const T speed2 = tx * tx + ty * ty;
-    const T speed = speed2 * t_rsqrt(t_max(speed2, t_tiny<T>()));
+    const T speed = speed2 * t_rsqrt0(speed2);
     const T phic = rho[2] + xp[6];
     const T q0 = -P.mu * ed[0] + P.dt * tx, q1 = -P.mu * ed[1] + P.dt * ty;
     const T qn = -ed[2] + t_abs(phic) + P.dt * speed;
     open = open && (qn >= T(0)) && (q0 * q0 + q1 * q1 <= qn * qn);
-    const T pneg = t_max(-phic, T(0));
-    pen += pneg * pneg;
+    const T pneg2 = t_abs(phic) - phic;              // 2 max(-phi_c, 0), exactly
+    pen4 += pneg2 * pneg2;
   }
   if (!open) return false;
+  const T pen = T(0.25) * pen4;
   // 1/2 dv^T M dv in state coordinates, as cube_loss_free_flight
   T vB[3], Iw[3], cxv[3];
   rot3t(R, dv + 3, vB);
@@ -1058,7 +1059,7 @@ CN_HD bool body_loss_free_flight_pts(const CubeParams<T>& P, const T* x, const T
   for (int c = 0; c < CUBE_NC; ++c) {
     // d loss / d p_c at f = 0: the penetration term only, -2 max(-phi_c, 0) R^T e_z
     const T phic = c < n_c ? R[6] * pts[3 * c] + R[7] * pts[3 * c + 1] + R[8] * pts[3 * c + 2] + xp[6] : T(0);
-    const T phibar = T(-2) * t_max(-phic, T(0)) * wpts;
+    const T phibar = (phic - t_abs(phic)) * wpts;
 #pragma unroll
     for (int k = 0; k < 3; ++k) if (grad_pts) grad_pts[3 * c + k] = (grad11 && c < n_c) ? phibar * R[6 + k] : T(0);
   }
@@ -1116,7 +1117,7 @@ CN_HD void body_loss_prologue_pts(const CubeParams<T>& P, const T* x, const T* x
   rot3(R, A.dv, dvW); rot3(R, A.vp, vW);
 #pragma unroll
   for (int i = 0; i < 3; ++i) { dvW[3 + i] = A.dv[3 + i]; vW[3 + i] = A.vp[3 + i]; }
-  T pen = T(0), a_min = T(2);
+  T pen4 = T(0), a_min = T(2);
 #pragma unroll UNR
   for (int c = 0; c < CUBE_NC; ++c) {
     if (c < n_c) {
@@ -1125,28 +1126,26 @@ CN_HD void body_loss_prologue_pts(const CubeParams<T>& P, const T* x, const T* x
 #pragma unroll
       for (int i = 0; i < 3; ++i) S.rho(3 * c + i) = rho[i];
       T ed[3], ev[3];
-      cross3(dvW, rho, ed); cross3(vW, rho, ev);
-#pragma unroll
-      for (int i = 0; i < 3; ++i) { ed[i] += dvW[3 + i]; ev[i] += vW[3 + i]; }
+      cross3_add(dvW, rho, dvW + 3, ed); cross3_add(vW, rho, vW + 3, ev);
       const T sx = P.mu * ev[0], sy = P.mu * ev[1];
       const T speed2 = sx * sx + sy * sy;
-      const T speed = speed2 * t_rsqrt(t_max(speed2, t_tiny<T>()));
+      const T speed = speed2 * t_rsqrt0(speed2);
       const T phic = rho[2] + A.pos_z;
       const T s0 = P.dt * sx, s1 = P.dt * sy, s2 = t_abs(phic) + P.dt * speed;
       const T e0 = -P.mu * ed[0], e1 = -P.mu * ed[1], e2 = -ed[2];
       S.q(3 * c) = e0 + s0;
       S.q(3 * c + 1) = e1 + s1;
       S.q(3 * c + 2) = e2 + s2;
-      const T pneg = t_max(-phic, T(0));
-      pen += pneg * pneg;
-      if (CN_LOSS_START_FACTOR > 0) {
-        const T Aq = e0 * e0 + e1 * e1 - e2 * e2, Bq = T(2) * (s0 * e0 + s1 * e1 - s2 * e2);
-        const T Cq = t_min(s0 * s0 + s1 * s1 - s2 * s2, T(0));
-        const T disc = Bq * Bq - T(4) * Aq * Cq;
-        const T dpos = t_max(disc, T(0));
-        const T den = Bq + dpos * t_rsqrt(t_max(dpos, t_tiny<T>()));
-        const T a_c = (disc >= T(0) && den > T(0)) ? T(-2) * Cq * t_rcp(den) : T(2);
-        a_min = t_min(a_min, a_c);
+      const T pneg2 = t_abs(phic) - phic;
+      pen4 += pneg2 * pneg2;
+      if (CN_LOSS_START_FACTOR > 0) {             // as cube_loss_prologue
+        const T Aq = e0 * e0 + e1 * e1 - e2 * e2, Bh = s0 * e0 + s1 * e1 - s2 * e2;
+        const T cs = s0 * s0 + s1 * s1 - s2 * s2;
+        const T Cq = T(0.5) * (cs - t_abs(cs));
+        const T disc = Bh * Bh - Aq * Cq;
+        const T den = Bh + disc * t_rsqrt0(disc);
+        const T a_c = den > T(0) ? -Cq * t_rcp(den) : T(2);
+        a_min = a_c < a_min ? a_c : a_min;
       }
     } else {
 #pragma unroll
@@ -1154,6 +1153,7 @@ CN_HD void body_loss_prologue_pts(const CubeParams<T>& P, const T* x, const T* x
       S.q(3 * c) = T(0); S.q(3 * c + 1) = T(0); S.q(3 * c + 2) = contact_off<T>();
     }
   }
+  const T pen = T(0.25) * pen4;
   A.a_min = a_min;
 #pragma unroll
   for (int i = 0; i < 6; ++i) A.dvW[i] = dvW[i];
@@ -1172,7 +1172,8 @@ CN_HD T body_loss_epilogue_pts(const CubeParams<T>& P, const CubeProb<T>& S, con
                                T wpts, T* grad11, T* grad_pts, T* force_out) {
   const T* R = A.R;
   T zW[6] = {T(0), T(0), T(0), T(0), T(0), T(0)};
-  T qf = T(0), ff = T(0), fmax = T(0);
+  T qf = T(0), ff = T(0);
+  bool fok = true;
 #pragma unroll UNR
   for (int c = 0; c < CUBE_NC; ++c) {
     T f[3] = {T(0), T(0), T(0)};
@@ -1181,14 +1182,12 @@ CN_HD T body_loss_epilogue_pts(const CubeParams<T>& P, const CubeProb<T>& S, con
       cube_contact_residual(P, S, c, u, rho, r);
       cone_eval<T, false>(r, P.inv_eps, P.mu, f, (T*)nullptr);
       const T ft[3] = {P.mu * f[0], P.mu * f[1], f[2]};
-      T tq[3];
-      cross3(rho, ft, tq);
+      cross3_add(rho, ft, zW, zW);
 #pragma unroll
       for (int i = 0; i < 3; ++i) {
-        zW[i] += tq[i]; zW[3 + i] += ft[i];
+        zW[3 + i] += ft[i];
         qf += S.q(3 * c + i) * f[i]; ff += f[i] * f[i];
-        const T af = t_abs(f[i]);
-        fmax = (af > fmax || af != af) ? af : fmax;
+        fok = fok && t_abs(f[i]) <= T(1e3);
       }
       if (PARK) {
 #pragma unroll
@@ -1201,7 +1200,7 @@ CN_HD T body_loss_epilogue_pts(const CubeParams<T>& P, const CubeProb<T>& S, con
 #pragma unroll 1
     for (int i = 0; i < 12; ++i) grad_pts[i] = T(0);
   }
-  if (!(fmax <= T(1e3))) {
+  if (!fok) {
     if (force_out) for (int i = 0; i < 12; ++i) force_out[i] = T(0);
     return T(0);
   }
@@ -1246,23 +1245,24 @@ CN_HD T body_loss_epilogue_pts(const CubeParams<T>& P, const CubeProb<T>& S, con
       }
       const T ftx = f[0], fty = f[1], fn = f[2];
       T eb[3], ev[3];
-      cross3(bW, rho, eb); cross3(wW, rho, ev);
-#pragma unroll
-      for (int i = 0; i < 3; ++i) { eb[i] += b[3 + i]; ev[i] += w[3 + i]; }
+      cross3_add(bW, rho, b + 3, eb); cross3_add(wW, rho, w + 3, ev);
       const T sx = P.mu * ev[0], sy = P.mu * ev[1];
-      const T sinv = t_rsqrt(t_max(sx * sx + sy * sy, t_tiny<T>()));
+      const T sinv = t_rsqrt0(sx * sx + sy * sy);
       const T ux = sx * sinv, uy = sy * sinv;
       const T gx = P.dt * (fn * ux + ftx), gy = P.dt * (fn * uy + fty);
-      gmu += ftx * eb[0] + fty * eb[1] + gx * ev[0] + gy * ev[1];
+      gmu = gmu + ftx * eb[0] + fty * eb[1] + gx * ev[0] + gy * ev[1];
+      const T phic = rho[2] + A.pos_z;
+      const T phibar = (phic > T(0) ? fn : (phic < T(0) ? -fn : T(0))) - (t_abs(phic) - phic);
+      // as cube_loss_epilogue: R^T (ft x bW + gt x wW + phibar e_z)
       const T ft[3] = {P.mu * ftx, P.mu * fty, fn};
       const T gt[3] = {P.mu * gx, P.mu * gy, T(0)};
-      T ftB[3], gtB[3], p1[3], p2[3];
-      rot3t(R, ft, ftB); rot3t(R, gt, gtB);
-      cross3(ftB, b, p1); cross3(gtB, w, p2);
-      const T phic = rho[2] + A.pos_z;
-      const T phibar = (phic > T(0) ? fn : (phic < T(0) ? -fn : T(0))) - T(2) * t_max(-phic, T(0));
+      T p[3], pB[3];
+      cross3(ft, bW, p);
+      cross3_add(gt, wW, p, p);
+      p[2] += phibar;
+      rot3t(R, p, pB);
 #pragma unroll
-      for (int k = 0; k < 3; ++k) if (grad_pts) grad_pts[3 * c + k] = wpts * (p1[k] + p2[k] + phibar * R[6 + k]);
+      for (int k = 0; k < 3; ++k) if (grad_pts) grad_pts[3 * c + k] = wpts * pB[k];
     }
   }
   grad11[10] += gmu;
