@@ -17,6 +17,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/dair_pll_b200.h"
+#include "../../include/dair_pll_b200_warm.h"
 #include "cn_elbow_wf.cuh"
 #include "cn_launch.cuh"
 #include "cn_reduce.cuh"
@@ -102,16 +103,21 @@ __device__ __forceinline__ void ew_load_params(cn::ElbowParams<T>& P, const IO* 
   cn::elbow_params_init(P, in, m, h, kn, dt, eps);
 }
 
-template <typename T, typename IO>
+template <typename T, typename IO, bool WARM>
 __global__ void __launch_bounds__(kEwWarps * 32)
 elbow_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const IO* __restrict__ weight,
                      const IO* __restrict__ inertia, const IO* __restrict__ mu, const IO* __restrict__ half,
                      const IO* __restrict__ kin, const IO* __restrict__ pts, T dt, T eps, int64_t B,
                      IO* __restrict__ loss, IO* __restrict__ force, IO* __restrict__ grad_pts,
                      int32_t* __restrict__ iters, T* __restrict__ partials, int want_grad,
-                     const int32_t* __restrict__ skip_flag, unsigned long long* __restrict__ dyn_counter) {
+                     const int32_t* __restrict__ skip_flag, unsigned long long* __restrict__ dyn_counter,
+                     const IO* u_init, IO* u_out) {
   // dyn_counter != nullptr (DPLL_LOSS_DYNAMIC): warps draw their 32-sample chunks from a global counter, in batch
   // order (cost-ordered batches: uniform chunks, longest solves first), as cube_loss_wf_kernel does.
+  // WARM (u_init / u_out, nullable, (B, 7); they may be the same array): a solve starts from u_init[b] instead of the
+  // feasible-segment point, and every sample's optimum (zero for free flight) goes to u_out[b].  Row b is read when its
+  // sample gets a slot and written when that sample is finalised.  The cold instances take the two parameters last and
+  // never read them: their warm code sits in `if constexpr` branches, so their register allocation stays as it was.
   if (skip_flag && *skip_flag) return;
   extern __shared__ __align__(16) unsigned char ew_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -179,6 +185,12 @@ elbow_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const 
           if (loss) loss[b] = IO(l);
           gs[DPLL_ELBOW_NPARAM] = l;
           if (iters) iters[b] = 0;
+          if constexpr (WARM) {
+            if (u_out) {
+#pragma unroll 1
+              for (int i = 0; i < 7; ++i) u_out[b * 7 + i] = IO(0);
+            }
+          }
         } else {
           queue = true;
         }
@@ -258,8 +270,19 @@ elbow_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const 
             if (loss) loss[b] = IO(l);
             gs[DPLL_ELBOW_NPARAM] = l;
             if (iters) iters[b] = pool->iters[slot] & 0xff;
+            if constexpr (WARM) {
+              if (u_out) {
+#pragma unroll
+                for (int i = 0; i < 7; ++i) u_out[b * 7 + i] = IO(u[i]);
+              }
+            }
             pool->sample[slot] = -1;
           } else {
+            if constexpr (WARM) {
+#pragma unroll
+              for (int i = 0; i < 7; ++i)
+                pool->field[77 + i][slot] = u_init ? T(u_init[b * 7 + i]) : (T(1) - A.a_start) * A.dv[i];
+            } else
 #pragma unroll
             for (int i = 0; i < 7; ++i) pool->field[77 + i][slot] = (T(1) - A.a_start) * A.dv[i];
             pool->field[91][slot] = T(-1);
@@ -300,11 +323,14 @@ template <typename T, typename IO>
 int launch_elbow_loss(const IO* x, const IO* xp, const IO* weight, const IO* inertia, const IO* mu, const IO* half,
                       const IO* kin, const IO* pts, T dt, T eps, int64_t B, IO* loss, IO* force, IO* grad_pts,
                       int32_t* iters, IO* grad, IO* loss_sum,
-                      const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream, int flags) {
+                      const int32_t* skip_flag, void* workspace, size_t workspace_bytes, void* stream, int flags,
+                      const IO* u_init = nullptr, IO* u_out = nullptr) {
   if (B < 0 || !inertia || !mu || (!half && !pts) || !kin || (grad_pts && (!pts || !grad))) return DPLL_EINVAL;
   if (B > 0 && (!x || !xp)) return DPLL_EINVAL;
   const bool want_red = grad || loss_sum;
   if (want_red && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
+  const bool warm = u_init || u_out;
+  if (warm && B == 0 && !want_red) return DPLL_OK;      // nothing to write: an empty warm call launches nothing
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   T* partials = want_red ? static_cast<T*>(workspace) : nullptr;
   unsigned long long* dyn = nullptr;
@@ -312,18 +338,19 @@ int launch_elbow_loss(const IO* x, const IO* xp, const IO* weight, const IO* ine
     if (!cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
     if (int rc = cn::dynamic_counter(workspace, st, &dyn)) return rc;
   }
+  // with both warm-start pointers NULL the cold instance runs, exactly as dpll_elbow_loss_*
+  auto kernel = warm ? elbow_loss_wf_kernel<T, IO, true> : elbow_loss_wf_kernel<T, IO, false>;
   const size_t smem = sizeof(EwWarpPool<T>) * kEwWarps;
-  cudaError_t ea = cudaFuncSetAttribute(elbow_loss_wf_kernel<T, IO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t ea = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (ea != cudaSuccess) return (int)ea;
   // at most one resident set; a warp wants >= 128 samples to keep its pool busy
   int blocks;
   int64_t cap;
-  if (int rc = cn::resident_blocks(elbow_loss_wf_kernel<T, IO>, kEwWarps * 32, smem, (B + kEwWarps * 128 - 1) / (kEwWarps * 128),
+  if (int rc = cn::resident_blocks(kernel, kEwWarps * 32, smem, (B + kEwWarps * 128 - 1) / (kEwWarps * 128),
                                    kEwMaxBlocks, &blocks, &cap))
     return rc;
-  elbow_loss_wf_kernel<T, IO><<<blocks, kEwWarps * 32, smem, st>>>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B,
-                                                                   loss, force, grad_pts, iters, partials, grad ? 1 : 0,
-                                                                   skip_flag, dyn);
+  kernel<<<blocks, kEwWarps * 32, smem, st>>>(x, xp, weight, inertia, mu, half, kin, pts, dt, eps, B, loss, force,
+                                              grad_pts, iters, partials, grad ? 1 : 0, skip_flag, dyn, u_init, u_out);
   if (int rc = cn::launch_status()) return rc;
   if (!want_red) return DPLL_OK;
   reduce_partials_kernel<T, IO, kEwNAcc, DPLL_ELBOW_NPARAM><<<1, 32 * kEwNAcc, 0, st>>>(partials, blocks, grad, loss_sum,
@@ -353,6 +380,26 @@ int dpll_elbow_loss_f32(const float* x, const float* x_plus, const float* weight
   return launch_elbow_loss<double, float>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, (double)dt, (double)eps, B,
                                           loss, force, grad_pts, iters, grad, loss_sum, skip_flag, workspace,
                                           workspace_bytes, stream, flags);
+}
+
+int dpll_elbow_loss_warm_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
+                             const double* mu_pair, const double* half, const double* kin, const double* pts, double dt,
+                             double eps, int64_t B, int32_t flags, double* loss, double* force, double* grad_pts,
+                             int32_t* iters, double* grad, double* loss_sum, const int32_t* skip_flag,
+                             const double* u_init, double* u_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return launch_elbow_loss<double, double>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, loss, force,
+                                           grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream,
+                                           flags, u_init, u_out);
+}
+
+int dpll_elbow_loss_warm_f32(const float* x, const float* x_plus, const float* weight, const float* inertia,
+                             const float* mu_pair, const float* half, const float* kin, const float* pts, float dt,
+                             float eps, int64_t B, int32_t flags, float* loss, float* force, float* grad_pts,
+                             int32_t* iters, float* grad, float* loss_sum, const int32_t* skip_flag,
+                             const float* u_init, float* u_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return launch_elbow_loss<double, float>(x, x_plus, weight, inertia, mu_pair, half, kin, pts, (double)dt, (double)eps, B,
+                                          loss, force, grad_pts, iters, grad, loss_sum, skip_flag, workspace,
+                                          workspace_bytes, stream, flags, u_init, u_out);
 }
 
 }  // extern "C"

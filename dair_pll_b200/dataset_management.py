@@ -44,7 +44,7 @@ class DeviceTrajectorySliceDataset:
         self._future: List[Tensor] = []
         self._dense: Optional[Tuple[Tensor, Tensor]] = None
         self._cost: Optional[Tensor] = None      # (N,) int32 per-slice cost hint (last epoch's Newton counts)
-        self._usol: Optional[Tensor] = None      # (N, 6) last epoch's QP optima: next epoch's warm starts
+        self._usol: Optional[Tensor] = None      # (N, 6) cube / (N, 7) elbow: last epoch's QP optima, next epoch's warm starts
 
     def add_slices_from_trajectory(self, trajectory: Tensor) -> None:
         """``trajectory``: (T, n_x).  Slice i predicts from time index ``t_skip + i``
@@ -108,11 +108,16 @@ class DeviceTrajectorySliceDataset:
             self._cost[indices.reshape(-1).to(self.device)] = it
 
     def update_solutions(self, indices: Optional[Tensor], qp_solution: Tensor) -> None:
-        """Records ``BatchLoss.qp_solution`` (the cone QPs' optima) of the slices ``indices`` (None: all)."""
+        """Records ``BatchLoss.qp_solution`` (the cone QPs' optima) of the slices ``indices`` (None: all).  The width of a
+        solution (6 for the cube, 7 for the elbow) is taken from the first one recorded; a later one of another width
+        raises."""
         n = len(self)
+        width = qp_solution.shape[-1]
         if self._usol is None:
-            self._usol = torch.zeros((n, 6), dtype=self.dtype, device=self.device)
-        u = qp_solution.reshape(-1, 6).to(device=self.device, dtype=self.dtype)
+            self._usol = torch.zeros((n, width), dtype=self.dtype, device=self.device)
+        elif width != self._usol.shape[1]:
+            raise ValueError(f'QP solutions of width {width}, but this data set records width {self._usol.shape[1]}')
+        u = qp_solution.reshape(-1, width).to(device=self.device, dtype=self.dtype)
         if indices is None:
             assert u.shape[0] == n
             self._usol.copy_(u)
@@ -120,7 +125,7 @@ class DeviceTrajectorySliceDataset:
             self._usol[indices.reshape(-1).to(self.device)] = u
 
     def warm_start(self, indices: Optional[Tensor] = None) -> Optional[Tensor]:
-        """(len(indices), 6) warm starts for ``system.qp_warm_start`` (zeros before the first epoch); None if no
+        """(len(indices), width) warm starts for ``system.qp_warm_start`` (zeros for slices not recorded yet); None if no
         solution has been recorded yet."""
         if self._usol is None:
             return None

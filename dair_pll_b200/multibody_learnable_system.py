@@ -61,9 +61,10 @@ class MultibodyLearnableSystem(System):
         self.race_expensive_head = True  # with dynamic_schedule, small launches: the first B/64 samples of the (cost-ordered)
                                          # batch are solved from eight start points at once, first to converge wins (cube)
         self.record_newton_iters = False  # BatchLoss.newton_iters: per-sample cost hint for the data set
-        self.qp_warm_start = None        # (B, 6) contiguous start points of the next contactnets_loss call's solves
-                                         # (cube); with record_qp_solution it is overwritten in place by the optima
-        self.record_qp_solution = False  # BatchLoss.qp_solution (B, 6): the optima, next epoch's warm start
+        self.qp_warm_start = None        # (B, 6) / (B, 7) contiguous start points of the next contactnets_loss call's solves
+                                         # (cube, elbow); with record_qp_solution it is overwritten in place by the optima
+        self.record_qp_solution = False  # BatchLoss.qp_solution (B, 6) / (B, 7): the optima, next epoch's warm start
+                                         # (cube, elbow)
         self._kin_cache = {}
 
     # -- helpers ---------------------------------------------------------
@@ -209,16 +210,36 @@ class MultibodyLearnableSystem(System):
                                           'parallel.GradientAllReduce (NCCL) for this system')
             inertia, mu, half, kin = self._elbow_params(x.dtype, x.device)
             xf, xpf = self._flat(x), self._flat(x_plus)
+            warm, self.qp_warm_start = self.qp_warm_start, None          # consumed by this call
+            if warm is not None and (warm.shape[-1] != 7 or warm.numel() != 7 * xf.shape[0] or warm.dtype != x.dtype or
+                                     (self.record_qp_solution and not warm.is_contiguous())):
+                raise ValueError(f'qp_warm_start must be a contiguous ({xf.shape[0]}, 7) {x.dtype} tensor for this batch, '
+                                 f'got {tuple(warm.shape)} {warm.dtype}')
+            u_init = warm.reshape(-1, 7) if warm is not None else None
             if half is None:      # learned geometry: witness points from the support-function networks
                 pts = self._elbow_witness_points(xpf[:, :8])
-                loss = ops.ElbowContactNetsLossPts.apply(xf, xpf, inertia, mu, pts, kin, float(self.dt), LOSS_EPS)
+                if u_init is None and not self.record_qp_solution:
+                    loss = ops.ElbowContactNetsLossPts.apply(xf, xpf, inertia, mu, pts, kin, float(self.dt), LOSS_EPS)
+                    usol = None
+                else:
+                    loss, usol = ops.ElbowContactNetsLossPts.apply(xf, xpf, inertia, mu, pts, kin, float(self.dt), LOSS_EPS,
+                                                                   u_init, self.record_qp_solution)
+                out = loss.reshape(batch).as_subclass(ops.BatchLoss)
+                out._dpll_fused = None           # mean() / sum() are plain reductions: the points' gradient needs the graph
+                out.newton_iters = None
             else:
                 flags = ops.LOSS_DYNAMIC if self.dynamic_schedule else 0
-                loss, sums, means, iters = ops.ElbowContactNetsLoss.apply(xf, xpf, inertia, mu, half, kin, float(self.dt),
-                                                                          LOSS_EPS, flags, self.record_newton_iters)
+                loss, sums, means, iters, usol = ops.ElbowContactNetsLoss.apply(
+                    xf, xpf, inertia, mu, half, kin, float(self.dt), LOSS_EPS, flags, self.record_newton_iters, u_init,
+                    self.record_qp_solution)
                 # mean() / sum() of the result reuse the launch's own reduction and fused gradient (ops.BatchLoss)
-                return ops.batch_loss(loss.reshape(batch), sums, means, 28, (inertia, mu, half),
-                                      iters.reshape(batch) if self.record_newton_iters else None)
+                out = ops.batch_loss(loss.reshape(batch), sums, means, 28, (inertia, mu, half),
+                                     iters.reshape(batch) if self.record_newton_iters else None)
+            out.qp_solution = None
+            if self.record_qp_solution:
+                # with a warm start the optima were written back into the warm-start tensor itself
+                out.qp_solution = (warm if warm is not None else usol).reshape(batch + (7,))
+            return out
         elif self._kind() == 'chain' and not self._chain_boxes_only():
             # other shapes than boxes on the links: each shape's support points (host side, ordinary torch functions of the
             # shape parameters) become the witness points of the tree kernels

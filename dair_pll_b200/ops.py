@@ -369,10 +369,14 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
                    dt: float, eps: float, weight: Optional[Tensor] = None, want_grad: bool = True,
                    want_force: bool = False, want_iters: bool = False, want_loss: bool = True,
                    skip_flag: Optional[Tensor] = None, grad_out: Optional[Tensor] = None,
-                   pts: Optional[Tensor] = None, want_grad_pts: bool = False, flags: int = 0):
+                   pts: Optional[Tensor] = None, want_grad_pts: bool = False, flags: int = 0,
+                   u_init: Optional[Tensor] = None, u_out: Optional[Tensor] = None):
     """Direct call of ``dpll_elbow_loss_*`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,15); inertia (20), mu_pair (2), half (6) or
     witness points pts (B,8,3), kin (12).  Returns (loss (B,) | None, grad (28,) | None, loss_sum (1,),
-    force (B,24) | None, iters (B,) | None[, grad_pts (B,8,3)])."""
+    force (B,24) | None, iters (B,) | None[, grad_pts (B,8,3)]).  ``u_init`` (B,7): start point of every sample's Newton
+    solve (e.g. last epoch's optima); ``u_out`` (B,7), contiguous, of the launch dtype: receives every sample's optimum
+    (zero for free flight) and may be ``u_init`` itself.  With either the warm entry point
+    ``dpll_elbow_loss_warm_*`` runs; the optimum is unique, so only the Newton count depends on the start."""
     dtype = _check_inputs(x, x_plus, inertia, mu_pair, kin, half, pts)
     x, x_plus = x.contiguous(), x_plus.contiguous()
     inertia, mu_pair, kin = inertia.contiguous(), mu_pair.contiguous(), kin.contiguous()
@@ -395,8 +399,18 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
     if weight is not None:
         weight = weight.to(dtype).contiguous()
     grad_pts = torch.zeros((B, 8, 3), dtype=dtype, device=dev) if (want_grad_pts and want_grad) else None
-    _call('dpll_elbow_loss', dev, x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, flags, loss, force,
-          grad_pts, iters, grad, loss_sum, skip_flag, dtype=dtype, workspace=True)
+    if u_init is not None:
+        if tuple(u_init.shape) != (B, 7):
+            raise ValueError(f'u_init must be (B,7), got {tuple(u_init.shape)}')
+        u_init = u_init.detach().to(dtype).contiguous()
+    if u_out is not None and (tuple(u_out.shape) != (B, 7) or u_out.dtype != dtype or not u_out.is_contiguous()):
+        raise ValueError(f'u_out must be a contiguous (B,7) {dtype} tensor, got {tuple(u_out.shape)} {u_out.dtype}')
+    if u_init is None and u_out is None:
+        _call('dpll_elbow_loss', dev, x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, flags, loss, force,
+              grad_pts, iters, grad, loss_sum, skip_flag, dtype=dtype, workspace=True)
+    else:
+        _call('dpll_elbow_loss_warm', dev, x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, flags, loss,
+              force, grad_pts, iters, grad, loss_sum, skip_flag, u_init, u_out, dtype=dtype, workspace=True)
     if want_grad_pts:
         return loss, grad, loss_sum, force, iters, grad_pts
     return loss, grad, loss_sum, force, iters
@@ -406,57 +420,88 @@ class ElbowContactNetsLoss(torch.autograd.Function):
     """ContactNets loss of the elbow (floating base + hinge, two boxes); differentiable w.r.t. the
     callable-level parameters (two inertia 10-vectors, two pair frictions, two half-length triples).
     Same fused-backward protocol as :class:`CubeContactNetsLoss`; also returns the launch's
-    [gradient (28) | loss] sums and means for :class:`BatchLoss`."""
+    [gradient (28) | loss] sums and means for :class:`BatchLoss`, the Newton counts (empty unless ``want_iters``) and the
+    QP optima (below).
+
+    ``u_init`` (B,7): warm start of every sample's solve; ``want_u``: record the optima.  As for
+    :class:`CubeContactNetsLossLeaf`, with a warm start they are written back into ``u_init`` in place and the returned
+    ``usol`` is empty; without one ``usol`` is a new (B,7) tensor (empty unless ``want_u``).  A weighted backward re-launch
+    starts from the optima (or from ``u_init``) and records nothing."""
 
     @staticmethod
-    def forward(ctx, x, x_plus, inertia, mu_pair, half, kin, dt, eps, flags=0, want_iters=False):
+    def forward(ctx, x, x_plus, inertia, mu_pair, half, kin, dt, eps, flags=0, want_iters=False, u_init=None, want_u=False):
         need = any(ctx.needs_input_grad[2:5])
+        u_out = _optima_buffer(x, u_init, want_u)
         loss, grad, loss_sum, _, iters = elbow_loss_raw(x, x_plus, inertia, mu_pair, half, kin, dt, eps, want_grad=need,
-                                                        want_iters=want_iters, flags=flags)
+                                                        want_iters=want_iters, flags=flags, u_init=u_init, u_out=u_out)
         ctx.dt, ctx.eps = dt, eps
-        if need:
-            ctx.save_for_backward(grad, x, x_plus, inertia, mu_pair, half, kin)
+        if need:      # the last one is the start point of a weighted re-launch
+            ctx.save_for_backward(grad, x, x_plus, inertia, mu_pair, half, kin, u_out if u_out is not None else u_init)
         else:
             grad = torch.zeros(28, dtype=loss.dtype, device=loss.device)
         sums = torch.cat((grad, loss_sum))
         means = sums / max(loss.numel(), 1) if loss.numel() > 0 else sums * float('nan')
         if iters is None:
             iters = torch.empty(0, dtype=torch.int32, device=loss.device)
-        ctx.mark_non_differentiable(sums, means, iters)
-        return loss, sums, means, iters
+        usol = u_out if (u_out is not None and u_init is None) else torch.empty(0, dtype=loss.dtype, device=loss.device)
+        ctx.mark_non_differentiable(sums, means, iters, usol)
+        return loss, sums, means, iters, usol
 
     @staticmethod
-    def backward(ctx, grad_loss, _g_sums, _g_means, _g_iters):
-        grad, x, x_plus, inertia, mu_pair, half, kin = ctx.saved_tensors
+    def backward(ctx, grad_loss, _g_sums, _g_means, _g_iters, _g_u):
+        grad, x, x_plus, inertia, mu_pair, half, kin, u_start = ctx.saved_tensors
         g = _fused_grad(grad, grad_loss, lambda w, skip, out: elbow_loss_raw(
-            x, x_plus, inertia, mu_pair, half, kin, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip, grad_out=out))
-        return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None, None)
+            x, x_plus, inertia, mu_pair, half, kin, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip, grad_out=out,
+            u_init=u_start))
+        return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None, None, None, None)
+
+
+def _optima_buffer(x: Tensor, u_init: Optional[Tensor], want_u: bool) -> Optional[Tensor]:
+    """Where a warm-started elbow launch writes its optima: ``u_init`` itself (in place: a training loop keeps one (B,7)
+    buffer per batch and copies nothing between epochs), a new (B,7) tensor, or nowhere."""
+    if not want_u:
+        return None
+    if u_init is None:
+        return torch.empty((x.shape[0], 7), dtype=x.dtype, device=x.device)
+    if u_init.dtype != x.dtype or not u_init.is_contiguous():
+        raise ValueError(f'a warm start that records the optima in place must be a contiguous {x.dtype} tensor, got '
+                         f'{u_init.dtype}')
+    return u_init
 
 
 class ElbowContactNetsLossPts(torch.autograd.Function):
     """ContactNets loss of the elbow with LEARNED geometry: the 4 + 4 witness points ``pts`` (B,8,3) come
     from the support-function networks (``DeepSupportConvex.get_vertices``).  Differentiable w.r.t.
     inertia (20), mu_pair (2) and ``pts``; the per-sample d loss_b / d pts[b] is produced by the forward
-    launch and scaled by the upstream gradient (exact for any upstream weights)."""
+    launch and scaled by the upstream gradient (exact for any upstream weights).
+
+    ``u_init`` / ``want_u`` as for :class:`ElbowContactNetsLoss`.  When either is given the Function returns
+    (loss, usol), ``usol`` non-differentiable (empty when the optima went into ``u_init`` in place); otherwise the loss
+    alone."""
 
     @staticmethod
-    def forward(ctx, x, x_plus, inertia, mu_pair, pts, kin, dt, eps):
+    def forward(ctx, x, x_plus, inertia, mu_pair, pts, kin, dt, eps, u_init=None, want_u=False):
         need = any(ctx.needs_input_grad[2:5])
+        u_out = _optima_buffer(x, u_init, want_u)
         out = elbow_loss_raw(x, x_plus, inertia, mu_pair, None, kin, dt, eps, want_grad=need, pts=pts,
-                             want_grad_pts=True)
+                             want_grad_pts=True, u_init=u_init, u_out=u_out)
         loss, grad, gpts = out[0], out[1], out[5]
         ctx.dt, ctx.eps = dt, eps
         if need:
-            ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts, kin)
-        return loss
+            ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts, kin, u_out if u_out is not None else u_init)
+        if u_init is None and not want_u:
+            return loss
+        usol = u_out if (u_out is not None and u_init is None) else torch.empty(0, dtype=loss.dtype, device=loss.device)
+        ctx.mark_non_differentiable(usol)
+        return loss, usol
 
     @staticmethod
-    def backward(ctx, grad_loss):
-        grad, gpts, x, x_plus, inertia, mu_pair, pts, kin = ctx.saved_tensors
+    def backward(ctx, grad_loss, _g_u=None):
+        grad, gpts, x, x_plus, inertia, mu_pair, pts, kin, u_start = ctx.saved_tensors
         g = _fused_grad(grad, grad_loss, lambda w, skip, out: elbow_loss_raw(
             x, x_plus, inertia, mu_pair, None, kin, ctx.dt, ctx.eps, weight=w, want_loss=False, skip_flag=skip,
-            grad_out=out, pts=pts))
-        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1), None, None, None)
+            grad_out=out, pts=pts, u_init=u_start))
+        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1), None, None, None, None, None)
 
 
 def elbow_rollout_saved(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Optional[Tensor], kin: Tensor, dt: float,
