@@ -1,5 +1,5 @@
-"""ctypes binding of ``libdair_pll_b200.so`` (C ABI: ``include/dair_pll_b200.h`` and its warm-start extension
-``include/dair_pll_b200_warm.h``).
+"""ctypes binding of ``libdair_pll_b200.so`` (C ABI: ``include/dair_pll_b200.h`` and its warm-start extensions
+``include/dair_pll_b200_warm.h`` and ``include/dair_pll_b200_warm_body_tree.h``).
 
 There is deliberately no fallback: if the CUDA library is missing or a call fails, the
 caller gets an exception.  The library is built in-tree by ``dair_pll_b200.build``.
@@ -15,6 +15,7 @@ ABI_VERSION = 214        # DPLL_VERSION of include/dair_pll_b200.h this binding 
 _INCLUDE = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'include')
 HEADER = os.path.join(_INCLUDE, 'dair_pll_b200.h')
 WARM_HEADER = os.path.join(_INCLUDE, 'dair_pll_b200_warm.h')
+WARM_BODY_TREE_HEADER = os.path.join(_INCLUDE, 'dair_pll_b200_warm_body_tree.h')
 
 _SCALARS = {'double': ctypes.c_double, 'float': ctypes.c_float, 'int': ctypes.c_int32, 'int32_t': ctypes.c_int32,
             'int64_t': ctypes.c_int64, 'uint32_t': ctypes.c_uint32, 'size_t': ctypes.c_size_t}
@@ -52,6 +53,7 @@ def _signatures(path: str = HEADER) -> dict:
 
 EXPORTS = _signatures()                      # the main header's entry points
 WARM_EXPORTS = _signatures(WARM_HEADER)      # the warm-started elbow loss (its own header)
+WARM_BODY_TREE_EXPORTS = _signatures(WARM_BODY_TREE_HEADER)      # the warm-started tree losses (their own header)
 
 
 def lib_path() -> str:
@@ -72,7 +74,7 @@ def load() -> ctypes.CDLL:
             # argtypes are positional: a library older than its sources could take shifted pointers
             raise RuntimeError(f'{path} is older than csrc/ or include/: rebuild it with `python -m dair_pll_b200.build`')
         lib = ctypes.CDLL(path)
-        for name, (argtypes, restype) in (*EXPORTS.items(), *WARM_EXPORTS.items()):
+        for name, (argtypes, restype) in (*EXPORTS.items(), *WARM_EXPORTS.items(), *WARM_BODY_TREE_EXPORTS.items()):
             fn = getattr(lib, name)      # AttributeError if the symbol is missing
             fn.argtypes = argtypes
             fn.restype = restype

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/dair_pll_b200.h"
+#include "../../include/dair_pll_b200_warm_body_tree.h"
 #include "cn_chain.cuh"
 #include "cn_launch.cuh"
 
@@ -19,15 +20,18 @@ template <typename T> __device__ __forceinline__ T ch_warp_sum(T v) {
   return v;
 }
 
-template <typename T, int N>
+template <typename T, int N, bool WARM = false>
 __global__ void __launch_bounds__(kChThreads)
 chain_loss_kernel(const T* __restrict__ x, const T* __restrict__ xp, const T* __restrict__ weight,
                   const T* __restrict__ inertia, const T* __restrict__ mu, const T* __restrict__ half,
                   const T* __restrict__ kin, T dt, T eps, int64_t B, T* __restrict__ loss, T* __restrict__ force,
                   int32_t* __restrict__ iters, T* __restrict__ partials, int want_grad,
-                  const T* __restrict__ pts = nullptr, unsigned npts = 0u, T* __restrict__ grad_pts = nullptr) {
+                  const T* __restrict__ pts = nullptr, unsigned npts = 0u, T* __restrict__ grad_pts = nullptr,
+                  const T* u_init = nullptr, T* u_out = nullptr) {
   // pts (nullable, (B, N, 4, 3)): witness points per box slot instead of box corners (half is then unused and may be
   // null); grad_pts (nullable, same shape): w_b d loss_b / d pts_b
+  // WARM (u_init / u_out, nullable, (B, 5 + N); they may be the same array): sample b's solve starts from u_init[b] and
+  // its optimum goes to u_out[b] (chain_loss_sample).  The cold instances never read the two parameters.
   constexpr int NX = 13 + 2 * (N - 1), NP = 14 * N, NF = 12 * N;
   cn::ChainParams<T, N> P;
   cn::chain_params_init<T, N>(P, inertia, mu, half, kin, dt, eps);
@@ -42,8 +46,18 @@ chain_loss_kernel(const T* __restrict__ x, const T* __restrict__ xp, const T* __
     int it;
     T ps[12 * N], gps[12 * N];
     if (pts) for (int i = 0; i < 12 * N; ++i) ps[i] = pts[b * 12 * N + i];
-    const T l = cn::chain_loss_sample<T, N>(P, cfg, xs, xps, (want_grad || grad_pts) ? gs : (T*)nullptr, force ? fo : (T*)nullptr, &it,
-                                            pts ? ps : (const T*)nullptr, npts, grad_pts ? gps : (T*)nullptr);
+    T l;
+    if constexpr (WARM) {
+      constexpr int NV = 5 + N;
+      T u0[NV], uo[NV];
+      if (u_init) for (int i = 0; i < NV; ++i) u0[i] = u_init[b * NV + i];
+      l = cn::chain_loss_sample<T, N>(P, cfg, xs, xps, (want_grad || grad_pts) ? gs : (T*)nullptr, force ? fo : (T*)nullptr,
+                                      &it, pts ? ps : (const T*)nullptr, npts, grad_pts ? gps : (T*)nullptr,
+                                      u_init ? u0 : (const T*)nullptr, u_out ? uo : (T*)nullptr);
+      if (u_out) for (int i = 0; i < NV; ++i) u_out[b * NV + i] = uo[i];
+    } else
+    l = cn::chain_loss_sample<T, N>(P, cfg, xs, xps, (want_grad || grad_pts) ? gs : (T*)nullptr, force ? fo : (T*)nullptr, &it,
+                                    pts ? ps : (const T*)nullptr, npts, grad_pts ? gps : (T*)nullptr);
     if (force) for (int i = 0; i < NF; ++i) force[b * NF + i] = fo[i];
     const T w = weight ? weight[b] : T(1);
     if (grad_pts) for (int i = 0; i < 12 * N; ++i) grad_pts[b * 12 * N + i] = w * gps[i];
@@ -106,13 +120,22 @@ template <int N>
 int launch_chain_loss(const double* x, const double* xp, const double* weight, const double* inertia, const double* mu,
                       const double* half, const double* kin, double dt, double eps, int64_t B, double* loss, double* force,
                       int32_t* iters, double* grad, double* loss_sum, void* workspace, size_t workspace_bytes,
-                      cudaStream_t st, const double* pts = nullptr, unsigned npts = 0u, double* grad_pts = nullptr) {
+                      cudaStream_t st, const double* pts = nullptr, unsigned npts = 0u, double* grad_pts = nullptr,
+                      const double* u_init = nullptr, double* u_out = nullptr) {
   const bool want_red = grad || loss_sum;
   if (want_red && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
+  const bool warm = u_init || u_out;
+  if (warm && B == 0 && !want_red) return DPLL_OK;      // nothing to write: an empty warm call launches nothing
   int64_t need = (B + kChThreads - 1) / kChThreads;
   int blocks = (int)(need < kChMaxBlocks ? need : kChMaxBlocks);
   if (blocks < 1) blocks = 1;
   double* partials = want_red ? static_cast<double*>(workspace) : nullptr;
+  // with both warm-start pointers NULL the cold instance runs, exactly as dpll_chain_loss_f64 / dpll_chain_loss_pts_f64
+  if (warm)
+    chain_loss_kernel<double, N, true><<<blocks, kChThreads, 0, st>>>(x, xp, weight, inertia, mu, half, kin, dt, eps, B, loss,
+                                                                     force, iters, partials, grad ? 1 : 0, pts, npts,
+                                                                     grad_pts, u_init, u_out);
+  else
   chain_loss_kernel<double, N><<<blocks, kChThreads, 0, st>>>(x, xp, weight, inertia, mu, half, kin, dt, eps, B, loss, force,
                                                              iters, partials, grad ? 1 : 0, pts, npts, grad_pts);
   if (int rc = cn::launch_status()) return rc;
@@ -194,6 +217,35 @@ int dpll_chain_loss_pts_f64(int32_t n_links, const double* x, const double* x_pl
     return launch_chain_loss<N>(x, x_plus, weight, inertia, mu_pair, nullptr, kin, dt, eps, B, loss, nullptr, nullptr, grad,
                                 loss_sum, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), pts, n_pts_packed,
                                 grad_pts);
+  });
+}
+
+int dpll_chain_loss_warm_f64(int32_t n_links, const double* x, const double* x_plus, const double* weight,
+                             const double* inertia, const double* mu_pair, const double* half, const double* kin,
+                             double dt, double eps, int64_t B, double* loss, double* force, int32_t* iters, double* grad,
+                             double* loss_sum, const double* u_init, double* u_out, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+  if (B < 0 || !inertia || !mu_pair || !half || !kin) return DPLL_EINVAL;
+  if (B > 0 && (!x || !x_plus)) return DPLL_EINVAL;
+  return cn::with_links(n_links, [&](auto N) {
+    return launch_chain_loss<N>(x, x_plus, weight, inertia, mu_pair, half, kin, dt, eps, B, loss, force, iters, grad,
+                                loss_sum, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), nullptr, 0u,
+                                nullptr, u_init, u_out);
+  });
+}
+
+int dpll_chain_loss_pts_warm_f64(int32_t n_links, const double* x, const double* x_plus, const double* weight,
+                                 const double* inertia, const double* mu_pair, const double* kin, const double* pts,
+                                 uint32_t n_pts_packed, double dt, double eps, int64_t B, double* loss, double* grad_pts,
+                                 double* grad, double* loss_sum, const double* u_init, double* u_out, int32_t* iters,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  if (B < 0 || !inertia || !mu_pair || !kin) return DPLL_EINVAL;
+  if (B > 0 && (!x || !x_plus || !pts)) return DPLL_EINVAL;
+  if (B == 0) return DPLL_OK;                            // as dpll_chain_loss_pts_f64
+  return cn::with_links(n_links, [&](auto N) {
+    return launch_chain_loss<N>(x, x_plus, weight, inertia, mu_pair, nullptr, kin, dt, eps, B, loss, nullptr, iters, grad,
+                                loss_sum, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), pts, n_pts_packed,
+                                grad_pts, u_init, u_out);
   });
 }
 

@@ -351,16 +351,23 @@ CN_HD void chain_eval(const ChainParams<T, N>& P, const ChainProb<T, N>& S, cons
   scale2 = t_max(a2, b2);
 }
 
-// the visit scheme of cube_newton_visit / elbow_solve, dimension NV, dense Cholesky
-template <typename T, int N>
-CN_HD int chain_solve(const ChainParams<T, N>& P, const ChainProb<T, N>& S, const SolverCfg<T>& cfg, T* u) {
-  constexpr int NV = 6 + N - 1, NC = 4 * N;
+// every contact's q in the polar cone: u = 0 is the exact optimum (free flight)
+template <typename T, int N> CN_HD bool chain_open(const ChainProb<T, N>& S) {
+  constexpr int NC = 4 * N;
   bool open = true;
   for (int c = 0; c < NC; ++c) {
     const T q0 = S.q[3 * c], q1 = S.q[3 * c + 1], qn = S.q[3 * c + 2];
     open = open && (qn >= T(0)) && (q0 * q0 + q1 * q1 <= qn * qn);
   }
-  if (open) return 0;
+  return open;
+}
+
+// the visit scheme of cube_newton_visit / elbow_solve, dimension NV, dense Cholesky.  Free flight returns at once and
+// leaves u as it is.
+template <typename T, int N>
+CN_HD int chain_solve(const ChainParams<T, N>& P, const ChainProb<T, N>& S, const SolverCfg<T>& cfg, T* u) {
+  constexpr int NV = 6 + N - 1;
+  if (chain_open<T, N>(S)) return 0;
   int it = 0;
   T d[NV], d0 = T(0), best = T(-1);
   T alpha = T(1), lo = T(0), hi = T(1);
@@ -434,10 +441,12 @@ template <typename T, int N> CN_HD void chain_to_world(const T* R0, const T* v, 
 }
 
 // ContactNets loss + envelope backward.  grad layout (14 N): [inertia N x 10 | mu N | half N x 3]; force_out (3 NC,
-// nullable): [n (NC); (tx, ty) (NC)].
+// nullable): [n (NC); (tx, ty) (NC)].  u0 (NV, nullable): start point of the solve instead of u = 0 (a warm start);
+// u_opt (NV, nullable): the optimum, 0 for free flight and for a sample whose forces are clipped (loss 0).
 template <typename T, int N>
 CN_HD T chain_loss_sample(const ChainParams<T, N>& P, const SolverCfg<T>& cfg, const T* x, const T* xp, T* grad,
-                          T* force_out, int* iters_out, const T* pts = nullptr, unsigned npts = 0u, T* grad_pts = nullptr) {
+                          T* force_out, int* iters_out, const T* pts = nullptr, unsigned npts = 0u, T* grad_pts = nullptr,
+                          const T* u0 = nullptr, T* u_opt = nullptr) {
   constexpr int NV = 6 + N - 1, NC = 4 * N, NQ = 7 + N - 1;
   ChainKin<T, N> K;
   ChainProb<T, N> S;
@@ -481,6 +490,9 @@ CN_HD T chain_loss_sample(const ChainParams<T, N>& P, const SolverCfg<T>& cfg, c
   const T konst = T(0.5) * e + pen;
   T u[NV];
   for (int i = 0; i < NV; ++i) u[i] = T(0);
+  // a start point counts only where there is something to solve: in free flight chain_solve leaves u as it is
+  if (u0 && !chain_open<T, N>(S))
+    for (int i = 0; i < NV; ++i) u[i] = u0[i];
   const int it = chain_solve<T, N>(P, S, cfg, u);
   if (iters_out) *iters_out = it;
   // forces, loss
@@ -510,8 +522,10 @@ CN_HD T chain_loss_sample(const ChainParams<T, N>& P, const SolverCfg<T>& cfg, c
   }
   if (!(fmax <= T(1e3))) {
     if (force_out) for (int i = 0; i < 3 * NC; ++i) force_out[i] = T(0);
+    if (u_opt) for (int i = 0; i < NV; ++i) u_opt[i] = T(0);     // its next solve starts cold
     return T(0);
   }
+  if (u_opt) for (int i = 0; i < NV; ++i) u_opt[i] = u[i];
   if (force_out)
     for (int c = 0; c < NC; ++c) {
       force_out[c] = f[3 * c + 2]; force_out[NC + 2 * c] = f[3 * c]; force_out[NC + 2 * c + 1] = f[3 * c + 1];

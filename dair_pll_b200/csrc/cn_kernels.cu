@@ -8,6 +8,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/dair_pll_b200.h"
+#include "../../include/dair_pll_b200_warm_body_tree.h"
 #include "cn_cube.cuh"
 #include "cn_params.cuh"
 #include "cn_elbow.cuh"
@@ -502,6 +503,238 @@ cube_loss_wf_kernel(const IO* __restrict__ x, const IO* __restrict__ xp, const I
     T s = T(0);
 #pragma unroll
     for (int w = 0; w < kWfWarps; ++w) s += red[w][threadIdx.x];
+    partials[(int64_t)blockIdx.x * kNAcc + threadIdx.x] = s;
+  }
+}
+
+// Warm-started witness-point loss of the single body (dpll_body_loss_pts_warm_f64): the PTS instance of
+// cube_loss_wf_kernel -- same triage, slots, Newton visits and PE passes, same accumulators -- with a start point and an
+// optimum per sample.  u_init (nullable, (B, 6)): PE pass 1 seeds the slot's u from row b instead of the feasible-segment
+// point; u_out (nullable, (B, 6)): PE pass 0 writes the slot's u, the triage writes zeros for free flight (its exact
+// optimum).  Row b is read when its sample gets a slot and written when that sample is finalised, so u_init == u_out
+// works.  A kernel of its own: statements added to cube_loss_wf_kernel, even in discarded `if constexpr` branches, changed
+// ptxas's register allocation of its box instances.
+template <int UNR>
+__global__ void __launch_bounds__(kWfWarps * 32, CN_WF_MIN_BLOCKS)
+body_loss_pts_warm_kernel(const double* __restrict__ x, const double* __restrict__ xp, const double* __restrict__ weight,
+                          const double* __restrict__ inertia, const double* __restrict__ mu,
+                          const double* __restrict__ pts, int n_c, double dt, double eps, int64_t B,
+                          double* __restrict__ loss, double* __restrict__ force, double* __restrict__ grad_pts,
+                          int32_t* __restrict__ iters, double* __restrict__ partials, int want_grad,
+                          const int32_t* __restrict__ skip_flag, unsigned long long* __restrict__ dyn_counter,
+                          const double* u_init, double* u_out) {
+  using T = double;
+  if (skip_flag && *skip_flag) return;
+  extern __shared__ __align__(16) unsigned char wf_smem[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  WfWarpPool<T>* pool = reinterpret_cast<WfWarpPool<T>*>(wf_smem) + warp;
+  const unsigned lt_mask = (1u << lane) - 1u;
+
+  cn::CubeParams<T> P;
+  {
+    T in[10], m[1], h[3] = {T(0), T(0), T(0)};
+#pragma unroll
+    for (int i = 0; i < 10; ++i) in[i] = inertia[i];
+    m[0] = mu[0];
+    cn::cube_params_init(P, in, m, h, dt, eps);
+  }
+  const cn::SolverCfg<T> cfg = cn::default_cfg<T>();
+  T acc[12];                       // [d/d inertia 10 | d/d mu | loss sum], as the PTS instance
+#pragma unroll
+  for (int i = 0; i < 12; ++i) acc[i] = T(0);
+
+  const int64_t gw = (int64_t)blockIdx.x * kWfWarps + warp, W = (int64_t)gridDim.x * kWfWarps;
+  const int64_t base = B / W, rem = B % W;
+  const int64_t lo = dyn_counter ? 0 : gw * base + (gw < rem ? gw : rem);
+  const int64_t hi = dyn_counter ? B : lo + base + (gw < rem ? 1 : 0);
+  int64_t next = lo;
+
+  for (int s = lane; s < kWfSlots; s += 32) { pool->q_done[s] = (uint8_t)s; pool->sample[s] = -1; }
+  int n_act = 0, n_done = kWfSlots, h_act = 0, h_done = 0, n_in = 0, h_in = 0;
+  __syncwarp();
+
+  while (true) {
+    int phase;   // 0 = PE, 1 = N, 2 = T (triage): the scheduling of cube_loss_wf_kernel
+    const bool drain = next >= hi && n_in == 0;
+    if (next < hi && n_in < 32) phase = 2;
+    else if (drain) {
+      if (n_act > 0) phase = 1;
+      else if (n_done > 0) phase = 0;
+      else break;
+    } else if (n_done >= kWfPeMin) phase = 0;
+    else phase = 1;
+
+    if (phase == 2) {
+      int64_t first = next;
+      if (dyn_counter) {
+        unsigned long long t = 0;
+        if (lane == 0) t = atomicAdd(dyn_counter, 32ull);
+        first = (int64_t)__shfl_sync(0xffffffffu, t, 0);
+        if (first >= B) first = B;
+      }
+      const int64_t left = hi - first;
+      const int cnt = left < 32 ? (int)left : 32;
+      bool queue = false;
+      const int64_t b = first + lane;
+      if (lane < cnt) {
+        T xs[13], xps[13], gs[11];
+#pragma unroll
+        for (int i = 0; i < 13; ++i) { xs[i] = x[b * 13 + i]; xps[i] = xp[b * 13 + i]; }
+#pragma unroll
+        for (int i = 0; i < 11; ++i) gs[i] = T(0);
+        T l = T(0);
+        const T w = weight ? weight[b] : T(1);
+        if (cn::body_loss_free_flight_pts<T>(P, xs, xps, pts + b * 12, n_c, w, want_grad ? gs : (T*)nullptr,
+                                             grad_pts ? grad_pts + b * 12 : (T*)nullptr, &l)) {
+          if (force) {
+#pragma unroll
+            for (int i = 0; i < 12; ++i) force[b * 12 + i] = T(0);
+          }
+#pragma unroll
+          for (int i = 0; i < 11; ++i) acc[i] += w * gs[i];
+          if (loss) loss[b] = l;
+          acc[11] += l;
+          if (iters) iters[b] = 0;
+          if (u_out) {
+#pragma unroll 1
+            for (int i = 0; i < 6; ++i) u_out[b * 6 + i] = T(0);
+          }
+        } else {
+          queue = true;
+        }
+      }
+      const unsigned m_q = __ballot_sync(0xffffffffu, queue);
+      if (queue) pool->q_in[(h_in + n_in + __popc(m_q & lt_mask)) % kWfQin] = (int32_t)(b - lo);
+      n_in += __popc(m_q);
+      next = dyn_counter ? (first >= B ? B : lo) : next + cnt;
+    } else if (phase == 1) {
+      const int k = n_act < 32 ? n_act : 32;
+      const bool on = lane < k;
+      int st = -1;
+      int slot = 0;
+      if (on) {
+        slot = pool->q_act[(h_act + lane) % kWfSlots];
+        const cn::CubeProb<T> S{&pool->field[0][slot], kWfSlots};
+        T u[6], d[6];
+#pragma unroll
+        for (int i = 0; i < 6; ++i) { u[i] = pool->field[33 + i][slot]; d[i] = pool->field[40 + i][slot]; }
+        T best = pool->field[39][slot], d0 = pool->field[46][slot];
+        cn::CubeTrial<T> tr{pool->field[47][slot], pool->field[48][slot], pool->field[49][slot]};
+        int it = pool->iters[slot];
+        st = cn::cube_newton_visit<T, UNR>(P, S, cfg, u, d, d0, best, tr, it);
+        pool->iters[slot] = it;
+        pool->field[39][slot] = best;
+#pragma unroll
+        for (int i = 0; i < 6; ++i) { pool->field[33 + i][slot] = u[i]; pool->field[40 + i][slot] = d[i]; }
+        pool->field[46][slot] = d0;
+        pool->field[47][slot] = tr.alpha; pool->field[48][slot] = tr.lo; pool->field[49][slot] = tr.hi;
+      }
+      __syncwarp();
+      const unsigned m_done = __ballot_sync(0xffffffffu, st == cn::NEWTON_DONE);
+      const unsigned m_act = __ballot_sync(0xffffffffu, st == cn::NEWTON_CONTINUE);
+      h_act = (h_act + k) % kWfSlots; n_act -= k;
+      if (st == cn::NEWTON_DONE) pool->q_done[(h_done + n_done + __popc(m_done & lt_mask)) % kWfSlots] = (uint8_t)slot;
+      else if (st == cn::NEWTON_CONTINUE) pool->q_act[(h_act + n_act + __popc(m_act & lt_mask)) % kWfSlots] = (uint8_t)slot;
+      n_done += __popc(m_done); n_act += __popc(m_act);
+    } else {
+      // PE: pass 0 finalises the finished samples (optimum to u_out), pass 1 parks the next triaged ones (start from
+      // u_init)
+      const int k = n_done < 32 ? n_done : 32;
+      const bool on = lane < k;
+      int slot = 0, old = -1;
+      if (on) { slot = pool->q_done[(h_done + lane) % kWfSlots]; old = pool->sample[slot]; }
+      bool to_active = false;
+      int n_new = 0;
+#pragma unroll 1
+      for (int pass = 0; pass < 2; ++pass) {
+        if (pass == 0) {
+          if (!__any_sync(0xffffffffu, on && old >= 0)) continue;
+        } else {
+          n_new = n_in < k ? n_in : k;
+          if (n_new == 0) break;
+        }
+        const bool work = pass == 0 ? (on && old >= 0) : (lane < n_new);
+        if (work) {
+          const int32_t ent = pass == 0 ? old : pool->q_in[(h_in + lane) % kWfQin];
+          const int64_t b = lo + ent;
+          T xs[13], xps[13];
+#pragma unroll
+          for (int i = 0; i < 13; ++i) { xs[i] = x[b * 13 + i]; xps[i] = xp[b * 13 + i]; }
+          const cn::CubeProb<T> S{&pool->field[0][slot], kWfSlots};
+          cn::CubeLossAux<T> A;
+          cn::body_loss_prologue_pts<T, kWfUnrPE>(P, xs, xps, pts + b * 12, n_c, S, A);
+          if (pass == 0) {
+            T u[6], gs[11], fo[12];
+#pragma unroll
+            for (int i = 0; i < 6; ++i) u[i] = pool->field[33 + i][slot];
+#pragma unroll
+            for (int i = 0; i < 11; ++i) gs[i] = T(0);
+            const T w = weight ? weight[b] : T(1);
+            const T l = cn::body_loss_epilogue_pts<T, kWfUnrPE, true>(P, S, A, u, n_c, w, want_grad ? gs : (T*)nullptr,
+                                                                      grad_pts ? grad_pts + b * 12 : (T*)nullptr,
+                                                                      force ? fo : (T*)nullptr);
+            if (force) {
+#pragma unroll
+              for (int i = 0; i < 12; ++i) force[b * 12 + i] = fo[i];
+            }
+#pragma unroll
+            for (int i = 0; i < 11; ++i) acc[i] += w * gs[i];
+            if (loss) loss[b] = l;
+            acc[11] += l;
+            if (iters) iters[b] = pool->iters[slot] & 0xff;
+            if (u_out) {
+#pragma unroll
+              for (int i = 0; i < 6; ++i) u_out[b * 6 + i] = u[i];
+            }
+            pool->sample[slot] = -1;
+          } else {
+            T us[6];
+            if (u_init) {
+#pragma unroll
+              for (int i = 0; i < 6; ++i) us[i] = u_init[b * 6 + i];
+            } else {
+              cn::cube_loss_start<T>(A, T(CN_LOSS_START_FACTOR), us);
+            }
+#pragma unroll
+            for (int i = 0; i < 6; ++i) pool->field[33 + i][slot] = us[i];
+            pool->field[39][slot] = T(-1);
+            pool->field[46][slot] = T(0);
+            pool->sample[slot] = (int32_t)(b - lo);
+            pool->iters[slot] = 0;
+            to_active = true;
+          }
+        }
+      }
+      h_in = (h_in + n_new) % kWfQin; n_in -= n_new;
+      const bool more = next < hi || n_in > 0;
+      __syncwarp();
+      const unsigned m_act = __ballot_sync(0xffffffffu, to_active);
+      const unsigned m_keep = __ballot_sync(0xffffffffu, on && !to_active && more);
+      h_done = (h_done + k) % kWfSlots; n_done -= k;
+      if (to_active) pool->q_act[(h_act + n_act + __popc(m_act & lt_mask)) % kWfSlots] = (uint8_t)slot;
+      else if (on && more) pool->q_done[(h_done + n_done + __popc(m_keep & lt_mask)) % kWfSlots] = (uint8_t)slot;
+      n_act += __popc(m_act); n_done += __popc(m_keep);
+    }
+    __syncwarp();
+  }
+
+  if (!partials) return;
+  __shared__ T red[kWfWarps][kNAcc];
+#pragma unroll 1
+  for (int i = 0; i < 12; ++i) {
+    T v = T(0);
+#pragma unroll
+    for (int j = 0; j < 12; ++j) v = (j == i) ? acc[j] : v;
+    const T s = warp_sum(v);
+    if (lane == 0) red[warp][i] = s;
+  }
+  __syncthreads();
+  if (threadIdx.x < kNAcc) {
+    T s = T(0);
+    if (threadIdx.x < 12) {
+#pragma unroll
+      for (int w = 0; w < kWfWarps; ++w) s += red[w][threadIdx.x];
+    }
     partials[(int64_t)blockIdx.x * kNAcc + threadIdx.x] = s;
   }
 }
@@ -1037,6 +1270,48 @@ int dpll_body_loss_pts_f64(const double* x, const double* x_plus, const double* 
     return rc;
   if (!want_red) return DPLL_OK;
   reduce_partials_kernel<double, double, kNAcc, 11><<<1, 32 * kNAcc, 0, st>>>(partials, rows, grad, loss_sum, skip_flag);
+  return cn::launch_status();
+}
+
+int dpll_body_loss_pts_warm_f64(const double* x, const double* x_plus, const double* weight, const double* inertia,
+                                const double* mu_pair, const double* pts, int32_t n_contacts, double dt, double eps,
+                                int64_t B, int32_t flags, double* loss, double* force, double* grad_pts, int32_t* iters,
+                                double* grad, double* loss_sum, const int32_t* skip_flag, const double* u_init,
+                                double* u_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!u_init && !u_out)      // exactly what dpll_body_loss_pts_f64 launches
+    return dpll_body_loss_pts_f64(x, x_plus, weight, inertia, mu_pair, pts, n_contacts, dt, eps, B, flags, loss, force,
+                                  grad_pts, iters, grad, loss_sum, skip_flag, workspace, workspace_bytes, stream);
+  if (B < 0 || !inertia || !mu_pair || n_contacts < 1 || n_contacts > DPLL_CUBE_NC) return DPLL_EINVAL;
+  if (B > 0 && (!x || !x_plus || !pts)) return DPLL_EINVAL;
+  const bool want_red = grad || loss_sum;
+  const bool dynamic = (flags & DPLL_LOSS_DYNAMIC) != 0;
+  if ((want_red || dynamic) && !cn::workspace_ok(workspace, workspace_bytes)) return DPLL_EWORKSPACE;
+  if (B == 0 && !want_red) return DPLL_OK;      // nothing to write: an empty warm call launches nothing
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  double* partials = want_red ? static_cast<double*>(workspace) : nullptr;
+  // the grid and instance policy of launch_cube_wf
+  const size_t smem = sizeof(WfWarpPool<double>) * kWfWarps;
+  cudaError_t ea = cudaFuncSetAttribute(body_loss_pts_warm_kernel<kWfUnr>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)smem);
+  if (ea == cudaSuccess)
+    ea = cudaFuncSetAttribute(body_loss_pts_warm_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (ea != cudaSuccess) return (int)ea;
+  int blocks;
+  int64_t cap;
+  if (int rc = cn::resident_blocks(body_loss_pts_warm_kernel<kWfUnr>, kWfWarps * 32, smem,
+                                   (B + kWfWarps * kWfMinPerWarp - 1) / (kWfWarps * kWfMinPerWarp), kMaxBlocks,
+                                   &blocks, &cap))
+    return rc;
+  unsigned long long* dyn = nullptr;
+  if (dynamic)
+    if (int rc = cn::dynamic_counter(workspace, st, &dyn)) return rc;
+  const bool small = B <= cap * kWfWarps * 320;
+  auto kernel = small ? body_loss_pts_warm_kernel<4> : body_loss_pts_warm_kernel<kWfUnr>;
+  kernel<<<blocks, kWfWarps * 32, smem, st>>>(x, x_plus, weight, inertia, mu_pair, pts, n_contacts, dt, eps, B, loss, force,
+                                              grad_pts, iters, partials, grad ? 1 : 0, skip_flag, dyn, u_init, u_out);
+  if (int rc = cn::launch_status()) return rc;
+  if (!want_red) return DPLL_OK;
+  reduce_partials_kernel<double, double, kNAcc, 11><<<1, 32 * kNAcc, 0, st>>>(partials, blocks, grad, loss_sum, skip_flag);
   return cn::launch_status();
 }
 

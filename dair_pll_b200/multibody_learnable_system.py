@@ -61,10 +61,11 @@ class MultibodyLearnableSystem(System):
         self.race_expensive_head = True  # with dynamic_schedule, small launches: the first B/64 samples of the (cost-ordered)
                                          # batch are solved from eight start points at once, first to converge wins (cube)
         self.record_newton_iters = False  # BatchLoss.newton_iters: per-sample cost hint for the data set
-        self.qp_warm_start = None        # (B, 6) / (B, 7) contiguous start points of the next contactnets_loss call's solves
-                                         # (cube, elbow); with record_qp_solution it is overwritten in place by the optima
-        self.record_qp_solution = False  # BatchLoss.qp_solution (B, 6) / (B, 7): the optima, next epoch's warm start
-                                         # (cube, elbow)
+        self.qp_warm_start = None        # (B, 6) / (B, 7) / (B, 5 + n) contiguous start points of the next contactnets_loss
+                                         # call's solves (single body, elbow, trees of n links); with
+                                         # record_qp_solution it is overwritten in place by the optima
+        self.record_qp_solution = False  # BatchLoss.qp_solution (B, 6) / (B, 7) / (B, 5 + n): the optima, next epoch's
+                                         # warm start (every system)
         self._kin_cache = {}
 
     # -- helpers ---------------------------------------------------------
@@ -179,12 +180,17 @@ class MultibodyLearnableSystem(System):
             xf, xpf = self._flat(x).to(torch.float64), self._flat(x_plus).to(torch.float64)
             pts, n_c = self._body_witness_points(xpf[:, :4])
             flags = ops.LOSS_DYNAMIC if self.dynamic_schedule else 0
-            loss, iters = ops.BodyWitnessPointLoss.apply(xf, xpf, inertia, mu, pts, n_c, float(self.dt), LOSS_EPS, flags,
-                                                         self.record_newton_iters)
+            u_init = self._f64_warm_start(xf.shape[0], 6)
+            res = ops.BodyWitnessPointLoss.apply(xf, xpf, inertia, mu, pts, n_c, float(self.dt), LOSS_EPS, flags,
+                                                 self.record_newton_iters, u_init, self.record_qp_solution)
+            loss, iters = res[0], res[1]
             out = loss.to(x.dtype).reshape(batch).as_subclass(ops.BatchLoss)
             out._dpll_fused = None           # mean() / sum() are plain reductions: the points' gradient needs the graph
             out.newton_iters = iters.reshape(batch) if self.record_newton_iters else None
             out.qp_solution = None
+            if self.record_qp_solution:
+                # with a warm start the optima were written back into the warm-start tensor itself
+                out.qp_solution = (u_init if u_init is not None else res[2]).reshape(batch + (6,))
             return out
         if self._kind() == 'cube':
             lt, ct = self.multibody_terms.lagrangian_terms, self.multibody_terms.contact_terms
@@ -251,15 +257,42 @@ class MultibodyLearnableSystem(System):
                 mu = torch.cat((mu, mu.new_ones(n - mu.shape[0])))
             xf, xpf = self._flat(x).to(torch.float64), self._flat(x_plus).to(torch.float64)
             pts, packed = mt.chain_witness_points(xpf[:, :7 + n - 1])
-            loss = ops.ChainWitnessPointLoss.apply(xf, xpf, inertia.reshape(-1), mu, pts, mt.chain_kinematic_table(x.device, True),
-                                                   n, packed, float(self.dt), LOSS_EPS).to(x.dtype)
+            u_init = self._f64_warm_start(xf.shape[0], 5 + n)
+            iters = torch.empty(xf.shape[0], dtype=torch.int32, device=x.device) if self.record_newton_iters else None
+            out = ops.ChainWitnessPointLoss.apply(xf, xpf, inertia.reshape(-1), mu, pts, mt.chain_kinematic_table(x.device, True),
+                                                  n, packed, float(self.dt), LOSS_EPS, u_init, self.record_qp_solution, iters)
         elif self._kind() == 'chain':
             inertia, mu, half, kin, n = self._chain_params(x.device)
-            loss = ops.ChainContactNetsLoss.apply(self._flat(x).to(torch.float64), self._flat(x_plus).to(torch.float64),
-                                                  inertia, mu, half, kin, n, float(self.dt), LOSS_EPS).to(x.dtype)
+            xf = self._flat(x).to(torch.float64)
+            u_init = self._f64_warm_start(xf.shape[0], 5 + n)
+            iters = torch.empty(xf.shape[0], dtype=torch.int32, device=x.device) if self.record_newton_iters else None
+            out = ops.ChainContactNetsLoss.apply(xf, self._flat(x_plus).to(torch.float64), inertia, mu, half, kin, n,
+                                                 float(self.dt), LOSS_EPS, u_init, self.record_qp_solution, iters)
         else:
             raise NotImplementedError(f'no kernel specialisation for system kind {self._kind()!r}')
-        return loss.reshape(batch)
+        if u_init is None and not self.record_qp_solution and iters is None:
+            return out.to(x.dtype).reshape(batch)
+        loss, usol = out if (u_init is not None or self.record_qp_solution) else (out, None)
+        result = loss.to(x.dtype).reshape(batch).as_subclass(ops.BatchLoss)
+        result._dpll_fused = None                # mean() / sum() are plain reductions of the (B,) loss
+        result.newton_iters = iters.reshape(batch) if iters is not None else None
+        result.qp_solution = None
+        if self.record_qp_solution:
+            # with a warm start the optima were written back into the warm-start tensor itself
+            result.qp_solution = (u_init if u_init is not None else usol).reshape(batch + (5 + n,))
+        return result
+
+    def _f64_warm_start(self, B: int, width: int):
+        """Consumes ``qp_warm_start`` for the float64 kernels (trees, width 5 + n; the single body with witness points,
+        width 6): None, or the (B, width) start points, contiguous when the optima are to be written into it."""
+        warm, self.qp_warm_start = self.qp_warm_start, None          # consumed by this call
+        if warm is None:
+            return None
+        if warm.shape[-1] != width or warm.numel() != width * B or warm.dtype != torch.float64 or \
+                (self.record_qp_solution and not warm.is_contiguous()):
+            raise ValueError(f'qp_warm_start must be a contiguous ({B}, {width}) torch.float64 tensor for this batch, '
+                             f'got {tuple(warm.shape)} {warm.dtype}')
+        return warm.reshape(B, width)
 
     # -- simulation ------------------------------------------------------
     def _rollout(self, x_0: Tensor, steps: int) -> Tensor:

@@ -365,6 +365,33 @@ def cube_rollout(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, dt:
     return traj, force
 
 
+def _warm_rows(x: Tensor, u_init: Optional[Tensor], width: int) -> Optional[Tensor]:
+    """``u_init`` checked as (B, width) start points and passed contiguous in the launch dtype."""
+    if u_init is None:
+        return None
+    if tuple(u_init.shape) != (x.shape[0], width):
+        raise ValueError(f'u_init must be (B,{width}), got {tuple(u_init.shape)}')
+    return u_init.detach().to(x.dtype).contiguous()
+
+
+def _check_optima_out(x: Tensor, u_out: Optional[Tensor], width: int) -> None:
+    """``u_out``, when given, must be a contiguous (B, width) tensor of the launch dtype: the kernel writes it in place."""
+    if u_out is not None and (tuple(u_out.shape) != (x.shape[0], width) or u_out.dtype != x.dtype or
+                              not u_out.is_contiguous()):
+        raise ValueError(f'u_out must be a contiguous (B,{width}) {x.dtype} tensor, got {tuple(u_out.shape)} {u_out.dtype}')
+
+
+def _loss_and_optima(ctx, loss: Tensor, u_init: Optional[Tensor], want_u: bool, u_out: Optional[Tensor]):
+    """The return of a loss Function with the warm-start protocol of :class:`ElbowContactNetsLossPts`: the loss alone
+    without a warm start or a record request, else (loss, usol) with ``usol`` non-differentiable -- the new optima, or
+    empty when they went into ``u_init`` in place."""
+    if u_init is None and not want_u:
+        return loss
+    usol = u_out if (u_out is not None and u_init is None) else torch.empty(0, dtype=loss.dtype, device=loss.device)
+    ctx.mark_non_differentiable(usol)
+    return loss, usol
+
+
 def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, half: Optional[Tensor], kin: Tensor,
                    dt: float, eps: float, weight: Optional[Tensor] = None, want_grad: bool = True,
                    want_force: bool = False, want_iters: bool = False, want_loss: bool = True,
@@ -399,12 +426,8 @@ def elbow_loss_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, 
     if weight is not None:
         weight = weight.to(dtype).contiguous()
     grad_pts = torch.zeros((B, 8, 3), dtype=dtype, device=dev) if (want_grad_pts and want_grad) else None
-    if u_init is not None:
-        if tuple(u_init.shape) != (B, 7):
-            raise ValueError(f'u_init must be (B,7), got {tuple(u_init.shape)}')
-        u_init = u_init.detach().to(dtype).contiguous()
-    if u_out is not None and (tuple(u_out.shape) != (B, 7) or u_out.dtype != dtype or not u_out.is_contiguous()):
-        raise ValueError(f'u_out must be a contiguous (B,7) {dtype} tensor, got {tuple(u_out.shape)} {u_out.dtype}')
+    u_init = _warm_rows(x, u_init, 7)
+    _check_optima_out(x, u_out, 7)
     if u_init is None and u_out is None:
         _call('dpll_elbow_loss', dev, x, x_plus, weight, inertia, mu_pair, half, kin, pts, dt, eps, B, flags, loss, force,
               grad_pts, iters, grad, loss_sum, skip_flag, dtype=dtype, workspace=True)
@@ -456,13 +479,14 @@ class ElbowContactNetsLoss(torch.autograd.Function):
         return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None, None, None, None)
 
 
-def _optima_buffer(x: Tensor, u_init: Optional[Tensor], want_u: bool) -> Optional[Tensor]:
-    """Where a warm-started elbow launch writes its optima: ``u_init`` itself (in place: a training loop keeps one (B,7)
-    buffer per batch and copies nothing between epochs), a new (B,7) tensor, or nowhere."""
+def _optima_buffer(x: Tensor, u_init: Optional[Tensor], want_u: bool, width: int = 7) -> Optional[Tensor]:
+    """Where a warm-started launch writes its optima: ``u_init`` itself (in place: a training loop keeps one (B, width)
+    buffer per batch and copies nothing between epochs), a new (B, width) tensor, or nowhere.  ``width``: 7 for the elbow,
+    5 + n for a tree of n links."""
     if not want_u:
         return None
     if u_init is None:
-        return torch.empty((x.shape[0], 7), dtype=x.dtype, device=x.device)
+        return torch.empty((x.shape[0], width), dtype=x.dtype, device=x.device)
     if u_init.dtype != x.dtype or not u_init.is_contiguous():
         raise ValueError(f'a warm start that records the optima in place must be a contiguous {x.dtype} tensor, got '
                          f'{u_init.dtype}')
@@ -489,11 +513,7 @@ class ElbowContactNetsLossPts(torch.autograd.Function):
         ctx.dt, ctx.eps = dt, eps
         if need:
             ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts, kin, u_out if u_out is not None else u_init)
-        if u_init is None and not want_u:
-            return loss
-        usol = u_out if (u_out is not None and u_init is None) else torch.empty(0, dtype=loss.dtype, device=loss.device)
-        ctx.mark_non_differentiable(usol)
-        return loss, usol
+        return _loss_and_optima(ctx, loss, u_init, want_u, u_out)
 
     @staticmethod
     def backward(ctx, grad_loss, _g_u=None):
@@ -616,10 +636,13 @@ class ElbowStepPts(torch.autograd.Function):
 def body_loss_pts_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_contacts: int, dt: float,
                       eps: float, weight: Optional[Tensor] = None, want_grad: bool = True, want_loss: bool = True,
                       want_grad_pts: bool = True, want_iters: bool = False, want_force: bool = False, flags: int = 0,
-                      skip_flag: Optional[Tensor] = None, grad_out: Optional[Tensor] = None):
+                      skip_flag: Optional[Tensor] = None, grad_out: Optional[Tensor] = None,
+                      u_init: Optional[Tensor] = None, u_out: Optional[Tensor] = None):
     """Direct call of ``dpll_body_loss_pts_f64`` (``flags``: LOSS_DYNAMIC for cost-ordered batches).  x, x_plus (B,13), inertia
     (10), mu_pair (1), witness points pts (B,4,3) of which the first ``n_contacts`` rows are used.  Returns (loss (B,) | None,
-    grad (11,) | None, loss_sum (1,), grad_pts (B,4,3) | None, iters (B,) | None, force (B,12) | None)."""
+    grad (11,) | None, loss_sum (1,), grad_pts (B,4,3) | None, iters (B,) | None, force (B,12) | None).  ``u_init`` (B,6):
+    start point of every sample's solve; ``u_out`` (B,6), contiguous float64: receives every sample's optimum (zero for
+    free flight) and may be ``u_init`` itself.  With either, ``dpll_body_loss_pts_warm_f64`` runs."""
     _check_inputs(x, x_plus, inertia, mu_pair, pts, f64_only='the witness-point kernels are provided in float64')
     x, x_plus, pts = x.contiguous(), x_plus.contiguous(), pts.contiguous()
     B, dev = x.shape[0], x.device
@@ -634,8 +657,15 @@ def body_loss_pts_raw(x: Tensor, x_plus: Tensor, inertia: Tensor, mu_pair: Tenso
     force = torch.empty((B, 12), dtype=x.dtype, device=dev) if want_force else None
     if weight is not None:
         weight = weight.to(x.dtype).contiguous()
-    _call('dpll_body_loss_pts_f64', dev, x, x_plus, weight, inertia.contiguous(), mu_pair.contiguous(), pts, n_contacts, dt,
-          eps, B, flags, loss, force, gpts, iters, grad, loss_sum, skip_flag, workspace=True)
+    u_init = _warm_rows(x, u_init, 6)
+    _check_optima_out(x, u_out, 6)
+    if u_init is None and u_out is None:
+        _call('dpll_body_loss_pts_f64', dev, x, x_plus, weight, inertia.contiguous(), mu_pair.contiguous(), pts, n_contacts,
+              dt, eps, B, flags, loss, force, gpts, iters, grad, loss_sum, skip_flag, workspace=True)
+    else:
+        _call('dpll_body_loss_pts_warm_f64', dev, x, x_plus, weight, inertia.contiguous(), mu_pair.contiguous(), pts,
+              n_contacts, dt, eps, B, flags, loss, force, gpts, iters, grad, loss_sum, skip_flag, u_init, u_out,
+              workspace=True)
     return loss, grad, loss_sum, gpts, iters, force
 
 
@@ -645,27 +675,37 @@ class BodyWitnessPointLoss(torch.autograd.Function):
     the wavefront kernel.  Differentiable w.r.t. inertia (10), mu_pair (1) and ``pts``; float64.  Returns (loss, iters):
     ``iters`` (B,) int32 Newton directions per sample when ``want_iters``, else empty.  Backward: a uniform upstream
     gradient scales the forward's own sums; other weights take one weighted pass, which the device skips
-    (``skip_flag``) when they are uniform after all -- no host read, so the step can be captured into a CUDA graph."""
+    (``skip_flag``) when they are uniform after all -- no host read, so the step can be captured into a CUDA graph.
+
+    ``u_init`` (B,6): warm start of every sample's solve; ``want_u``: record the optima (``dpll_body_loss_pts_warm_f64``).
+    When either is given the Function returns (loss, iters, usol), ``usol`` non-differentiable: empty when the optima went
+    into ``u_init`` in place, else a new (B,6) tensor.  A weighted backward re-launch starts from the optima (or from
+    ``u_init``) and records nothing."""
 
     @staticmethod
-    def forward(ctx, x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, flags=0, want_iters=False):
+    def forward(ctx, x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, flags=0, want_iters=False, u_init=None,
+                want_u=False):
+        _warm_rows(x, u_init, 6)                         # shape check before the optima buffer is chosen
+        u_out = _optima_buffer(x, u_init, want_u, 6)
         loss, grad, _, gpts, iters, _ = body_loss_pts_raw(x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, flags=flags,
-                                                          want_iters=want_iters)
+                                                          want_iters=want_iters, u_init=u_init, u_out=u_out)
         ctx.args = (n_contacts, dt, eps, flags)
-        ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts)
+        ctx.save_for_backward(grad, gpts, x, x_plus, inertia, mu_pair, pts, u_out if u_out is not None else u_init)
         if iters is None:
             iters = torch.empty(0, dtype=torch.int32, device=loss.device)
         ctx.mark_non_differentiable(iters)
-        return loss, iters
+        out = _loss_and_optima(ctx, loss, u_init, want_u, u_out)
+        return (loss, iters) if out is loss else (loss, iters, out[1])
 
     @staticmethod
-    def backward(ctx, grad_loss, _g_iters):
-        grad, gpts, x, x_plus, inertia, mu_pair, pts = ctx.saved_tensors
+    def backward(ctx, grad_loss, _g_iters, _g_u=None):
+        grad, gpts, x, x_plus, inertia, mu_pair, pts, u_start = ctx.saved_tensors
         n_contacts, dt, eps, flags = ctx.args
         g = _fused_grad(grad, grad_loss, lambda w, skip, out: body_loss_pts_raw(
             x, x_plus, inertia, mu_pair, pts, n_contacts, dt, eps, weight=w, want_loss=False, want_grad_pts=False,
-            flags=flags, skip_flag=skip, grad_out=out))
-        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1), None, None, None, None, None)
+            flags=flags, skip_flag=skip, grad_out=out, u_init=u_start))
+        return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1), None, None, None, None, None,
+                None, None)
 
 
 def body_step_pts(x: Tensor, inertia: Tensor, mu_pair: Tensor, pts: Tensor, n_contacts: int, dt: float,
@@ -700,31 +740,51 @@ class BodyStepPts(torch.autograd.Function):
 
 class ChainContactNetsLoss(torch.autograd.Function):
     """ContactNets loss of a generic floating-base serial chain of ``n`` links (``dpll_chain_loss_f64``,
-    csrc/cn_chain.cuh): differentiable w.r.t. inertia (n,10), mu_pair (n), half (n,3); float64."""
+    csrc/cn_chain.cuh): differentiable w.r.t. inertia (n,10), mu_pair (n), half (n,3); float64.
+
+    ``u_init`` (B, 5+n): warm start of every sample's solve; ``want_u``: record the optima (``dpll_chain_loss_warm_f64``).
+    As for :class:`ElbowContactNetsLossPts`, when either is given the Function returns (loss, usol), ``usol``
+    non-differentiable: empty when the optima went into ``u_init`` in place, else a new (B, 5+n) tensor; otherwise the loss
+    alone.  The backward's weighted re-launch starts from the optima (or from ``u_init``) and records nothing.
+    ``iters_out`` (B,) int32, optional: receives every sample's Newton count (the data set's cost hint)."""
 
     @staticmethod
-    def forward(ctx, x, x_plus, inertia, mu_pair, half, kin, n, dt, eps):
+    def forward(ctx, x, x_plus, inertia, mu_pair, half, kin, n, dt, eps, u_init=None, want_u=False, iters_out=None):
         _check_inputs(x, x_plus, inertia, mu_pair, half, kin, f64_only='the generic chain kernels are provided in float64')
         x, x_plus = x.contiguous(), x_plus.contiguous()
         _check_states(13 + 2 * (n - 1), x, x_plus)
         B, dev = x.shape[0], x.device
         loss = torch.empty(B, dtype=x.dtype, device=dev)
+        start = _warm_rows(x, u_init, 5 + n)
+        u_out = _optima_buffer(x, u_init, want_u, 5 + n)
+        if u_out is not None and u_init is not None:
+            start = u_out                 # the optima overwrite the start points in place
         ctx.args = (n, dt, eps)
-        ctx.save_for_backward(x, x_plus, inertia, mu_pair, half, kin)
-        _call('dpll_chain_loss_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(), half.contiguous(),
-              kin.contiguous(), dt, eps, B, loss, None, None, None, None, workspace=True)
-        return loss
+        if start is None and u_out is None:
+            _call('dpll_chain_loss_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(),
+                  half.contiguous(), kin.contiguous(), dt, eps, B, loss, None, iters_out, None, None, workspace=True)
+        else:
+            _call('dpll_chain_loss_warm_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(),
+                  half.contiguous(), kin.contiguous(), dt, eps, B, loss, None, iters_out, None, None, start, u_out,
+                  workspace=True)
+        # the last one is the start point of the backward's weighted re-launch
+        ctx.save_for_backward(x, x_plus, inertia, mu_pair, half, kin, u_out if u_out is not None else start)
+        return _loss_and_optima(ctx, loss, u_init, want_u, u_out)
 
     @staticmethod
-    def backward(ctx, grad_loss):
-        x, x_plus, inertia, mu_pair, half, kin = ctx.saved_tensors
+    def backward(ctx, grad_loss, _g_u=None):
+        x, x_plus, inertia, mu_pair, half, kin, u_start = ctx.saved_tensors
         n, dt, eps = ctx.args
         B, dev = x.shape[0], x.device
         g = torch.zeros(14 * n, dtype=x.dtype, device=dev)
-        if B > 0:
+        if B > 0 and u_start is None:
             _call('dpll_chain_loss_f64', dev, n, x, x_plus, grad_loss.contiguous(), inertia.contiguous(), mu_pair.contiguous(),
                   half.contiguous(), kin.contiguous(), dt, eps, B, None, None, None, g, None, workspace=True)
-        return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None)
+        elif B > 0:
+            _call('dpll_chain_loss_warm_f64', dev, n, x, x_plus, grad_loss.contiguous(), inertia.contiguous(),
+                  mu_pair.contiguous(), half.contiguous(), kin.contiguous(), dt, eps, B, None, None, None, g, None, u_start,
+                  None, workspace=True)
+        return (None, None, *_split(g, inertia, mu_pair, half), None, None, None, None, None, None, None)
 
 
 def chain_rollout(x0: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, kin: Tensor, n: int, dt: float,
@@ -795,10 +855,12 @@ class ChainWitnessPointLoss(torch.autograd.Function):
     """ContactNets loss of a generic tree of ``n`` links whose contact sets are given by witness points ``pts``
     (B, n, 4, 3) in link coordinates (``n_pts_packed``: points per slot, 3 bits each) -- spheres, polygons, learned meshes,
     boxes in any frame on any link: ``dpll_chain_loss_pts_f64``.  Differentiable w.r.t. inertia (n,10), mu_pair (n) and
-    ``pts``; float64."""
+    ``pts``; float64.  ``u_init`` / ``want_u`` / ``iters_out`` as for :class:`ChainContactNetsLoss`
+    (``dpll_chain_loss_pts_warm_f64``)."""
 
     @staticmethod
-    def forward(ctx, x, x_plus, inertia, mu_pair, pts, kin, n, n_pts_packed, dt, eps):
+    def forward(ctx, x, x_plus, inertia, mu_pair, pts, kin, n, n_pts_packed, dt, eps, u_init=None, want_u=False,
+                iters_out=None):
         _check_inputs(x, x_plus, inertia, mu_pair, pts, kin, f64_only='the generic tree kernels are provided in float64')
         n_x = 13 + 2 * (n - 1)
         x, x_plus, pts = x.contiguous(), x_plus.contiguous(), pts.contiguous()
@@ -807,23 +869,36 @@ class ChainWitnessPointLoss(torch.autograd.Function):
             raise ValueError(f'expected (B,{n_x}) states and (B,{n},4,3) points, got {tuple(x.shape)} / {tuple(pts.shape)}')
         loss = torch.empty(B, dtype=x.dtype, device=dev)
         gpts = torch.empty_like(pts)
-        _call('dpll_chain_loss_pts_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(), kin.contiguous(),
-              pts, n_pts_packed, dt, eps, B, loss, gpts, None, None, workspace=True)
+        start = _warm_rows(x, u_init, 5 + n)
+        u_out = _optima_buffer(x, u_init, want_u, 5 + n)
+        if u_out is not None and u_init is not None:
+            start = u_out                 # the optima overwrite the start points in place
+        if start is None and u_out is None and iters_out is None:
+            _call('dpll_chain_loss_pts_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(),
+                  kin.contiguous(), pts, n_pts_packed, dt, eps, B, loss, gpts, None, None, workspace=True)
+        else:
+            _call('dpll_chain_loss_pts_warm_f64', dev, n, x, x_plus, None, inertia.contiguous(), mu_pair.contiguous(),
+                  kin.contiguous(), pts, n_pts_packed, dt, eps, B, loss, gpts, None, None, start, u_out, iters_out,
+                  workspace=True)
         ctx.args = (n, n_pts_packed, dt, eps)
-        ctx.save_for_backward(gpts, x, x_plus, inertia, mu_pair, pts, kin)
-        return loss
+        ctx.save_for_backward(gpts, x, x_plus, inertia, mu_pair, pts, kin, u_out if u_out is not None else start)
+        return _loss_and_optima(ctx, loss, u_init, want_u, u_out)
 
     @staticmethod
-    def backward(ctx, grad_loss):
-        gpts, x, x_plus, inertia, mu_pair, pts, kin = ctx.saved_tensors
+    def backward(ctx, grad_loss, _g_u=None):
+        gpts, x, x_plus, inertia, mu_pair, pts, kin, u_start = ctx.saved_tensors
         n, packed, dt, eps = ctx.args
         B, dev = x.shape[0], x.device
         g = torch.zeros(14 * n, dtype=x.dtype, device=dev)
-        if B > 0:
+        if B > 0 and u_start is None:
             _call('dpll_chain_loss_pts_f64', dev, n, x, x_plus, grad_loss.contiguous(), inertia.contiguous(),
                   mu_pair.contiguous(), kin.contiguous(), pts, packed, dt, eps, B, None, None, g, None, workspace=True)
+        elif B > 0:
+            _call('dpll_chain_loss_pts_warm_f64', dev, n, x, x_plus, grad_loss.contiguous(), inertia.contiguous(),
+                  mu_pair.contiguous(), kin.contiguous(), pts, packed, dt, eps, B, None, None, g, None, u_start, None, None,
+                  workspace=True)
         return (None, None, *_split(g, inertia, mu_pair), gpts * grad_loss.reshape(-1, 1, 1, 1), None, None, None, None,
-                None)
+                None, None, None, None)
 
 
 def chain_terms(q: Tensor, v: Tensor, inertia: Tensor, mu_pair: Tensor, half: Tensor, kin: Tensor, n: int, n_boxes: int):
